@@ -3,6 +3,7 @@
 
   python bench.py [--gpus N --steps K --warmup W]                 our CUDA path (libtdsfs.so through the C ABI)
   python bench.py --impl reference [--gpus N --steps K --warmup W] the reference's CPU algorithm (oracle port) on host cores
+  python bench.py ... --dump-outputs DIR                          also writes the window table of the last timed step to DIR
 
 One step = one pass of the hot path over the whole workload: genotype matrix + positions -> per-SNP counts/keys and
 genome-wide background spectra -> (all-reduce of the background across GPUs) -> window boundaries -> per-window
@@ -21,6 +22,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True  # the benchmark leaves the tree as it found it (it may be read-only)
 ROOT = os.path.dirname(os.path.abspath(__file__))
 PKG = os.path.join(ROOT, "2dsfs-scan_b200")
 if PKG not in sys.path:
@@ -389,6 +391,10 @@ def measure_workload(args, cfg, h, T, torch, dist, dev, stream, world, rank, do_
     t_a1 = time.time()
     windows.append((t_a0, t_a1))
     h.check()
+    outputs = None
+    if args.dump_outputs:  # the window table the last timed step left on the device, as a caller of tdsfs_run_bp receives it
+        outputs = h.fetch_results(h.candidates(W))
+        outputs["chrom"] = outputs["chrom"] + (chroms[0] if chroms else 0)
     fused, rec_bytes = h.scan_info()
     if os.environ.get("TDSFS_TAIL_STAMPS"):  # diagnostics: phases of the count kernel's tail in the last step (SM cycles of CTA 0)
         st = h.tail_stamps()
@@ -491,7 +497,22 @@ def measure_workload(args, cfg, h, T, torch, dist, dev, stream, world, rank, do_
     torch.cuda.empty_cache()
     return dict(value=value, ms_step=ms_step, kernel_ms=kernel_ms, launches_per_step=int(launches_per_step), e2e=e2e, verify=verify,
                 n_windows_total=n_windows_total, S_local=S_local, S_total=S_total, RW=RW, windows=windows, peer=peer["on"],
-                fused=fused, rec_bytes=rec_bytes)
+                fused=fused, rec_bytes=rec_bytes, outputs=outputs)
+
+
+DUMP_BYTES = 64 << 20
+
+
+def write_outputs(out_dir, res, seed, cap_bytes=DUMP_BYTES):
+    """One float64 .npy per result array, so that two builds can be compared window for window.  Beyond `cap_bytes` a seeded
+    sample of the windows is written; window_index.npy holds the window numbers written."""
+    n = len(res["start"])
+    cap = cap_bytes // (8 * (len(res) + 1))
+    keep = np.arange(n) if n <= cap else np.sort(np.random.default_rng(seed).choice(n, size=cap, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "window_index.npy"), keep.astype(np.float64))
+    for name, v in res.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v[keep].astype(np.float64))
 
 
 def roofline_record(cfg, m, world, workload):
@@ -530,7 +551,7 @@ def run_side(cmd, timeout):
     """A side benchmark in its own process (its JSON lines are parsed; failures are reported, not fatal)."""
     import subprocess
     try:
-        r = subprocess.run([sys.executable] + cmd, capture_output=True, text=True, timeout=timeout, cwd=ROOT)
+        r = subprocess.run([sys.executable, "-B"] + cmd, capture_output=True, text=True, timeout=timeout, cwd=ROOT)
         out = [json.loads(ln) for ln in r.stdout.splitlines() if ln.startswith("{")]
         return out if r.returncode == 0 else {"error": r.stderr[-300:], "lines": out}
     except Exception as e:  # noqa: BLE001
@@ -578,6 +599,14 @@ def run_b200(args, cfg):
         # BASELINE.json configs[0..2] (latency-bound, reference-sized): measured in their own processes after the timed regions
         extra["config3_sims_batch"] = run_side(["tools/bench_sims.py", "--generations", "2", "--replicates", "100", "--oracle-replicates", "2"], 240)
         extra["config1_2_ecb"] = run_side(["tools/bench_ecb.py"], 240)
+    if args.dump_outputs:
+        outputs = m["outputs"]
+        if world > 1:  # rank order is chromosome order: the concatenation is the table of the whole workload
+            parts = [None] * world
+            dist.all_gather_object(parts, outputs)
+            outputs = {k: np.concatenate([p[k] for p in parts]) for k in outputs}
+        if rank == 0:
+            write_outputs(args.dump_outputs, outputs, cfg["seed"])
 
     if rank != 0:
         if world > 1:
@@ -628,7 +657,12 @@ def main():
     ap.add_argument("--verify-windows", type=int, default=128, help="windows re-scored by the CPU oracle after the timed region")
     ap.add_argument("--no-graph", action="store_true", help="enqueue every pass call by call instead of replaying the captured CUDA graph")
     ap.add_argument("--no-extra", action="store_true", help="skip the config4 / config3 / ECB sub-records of the default N=1 run")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the window table of the last timed step to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computed; the reference arm only times a sample")
     cfg = dict(WORKLOADS[args.workload])
     if args.snps:
         cfg["S"] = args.snps

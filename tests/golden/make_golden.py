@@ -72,8 +72,10 @@ def do_chr1():
         cnt[i, 0:2] = v["calls"]["uv"]
         cnt[i, 2:4] = v["calls"]["bv"]
         codes[i] = vocab.setdefault(v["annotation"], len(vocab))
-    np.savez_compressed(f"{HERE}/chr1_counts.npz", chrom=np.array(chrom), pos=pos, cnt=cnt, ann_code=codes,
-                        ann_vocab=np.array(sorted(vocab, key=vocab.get)))
+    gaps = np.diff(pos.astype(np.int64), prepend=0)  # positions as uint16 gaps keep the file under 1 MB
+    assert gaps.min() >= 1 and gaps.max() < 1 << 16
+    np.savez_compressed(f"{HERE}/chr1_counts.npz", chrom=np.array(chrom), pos_delta=gaps.astype(np.uint16), cnt=cnt,
+                        ann_code=codes, ann_vocab=np.array(sorted(vocab, key=vocab.get)))
 
     # shipped CSV rows for chromosome "1"
     for tag in ("20kb", "500kb", "500snps"):

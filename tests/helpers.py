@@ -38,11 +38,16 @@ def rows_to_dict(rows, pops):
     return d
 
 
+def _chr1_pos(z):
+    """chr1_counts.npz stores the (increasing) positions as uint16 gaps: it stays under 1 MB that way."""
+    return np.cumsum(z["pos_delta"], dtype=np.int64).astype(np.int32)
+
+
 def load_chr1_dict():
     z = np.load(os.path.join(GOLDEN, "chr1_counts.npz"))
     chrom = str(z["chrom"])
     vocab = [str(v) for v in z["ann_vocab"]]
-    pos, cnt, ann = z["pos"], z["cnt"], z["ann_code"]
+    pos, cnt, ann = _chr1_pos(z), z["cnt"], z["ann_code"]
     d = {}
     for p, c, a in zip(pos.tolist(), cnt.tolist(), ann.tolist()):
         d[f"{chrom}-{p}"] = {"segregating": ("N", "N"), "context": "-N-", "calls": {"bv": (c[2], c[3]), "uv": (c[0], c[1])},
@@ -52,7 +57,7 @@ def load_chr1_dict():
 
 def load_chr1_arrays():
     z = np.load(os.path.join(GOLDEN, "chr1_counts.npz"))
-    return str(z["chrom"]), z["pos"].astype(np.int32), z["cnt"].astype(np.uint16), z["ann_code"], [str(v) for v in z["ann_vocab"]]
+    return str(z["chrom"]), _chr1_pos(z), z["cnt"].astype(np.uint16), z["ann_code"], [str(v) for v in z["ann_vocab"]]
 
 
 def load_ecb_csv(tag):

@@ -129,3 +129,28 @@ def test_bench_checksums_do_not_depend_on_the_sharding():
     # and they do depend on the content
     res["n2d"][17] += 1
     assert bench.result_checksums(res, res["chrom"].astype(np.int64), 8, (1, 2, 4))["int_checksum"] != whole["int_checksum"]
+
+
+def test_bench_dump_outputs_are_float_and_capped(tmp_path):
+    """bench.py --dump-outputs: one float64 .npy per result array, exact for the integer fields; above the byte cap the same
+    seeded sample of windows on every run."""
+    import sys
+    sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+    import bench
+    rng = np.random.default_rng(4)
+    n = 3000
+    res = dict(chrom=rng.integers(0, 32, n).astype(np.int32), start=(1 + 20000 * rng.integers(0, 1 << 30, n)).astype(np.int64),
+               T2D=rng.normal(300, 50, n), flags=rng.integers(0, 16, n).astype(np.uint8))
+    bench.write_outputs(str(tmp_path / "all"), res, 7)
+    for k, v in res.items():
+        got = np.load(tmp_path / "all" / f"{k}.npy")
+        assert got.dtype == np.float64 and np.array_equal(got, v)
+    assert np.array_equal(np.load(tmp_path / "all" / "window_index.npy"), np.arange(n))
+    cap = 8 * (len(res) + 1) * 500
+    for d in ("a", "b"):
+        bench.write_outputs(str(tmp_path / d), res, 7, cap_bytes=cap)
+    idx = np.load(tmp_path / "a" / "window_index.npy")
+    assert len(idx) == 500 and np.all(np.diff(idx) > 0)
+    assert np.array_equal(idx, np.load(tmp_path / "b" / "window_index.npy"))
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) < cap + 1024 * (len(res) + 1)
+    assert np.array_equal(np.load(tmp_path / "a" / "start.npy"), res["start"][idx.astype(np.int64)])
