@@ -139,9 +139,7 @@ struct tdsfs_ctx {
   unsigned long long* d_peer_flags = nullptr;  // this rank's flag array
   uint32_t* peer_exported_hist = nullptr;
   long long peer_words = 0;
-  unsigned long long peer_epoch = 0;
   bool peer_ready = false;
-  unsigned long long peer_pending = 0;  // epoch of the peers' "pushes landed" signal that nobody has waited for yet
   // windows / results
   long long ncand = 0, cand_cap = 0;
   std::vector<long long> cand_off_host;  // cached candidate offsets of (cand_W, cand_snp)
@@ -181,7 +179,6 @@ struct tdsfs_ctx {
 };
 
 static void peer_unmap(tdsfs_ctx* c);
-static int peer_settle(tdsfs_ctx* c);
 
 template <typename T>
 static int dev_alloc(T** p, long long n) {
@@ -576,7 +573,6 @@ extern "C" int tdsfs_background(tdsfs_t* c, int32_t mode, int32_t bg_chrom, int6
   CK(cudaSetDevice(c->device));
   NvtxRange nvtx("tdsfs:K1 count kernel (+ window sums)");
   cudaStream_t st = c->stream;
-  CKR(peer_settle(c));  // peers may still be pushing the previous exchange into the histogram
   c->ws_ready = false;  // the records (and any window sums) are rewritten by this pass
   CK(cudaEventRecord(c->ev[EV_BG0], st));
   const int NG = mode == TDSFS_BG_PER_CHROM ? c->C : 1;
@@ -637,7 +633,6 @@ extern "C" int tdsfs_background(tdsfs_t* c, int32_t mode, int32_t bg_chrom, int6
   }
 
   const int hist_bytes = (p.cr * p.cc + p.h1a + p.h1b) * 4;
-  if (const char* e = getenv("TDSFS_K1_DEBUG")) p.debug = atoi(e);  // profiling only: results are wrong
   if (c->dG) {
     const int RW = c->W1 + c->W2;
     const int blk_bytes = RW * BLK * 4;
@@ -649,7 +644,6 @@ extern "C" int tdsfs_background(tdsfs_t* c, int32_t mode, int32_t bg_chrom, int6
       const int fit = (226 * 1024 - hist_bytes) / (p.stage_bytes + 8);
       p.cwarps = std::min(K1_DEFAULT_WARPS, fit / 2);
       p.nstage = p.cwarps * 2;
-      p.interleave = 0;
       const int smem = p.nstage * p.stage_bytes + p.nstage * 8 + hist_bytes;
       CK(cudaFuncSetAttribute(k1_genotypes_wide, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
       for (auto& ch : c->chunks) {
@@ -667,8 +661,8 @@ extern "C" int tdsfs_background(tdsfs_t* c, int32_t mode, int32_t bg_chrom, int6
       // byte), fewer and larger requests for wide rows.  Deeper rings and more bytes in flight are slower on B200.
       // fused kernel (measured, profiles/README.md round 2): it is bound by per-warp instruction latency, not by bytes in
       // flight, so it takes as many warps as fit, with tiles of at most 8 KB halved until the warp limit is reached
-      // (config 5: 14 warps x 8 KB, config 4: 24 warps x 3.5 KB); the plain count kernel keeps the round-1 rule (128 KB in flight)
-      const bool old_kernel = getenv("TDSFS_K1_OLD") != nullptr || getenv("TDSFS_K1_PROBE") != nullptr;  // A/B + bandwidth probe
+      // (config 5: 14 warps x 8 KB, config 4: 24 warps x 3.5 KB); without window sums (an unplanned scan) it keeps the
+      // round-1 rule (128 KB in flight)
       // ---- fused scan: a plan for (W, mode) is pending -> the count kernel also leaves every window's background-independent sums
       FusedParams q;
       memset(&q, 0, sizeof q);
@@ -676,8 +670,8 @@ extern "C" int tdsfs_background(tdsfs_t* c, int32_t mode, int32_t bg_chrom, int6
       q.nw1 = (c->n1 + 2) / 2; q.nw2 = (c->n2 + 2) / 2;
       const int tab_words = HASH_SLOTS + ((q.nw1 + q.nw2 + 3) & ~3);
       const int smem_max = 227 * 1024;
-      bool fuse = !old_kernel && c->plan_W > 0 && c->plan_W <= 0x7FFFFFFFLL && score_small_ok(c->n1, c->n2, c->bins2d) &&
-                  !(c->plan_snp && c->plan_W > WCAP) && !getenv("TDSFS_NO_FUSE");
+      bool fuse = c->plan_W > 0 && c->plan_W <= 0x7FFFFFFFLL && score_small_ok(c->n1, c->n2, c->bins2d) &&
+                  !(c->plan_snp && c->plan_W > WCAP);
       auto fit_for = [&](int tile_blocks, bool with_tables) {
         const int stride = tile_blocks * blk_bytes + tile_blocks * BLK * 4;
         return (smem_max - hist_words * 4 - 16) / (stride + 8 + (with_tables ? tab_words * 4 : 0));
@@ -698,112 +692,82 @@ extern "C" int tdsfs_background(tdsfs_t* c, int32_t mode, int32_t bg_chrom, int6
       if (const char* e = getenv("TDSFS_K1_WARPS")) p.cwarps = std::max(1, std::min(std::min(max_warps, fit), atoi(e)));  // tuning knob
       int depth = 1;  // stages per warp
       if (const char* e = getenv("TDSFS_K1_DEPTH")) depth = std::max(1, atoi(e));  // tuning knob
-      p.nstage = p.cwarps;
-      if (old_kernel) {
-        depth = std::max(1, std::min(fit / p.cwarps, depth));
-        p.nstage = p.cwarps * depth;
-        const int smem = p.nstage * p.stage_bytes + p.nstage * 8 + hist_bytes;
-        void (*kern)(KeyParams) = k1_genotypes<0, 0>;
-        if (c->W1 == 32 && c->W2 == 32) kern = k1_genotypes<32, 32>;
-        else if (c->W1 == 14 && c->W2 == 14) kern = k1_genotypes<14, 14>;
-        if (getenv("TDSFS_K1_PROBE")) kern = k1_probe_ring;  // bandwidth probe, no spectra (profiling only)
-        CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        p.interleave = (p.bg_group == nullptr) ? 1 : 0;
-        if (const char* e = getenv("TDSFS_K1_INTERLEAVE")) p.interleave = atoi(e) != 0 && p.bg_group == nullptr;
-        for (auto& ch : c->chunks) {
-          if (ch.r1 <= ch.r0) continue;
-          if (ch.ev) CK(cudaStreamWaitEvent(st, ch.ev, 0));
-          p.r0 = ch.r0; p.r1 = ch.r1;
-          const long long nblk = (ch.r1 - ch.r0 + BLK - 1) / BLK;
-          const long long ntiles = (nblk + p.tile_blocks - 1) / p.tile_blocks;
-          const int grid = (int)std::min<long long>(ntiles, (long long)c->sm_count);
-          kern<<<grid, p.cwarps * 32, smem, st>>>(p);
-          c->launches++;
+      q.wmode = fuse ? (c->plan_snp ? 2 : 1) : 0;
+      q.tab_words = fuse ? tab_words : 0;
+      if (fuse) {
+        const long long ncand = c->cand_off_host[c->C];
+        if (ncand > c->ws_cap) {
+          CK(cudaStreamSynchronize(st));
+          dev_free(c->d_ws);
+          CKR(dev_alloc(&c->d_ws, ncand * 4));
+          c->ws_cap = ncand;
         }
+        q.W = (uint32_t)c->plan_W;
+        q.Wmagic = (uint32_t)std::min<unsigned long long>(0xFFFFFFFFull, (1ull << 32) / (unsigned long long)c->plan_W);
+        q.cand_off = c->d_cand_off;
+        q.ncand = ncand;
+        q.ws = c->d_ws;
+        q.dxI = c->d_dxI;
+        q.lnI = c->d_lnI;
       } else {
-        q.wmode = fuse ? (c->plan_snp ? 2 : 1) : 0;
-        q.tab_words = fuse ? tab_words : 0;
-        if (fuse) {
-          const long long ncand = c->cand_off_host[c->C];
-          if (ncand > c->ws_cap) {
-            CK(cudaStreamSynchronize(st));
-            dev_free(c->d_ws);
-            CKR(dev_alloc(&c->d_ws, ncand * 4));
-            c->ws_cap = ncand;
-          }
-          q.W = (uint32_t)c->plan_W;
-          q.Wmagic = (uint32_t)std::min<unsigned long long>(0xFFFFFFFFull, (1ull << 32) / (unsigned long long)c->plan_W);
-          q.cand_off = c->d_cand_off;
-          q.ncand = ncand;
-          q.ws = c->d_ws;
-          q.dxI = c->d_dxI;
-          q.lnI = c->d_lnI;
-        } else {
-          q.nw1 = q.nw2 = 0;
-        }
-        q.pos_tma = (((uintptr_t)c->dPos) & 15) == 0 && !getenv("TDSFS_NO_POS_TMA");
-        q.snap_nearest = getenv("TDSFS_SNAP_BACK") ? 0 : 1;  // A/B knob
-        // ring depth: as many stages per warp as asked for and as fit beside the histograms and the window tables
-        const int per_warp_fixed = q.tab_words * 4;
-        while (depth > 1 && p.cwarps * (depth * (stage_stride + 8) + per_warp_fixed) + hist_words * 4 + 16 > smem_max) --depth;
-        p.nstage = p.cwarps * depth;
-        const int smem = p.nstage * stage_stride + p.cwarps * q.tab_words * 4 + ((p.nstage + 1) & ~1) * 8 + hist_words * 4;
-        if (smem > smem_max) return fail(TDSFS_ERR_ARG, "count kernel geometry needs %d bytes of shared memory (warps %d, depth %d)", smem, p.cwarps, depth);
-        // PLAIN instantiation: every per-SNP branch that cannot trigger in the common configuration compiled out
-        const bool plain = !c->dFlags && c->nfix == 0 && p.bg_group == nullptr && p.bg_lo < 0 && c->fold && c->fmt.narrow &&
-                           c->n1 >= 32 && c->n2 >= 32 && c->n1 <= 1023 && c->n2 <= 1023 && !getenv("TDSFS_NO_PLAIN");
-        void (*kern)(FusedParams) = plain ? k1_fused<0, 0, true> : k1_fused<0, 0, false>;
-        if (plain && c->W1 == 32 && c->W2 == 32) kern = k1_fused<32, 32, true>;        // 500 + 500 diploids (BASELINE config 5)
-        else if (plain && c->W1 == 14 && c->W2 == 14) kern = k1_fused<14, 14, true>;   // 200 + 200 diploids (BASELINE config 4)
-        CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        // Tail of the launch: a pass that is ONE launch over resident data (the usual case) also builds the ln tables of its
-        // background after a grid-wide barrier - and, inside tdsfs_step_bp with the peer exchange mapped, exchanges the
-        // histogram with the other ranks first - instead of leaving that to separate launches.
-        const bool one_launch = c->chunks.size() == 1 && !c->chunks[0].ev && c->chunks[0].r1 > c->chunks[0].r0;
-        const bool tail_x = c->want_tail_exchange && one_launch && mode != TDSFS_BG_NONE && NG == 1 && c->peer_ready &&
-                            c->d_hist == c->peer_exported_hist && c->gstride == c->peer_words;
-        // (measured: without an exchange the tail only matches the separate finalize launch of a replayed graph - off unless TDSFS_TAIL=1)
-        const bool tail_fin = one_launch && mode != TDSFS_BG_NONE && !getenv("TDSFS_NO_TAIL") &&
-                              (tail_x || (!c->want_tail_exchange && getenv("TDSFS_TAIL") != nullptr));
-        if (tail_fin) {
-          CKR(ensure_tables(c, NG));
-          q.tail = tail_x ? 2 : 1;
-          q.gridbar = c->d_gridbar;
-          q.tail_timeout = PEER_TIMEOUT_CYCLES;
-          q.stamps = c->d_stamps;
-          FinParams& f = q.fin;
-          f.hist = c->d_hist; f.gstride = c->gstride; f.NG = NG; f.bins2d = c->bins2d; f.R1 = c->R1; f.R2 = c->R2;
-          f.n1 = c->n1; f.n2 = c->n2; f.lb2 = c->d_lb2; f.lb1a = c->d_lb1a; f.lb1b = c->d_lb1b; f.Bsum = c->d_Bsum; f.B = c->d_B;
-          if (tail_x) {
-            for (int r = 0; r < PEER_MAX; ++r) { q.peer.hist[r] = c->peer_hist[r]; q.peer.flags[r] = c->peer_flags[r]; }
-            q.peer.rank = c->peer_rank; q.peer.world = c->peer_world; q.peer.words = c->peer_words; q.peer.err = c->d_err;
-            q.peer.timeout_cycles = PEER_TIMEOUT_CYCLES;
-            q.peer.ticket = reinterpret_cast<unsigned int*>(c->d_peer_flags + PEER_MAX);
-            q.epoch_mem = c->d_peer_flags + PEER_MAX + 1;
-            c->peer_epoch += 2;  // host mirror of the device epoch
-          }
-        }
-        const long long tile_rows = (long long)p.tile_blocks * BLK;
-        for (auto& ch : c->chunks) {
-          if (ch.r1 <= ch.r0) continue;
-          if (ch.ev) CK(cudaStreamWaitEvent(st, ch.ev, 0));
-          p.r0 = ch.r0; p.r1 = ch.r1;
-          const long long ntiles = (ch.r1 - ch.r0 + tile_rows - 1) / tile_rows;
-          const int grid = (int)std::max<long long>(1, std::min<long long>((ntiles + p.cwarps - 1) / p.cwarps, (long long)c->sm_count));
-          q.k = p;
-          kern<<<grid, p.cwarps * 32, smem, st>>>(q);
-          c->launches++;
-        }
-        if (fuse) {
-          c->fused_W = c->plan_W;
-          c->fused_snp = c->plan_snp;
-          c->ws_ready = true;
-        }
-        if (tail_fin) {
-          c->tables_ready = true;
-          c->tables_from_exchange = true;
-          c->fin_timed = false;
-        }
+        q.nw1 = q.nw2 = 0;
+      }
+      q.pos_tma = (((uintptr_t)c->dPos) & 15) == 0 && !getenv("TDSFS_NO_POS_TMA");
+      // ring depth: as many stages per warp as asked for and as fit beside the histograms and the window tables
+      const int per_warp_fixed = q.tab_words * 4;
+      while (depth > 1 && p.cwarps * (depth * (stage_stride + 8) + per_warp_fixed) + hist_words * 4 + 16 > smem_max) --depth;
+      p.nstage = p.cwarps * depth;
+      const int smem = p.nstage * stage_stride + p.cwarps * q.tab_words * 4 + ((p.nstage + 1) & ~1) * 8 + hist_words * 4;
+      if (smem > smem_max) return fail(TDSFS_ERR_ARG, "count kernel geometry needs %d bytes of shared memory (warps %d, depth %d)", smem, p.cwarps, depth);
+      // PLAIN instantiation: every per-SNP branch that cannot trigger in the common configuration compiled out
+      const bool plain = !c->dFlags && c->nfix == 0 && p.bg_group == nullptr && p.bg_lo < 0 && c->fold && c->fmt.narrow &&
+                         c->n1 >= 32 && c->n2 >= 32 && c->n1 <= 1023 && c->n2 <= 1023;
+      void (*kern)(FusedParams) = plain ? k1_fused<0, 0, true> : k1_fused<0, 0, false>;
+      if (plain && c->W1 == 32 && c->W2 == 32) kern = k1_fused<32, 32, true>;        // 500 + 500 diploids (BASELINE config 5)
+      else if (plain && c->W1 == 14 && c->W2 == 14) kern = k1_fused<14, 14, true>;   // 200 + 200 diploids (BASELINE config 4)
+      CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+      // Tail of the launch: inside tdsfs_step_bp with the peer exchange mapped, a pass that is ONE launch over resident data (the
+      // usual case) exchanges the histogram with the other ranks after a grid-wide barrier and builds the ln tables of the
+      // background, instead of leaving that to a separate launch.  (Measured: without an exchange, ln tables in the tail only
+      // match the separate finalize launch of a replayed graph.)
+      const bool one_launch = c->chunks.size() == 1 && !c->chunks[0].ev && c->chunks[0].r1 > c->chunks[0].r0;
+      const bool tail = c->want_tail_exchange && one_launch && mode != TDSFS_BG_NONE && NG == 1 && c->peer_ready &&
+                        c->d_hist == c->peer_exported_hist && c->gstride == c->peer_words;
+      if (tail) {
+        CKR(ensure_tables(c, NG));
+        q.tail = 1;
+        q.gridbar = c->d_gridbar;
+        q.tail_timeout = PEER_TIMEOUT_CYCLES;
+        q.stamps = c->d_stamps;
+        FinParams& f = q.fin;
+        f.hist = c->d_hist; f.gstride = c->gstride; f.NG = NG; f.bins2d = c->bins2d; f.R1 = c->R1; f.R2 = c->R2;
+        f.n1 = c->n1; f.n2 = c->n2; f.lb2 = c->d_lb2; f.lb1a = c->d_lb1a; f.lb1b = c->d_lb1b; f.Bsum = c->d_Bsum; f.B = c->d_B;
+        for (int r = 0; r < PEER_MAX; ++r) { q.peer.hist[r] = c->peer_hist[r]; q.peer.flags[r] = c->peer_flags[r]; }
+        q.peer.rank = c->peer_rank; q.peer.world = c->peer_world; q.peer.words = c->peer_words; q.peer.err = c->d_err;
+        q.peer.timeout_cycles = PEER_TIMEOUT_CYCLES;
+        q.peer.ticket = reinterpret_cast<unsigned int*>(c->d_peer_flags + PEER_MAX);
+        q.epoch_mem = c->d_peer_flags + PEER_MAX + 1;
+      }
+      const long long tile_rows = (long long)p.tile_blocks * BLK;
+      for (auto& ch : c->chunks) {
+        if (ch.r1 <= ch.r0) continue;
+        if (ch.ev) CK(cudaStreamWaitEvent(st, ch.ev, 0));
+        p.r0 = ch.r0; p.r1 = ch.r1;
+        const long long ntiles = (ch.r1 - ch.r0 + tile_rows - 1) / tile_rows;
+        const int grid = (int)std::max<long long>(1, std::min<long long>((ntiles + p.cwarps - 1) / p.cwarps, (long long)c->sm_count));
+        q.k = p;
+        kern<<<grid, p.cwarps * 32, smem, st>>>(q);
+        c->launches++;
+      }
+      if (fuse) {
+        c->fused_W = c->plan_W;
+        c->fused_snp = c->plan_snp;
+        c->ws_ready = true;
+      }
+      if (tail) {
+        c->tables_ready = true;
+        c->tables_from_exchange = true;
+        c->fin_timed = false;
       }
     }
   } else {
@@ -839,7 +803,6 @@ extern "C" int tdsfs_background(tdsfs_t* c, int32_t mode, int32_t bg_chrom, int6
 extern "C" int tdsfs_background_device(tdsfs_t* c, void** dev_ptr, int64_t* n_words, int32_t* n_groups) {
   if (!c || !c->keys_ready) return fail(TDSFS_ERR_STATE, "tdsfs_background first");
   CK(cudaSetDevice(c->device));
-  CKR(peer_settle(c));
   c->tables_ready = c->float_bg;  // the caller is about to change the histogram (all-reduce): integer tables are rebuilt by finalize
   c->tables_from_exchange = false;
   if (dev_ptr) *dev_ptr = c->d_hist;
@@ -857,18 +820,6 @@ struct PeerBlob {  // TDSFS_PEER_BLOB_BYTES
 };
 static_assert(sizeof(PeerBlob) <= TDSFS_PEER_BLOB_BYTES, "blob size");
 
-
-
-// Something other than the finalize kernel is about to touch the histogram: wait (on the stream) for the peers' pushes.
-static int peer_settle(tdsfs_ctx* c) {
-  if (!c->peer_pending) return 0;
-  k_peer_wait<<<1, 32, 0, c->stream>>>(c->d_peer_flags, c->peer_world, c->peer_pending, c->d_err, PEER_TIMEOUT_CYCLES);
-  c->launches++;
-  c->peer_pending = 0;
-  CK(cudaGetLastError());
-  return 0;
-}
-
 static void peer_unmap(tdsfs_ctx* c) {
   drop_step_graph(c);
   for (int r = 0; r < c->peer_world; ++r) {
@@ -880,7 +831,6 @@ static void peer_unmap(tdsfs_ctx* c) {
     c->peer_flags[r] = nullptr;
   }
   c->peer_ready = false;
-  c->peer_pending = 0;
 }
 
 extern "C" int tdsfs_peer_export(tdsfs_t* c, int32_t rank, int32_t world, void* blob) {
@@ -893,8 +843,6 @@ extern "C" int tdsfs_peer_export(tdsfs_t* c, int32_t rank, int32_t world, void* 
   peer_unmap(c);
   if (!c->d_peer_flags) CKR(dev_alloc(&c->d_peer_flags, PEER_MAX + 2));  // flags, the reduce kernel's CTA counter, the epoch
   CK(cudaMemset(c->d_peer_flags, 0, (PEER_MAX + 2) * sizeof(unsigned long long)));
-  c->peer_pending = 0;
-  c->peer_epoch = 0;
   c->peer_rank = rank;
   c->peer_world = world;
   c->peer_words = c->gstride;
@@ -940,41 +888,8 @@ extern "C" int tdsfs_peer_import(tdsfs_t* c, const void* blobs) {
   return 0;
 }
 
-extern "C" int tdsfs_peer_allreduce_background(tdsfs_t* c) {
-  if (!c || !c->peer_ready) return fail(TDSFS_ERR_STATE, "tdsfs_peer_export / tdsfs_peer_import first");
-  if (!c->keys_ready) return fail(TDSFS_ERR_STATE, "tdsfs_background first");
-  if (c->d_hist != c->peer_exported_hist || c->NG != 1 || c->gstride != c->peer_words)
-    return fail(TDSFS_ERR_STATE, "the histogram changed since tdsfs_peer_export (panel or background mode): export again");
-  CK(cudaSetDevice(c->device));
-  NvtxRange nvtx("tdsfs:exchange (peer all-reduce of the background)");
-  cudaStream_t st = c->stream;
-  PeerParams p;
-  for (int r = 0; r < PEER_MAX; ++r) { p.hist[r] = c->peer_hist[r]; p.flags[r] = c->peer_flags[r]; }
-  p.rank = c->peer_rank; p.world = c->peer_world; p.words = c->peer_words; p.err = c->d_err;
-  p.timeout_cycles = PEER_TIMEOUT_CYCLES;
-  // one launch: barrier (every rank's count kernel has finished) -> pull / sum / push slice `rank` -> signal; the
-  // wait for everybody's signal is the head of tdsfs_finalize_background's kernel (or peer_settle)
-  CKR(peer_settle(c));
-  p.epoch = c->peer_epoch + 1;
-  c->peer_epoch += 2;
-  p.ticket = reinterpret_cast<unsigned int*>(c->d_peer_flags + PEER_MAX);
-  p.epoch_mem = c->d_peer_flags + PEER_MAX + 1;
-  const long long n4 = p.words / 4 / p.world + 1;
-  const int grid = (int)std::max<long long>(1, std::min<long long>((n4 + 255) / 256, (long long)c->sm_count));
-  CK(cudaEventRecord(c->ev[EV_X0], st));
-  k_peer_reduce<<<grid, 256, 0, st>>>(p);
-  CK(cudaEventRecord(c->ev[EV_X1], st));
-  c->x_timed = true;
-  c->launches += 1;
-  c->peer_pending = c->peer_epoch;
-  CK(cudaGetLastError());
-  c->tables_ready = false;
-  c->tables_from_exchange = false;
-  return finish(c);
-}
-
-// All-reduce of the background AND the ln tables in one launch (k_peer_reduce_finalize): replaces the pair
-// tdsfs_peer_allreduce_background + tdsfs_finalize_background (a later tdsfs_finalize_background is then a no-op).
+// All-reduce of the background AND the ln tables in one launch (k_peer_reduce_finalize); a later tdsfs_finalize_background
+// is then a no-op.
 extern "C" int tdsfs_peer_reduce_finalize(tdsfs_t* c) {
   if (!c || !c->peer_ready) return fail(TDSFS_ERR_STATE, "tdsfs_peer_export / tdsfs_peer_import first");
   if (!c->keys_ready) return fail(TDSFS_ERR_STATE, "tdsfs_background first");
@@ -983,7 +898,6 @@ extern "C" int tdsfs_peer_reduce_finalize(tdsfs_t* c) {
   CK(cudaSetDevice(c->device));
   NvtxRange nvtx("tdsfs:exchange + finalize (one launch)");
   cudaStream_t st = c->stream;
-  CKR(peer_settle(c));
   CKR(ensure_tables(c, 1));
   PeerFinParams q;
   memset(&q, 0, sizeof q);
@@ -992,7 +906,6 @@ extern "C" int tdsfs_peer_reduce_finalize(tdsfs_t* c) {
   q.x.timeout_cycles = PEER_TIMEOUT_CYCLES;
   q.x.ticket = reinterpret_cast<unsigned int*>(c->d_peer_flags + PEER_MAX);
   q.epoch_mem = c->d_peer_flags + PEER_MAX + 1;
-  c->peer_epoch += 2;  // host mirror of the device epoch (the split path passes it as an argument)
   FinParams& f = q.f;
   f.hist = c->d_hist; f.gstride = c->gstride; f.NG = 1; f.bins2d = c->bins2d; f.R1 = c->R1; f.R2 = c->R2;
   f.n1 = c->n1; f.n2 = c->n2; f.lb2 = c->d_lb2; f.lb1a = c->d_lb1a; f.lb1b = c->d_lb1b; f.Bsum = c->d_Bsum; f.B = c->d_B;
@@ -1010,10 +923,12 @@ extern "C" int tdsfs_peer_reduce_finalize(tdsfs_t* c) {
   return finish(c);
 }
 
+// the exchange always builds the ln tables in the same launch (include/tdsfs.h)
+extern "C" int tdsfs_peer_allreduce_background(tdsfs_t* c) { return tdsfs_peer_reduce_finalize(c); }
+
 extern "C" int tdsfs_peer_close(tdsfs_t* c) {
   if (!c) return fail(TDSFS_ERR_ARG, "ctx is NULL");
   CK(cudaSetDevice(c->device));
-  CKR(peer_settle(c));
   CK(cudaStreamSynchronize(c->stream));
   peer_unmap(c);
   c->peer_exported_hist = nullptr;
@@ -1026,7 +941,6 @@ extern "C" int tdsfs_get_background(tdsfs_t* c, int32_t group, uint64_t* s2, uin
   if (!c || !c->keys_ready) return fail(TDSFS_ERR_STATE, "tdsfs_background first");
   if (group < 0 || group >= c->NG) return fail(TDSFS_ERR_ARG, "group %d out of range", group);
   CK(cudaSetDevice(c->device));
-  CKR(peer_settle(c));
   std::vector<uint32_t> h((size_t)c->gstride);
   CK(cudaMemcpyAsync(h.data(), c->d_hist + (long long)group * c->gstride, (size_t)c->gstride * 4, cudaMemcpyDeviceToHost, c->stream));
   CK(cudaStreamSynchronize(c->stream));
@@ -1113,11 +1027,6 @@ extern "C" int tdsfs_finalize_background(tdsfs_t* c) {
   memset(&f, 0, sizeof f);
   f.hist = c->d_hist; f.gstride = c->gstride; f.NG = c->NG; f.bins2d = c->bins2d; f.R1 = c->R1; f.R2 = c->R2;
   f.n1 = c->n1; f.n2 = c->n2; f.lb2 = c->d_lb2; f.lb1a = c->d_lb1a; f.lb1b = c->d_lb1b; f.Bsum = c->d_Bsum; f.B = c->d_B;
-  if (c->peer_pending) {  // the kernel itself waits for the peers' pushes into this rank's histogram
-    f.wait_flags = c->d_peer_flags; f.wait_n = c->peer_world; f.wait_epoch = c->peer_pending; f.err = c->d_err;
-    f.timeout_cycles = PEER_TIMEOUT_CYCLES;
-    c->peer_pending = 0;
-  }
   // one bin per thread up to four CTAs per SM (measured: ~8 bins per thread with a smaller grid is slower for the 401 x 401 spectrum)
   dim3 grid((unsigned)std::max(1, std::min(c->sm_count * 4, (c->bins2d + 255) / 256)), (unsigned)c->NG);
   k_finalize_counts<<<grid, 256, 0, st>>>(f);

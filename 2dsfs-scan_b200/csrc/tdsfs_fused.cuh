@@ -37,9 +37,8 @@ struct FusedParams {
   int pos_tma;                // the tile's positions ride the TMA ring (16-byte aligned position array)
   int tab_words;              // per-warp window tables: HASH_SLOTS + packed 1D words, a multiple of 4
   int nw1, nw2;               // packed 1D words per population: (n + 2) / 2
-  int snap_nearest;           // range boundaries snap to the nearest window start (0: back to the start of the window that holds them)
-  // tail of the launch (single-launch passes only): after a grid-wide barrier the resident CTAs build the ln tables of the
-  // background themselves (1), after exchanging it with the other ranks through peer memory (2): no separate launches
+  // tail of the launch (single-launch passes with the peer exchange mapped): after a grid-wide barrier the resident CTAs
+  // exchange the background with the other ranks through peer memory and build its ln tables: no separate launches
   int tail;
   unsigned int* gridbar;
   long long tail_timeout;
@@ -115,7 +114,8 @@ __device__ __forceinline__ int next_window_start(const FusedParams& q, int t, in
 // Snap a range boundary `t` (a tile-aligned row) to the nearest window start, so that no window of at most WCAP SNPs is split
 // between two warps (warp-cooperative: all lanes call, all return the same value; monotone in t).  Nearest rather than
 // "back to the start of the window that holds t": the ranges of a small shard are only a few windows long, and their
-// lengths then differ by at most one window instead of two.
+// lengths then differ by at most one window instead of two.  nearest = false snaps back instead: the two ends of a launch,
+// because rows past the end may still be uploading.
 // is_start = the returned row starts a window (or lies in none); false when the window holding t began more than WCAP rows
 // earlier (such a window is larger than the warp tables: nobody sums it here, the CTA path scores it).
 __device__ __forceinline__ int snap_row(const FusedParams& q, int t, bool& is_start, int lane, bool nearest) {
@@ -290,14 +290,14 @@ __global__ void __launch_bounds__(k1f_max_warps<TW1, TW2>() * 32, 1) k1_fused(co
     const int hi_clamp = r1 < S ? snap_row(q, r1, sth, lane, false) : S;
     int slo = lo_clamp, shi = hi_clamp;
     if (j > 0) {
-      slo = snap_row(q, target(j), st0, lane, q.snap_nearest != 0);
+      slo = snap_row(q, target(j), st0, lane, true);
       if (slo <= lo_clamp) { slo = lo_clamp; st0 = stl; }
       if (slo >= hi_clamp) { slo = hi_clamp; st0 = sth; }
     } else {
       st0 = stl;
     }
     if (j + 1 < nparts) {
-      shi = snap_row(q, target(j + 1), st1, lane, q.snap_nearest != 0);
+      shi = snap_row(q, target(j + 1), st1, lane, true);
       if (shi <= lo_clamp) shi = lo_clamp;
       if (shi >= hi_clamp) shi = hi_clamp;
     }
@@ -576,7 +576,7 @@ __global__ void __launch_bounds__(k1f_max_warps<TW1, TW2>() * 32, 1) k1_fused(co
     stamp(1);
     grid_barrier(q.gridbar, p.err, q.tail_timeout);  // every CTA's private histograms are in the global histogram
     stamp(2);
-    if (q.tail == 2) peer_exchange(q.peer, q.epoch_mem, q.stamps);
+    peer_exchange(q.peer, q.epoch_mem, q.stamps);
     for (int g = 0; g < q.fin.NG; ++g) finalize_tables(q.fin, g, blockIdx.x, gridDim.x);
     stamp(6);
     finalize_totals(q.fin, gridDim.x);

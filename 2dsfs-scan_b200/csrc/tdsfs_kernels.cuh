@@ -66,9 +66,6 @@ struct KeyParams {
   int nstage, stage_bytes;  // K1 ring: stages of `tile_blocks` 32-SNP blocks; nstage is a multiple of cwarps
   int tile_blocks;
   int cwarps;               // active consumer warps (<= K1_CWARPS)
-  int debug;                // profiling only (TDSFS_K1_DEBUG): bit 0 = no record store, bit 1 = no histogram updates
-  int interleave;           // 1: tile i of the launch goes to CTA i % grid (all SMs stream one moving window of the matrix);
-                            // 0: contiguous tile range per CTA (keeps a CTA inside one background group)
 };
 
 // ------------------------------------------------------------------------------------------------ PTX helpers
@@ -210,41 +207,6 @@ __device__ __forceinline__ void count_block_b32(const uint32_t* blk, int Wrt, ui
   M = pc.miss.total();
 }
 
-// Both population blocks of one SNP at once (same word count): four independent carry-save chains (bits/missing x 2
-// populations) instead of two -- the count kernel is bound by dependent LOP3 latency with ~3 warps per scheduler.
-template <int TW>
-__device__ __forceinline__ void count_two_blocks_b32(const uint32_t* blk1, const uint32_t* blk2, uint32_t& T1, uint32_t& M1,
-                                                     uint32_t& T2, uint32_t& M2) {
-  PopCounts p1, p2;
-  int w = 0;
-#pragma unroll
-  for (; w + 8 <= TW; w += 8) {
-    const uint32_t* q1 = blk1 + w * BLK;
-    const uint32_t* q2 = blk2 + w * BLK;
-    uint4 a1 = make_uint4(q1[0], q1[BLK], q1[2 * BLK], q1[3 * BLK]);
-    uint4 a2 = make_uint4(q2[0], q2[BLK], q2[2 * BLK], q2[3 * BLK]);
-    uint4 b1 = make_uint4(q1[4 * BLK], q1[5 * BLK], q1[6 * BLK], q1[7 * BLK]);
-    uint4 b2 = make_uint4(q2[4 * BLK], q2[5 * BLK], q2[6 * BLK], q2[7 * BLK]);
-    p1.chunk8(a1, b1);
-    p2.chunk8(a2, b2);
-  }
-  if (w + 4 <= TW) {
-    const uint32_t* q1 = blk1 + w * BLK;
-    const uint32_t* q2 = blk2 + w * BLK;
-    p1.chunk4(q1[0], q1[BLK], q1[2 * BLK], q1[3 * BLK]);
-    p2.chunk4(q2[0], q2[BLK], q2[2 * BLK], q2[3 * BLK]);
-    w += 4;
-  }
-  if (w < TW) {
-    const uint32_t* q1 = blk1 + w * BLK;
-    const uint32_t* q2 = blk2 + w * BLK;
-    p1.chunk4(q1[0], (w + 1 < TW) ? q1[BLK] : 0u, (w + 2 < TW) ? q1[2 * BLK] : 0u, 0u);
-    p2.chunk4(q2[0], (w + 1 < TW) ? q2[BLK] : 0u, (w + 2 < TW) ? q2[2 * BLK] : 0u, 0u);
-  }
-  T1 = p1.bits.total(); M1 = p1.miss.total();
-  T2 = p2.bits.total(); M2 = p2.miss.total();
-}
-
 // ------------------------------------------------------------------------------------------------ row sink
 // Shared-memory privatised background histograms of ONE background group per CTA.
 struct SinkSmem {
@@ -348,8 +310,7 @@ __device__ __forceinline__ uint2 sink_row(const KeyParams& p, long long s, int r
         nrec = (uint32_t)k1 | ((uint32_t)k2 << p.fmt.b1) | ((uint32_t)d1 << (p.fmt.b1 + p.fmt.b2)) |
                ((uint32_t)d2 << (p.fmt.b1 + p.fmt.b2 + p.fmt.md));
       }
-      int g = group_of_row(p, s, cc);
-      if (p.debug & 2) g = -1;
+      const int g = group_of_row(p, s, cc);
       if (g >= 0) {
         uint32_t* gh = p.hist + (long long)g * p.gstride;
         if (key) {
@@ -367,10 +328,9 @@ __device__ __forceinline__ uint2 sink_row(const KeyParams& p, long long s, int r
       }
     }
   }
-  if (!(p.debug & 1)) {  // streaming store: read once by the scorer, from L2 or HBM
-    if (p.fmt.narrow) __stcs(reinterpret_cast<uint32_t*>(p.rec) + s, nrec);
-    else __stcs(reinterpret_cast<uint2*>(p.rec) + s, make_uint2(key, alts));
-  }
+  // streaming store: read once by the scorer, from L2 or HBM
+  if (p.fmt.narrow) __stcs(reinterpret_cast<uint32_t*>(p.rec) + s, nrec);
+  else __stcs(reinterpret_cast<uint2*>(p.rec) + s, make_uint2(key, alts));
   return make_uint2(key, alts);
 }
 
@@ -401,158 +361,9 @@ __device__ __forceinline__ int tile_group(const KeyParams& p, long long row0, Ch
 }
 
 // ------------------------------------------------------------------------------------------------ K1 (genotypes)
-// One persistent CTA per SM, 12 warps, no producer warp: every warp runs its OWN ring of `depth` TMA stages
-// (cp.async.bulk + one mbarrier per stage).  Tile i of the CTA (tile_blocks 32-SNP blocks, contiguous in the B32 layout)
-// belongs to warp i % cwarps; after counting a tile the warp's lane 0 refills the stage it just drained, so stages are
-// never blocked behind another warp.  Each lane owns one SNP of a block: bit-sliced popcount of its two population
-// blocks straight from shared memory (word w at +128 B: bank = lane), fold/key, one coalesced 8-byte record store,
-// privatised background histograms.
-template <int TW1, int TW2>
-__global__ void __launch_bounds__(K1_THREADS, 1) k1_genotypes(const __grid_constant__ KeyParams p) {
-  extern __shared__ __align__(128) uint8_t smem[];
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int W1 = TW1 > 0 ? TW1 : p.W1, W2 = TW2 > 0 ? TW2 : p.W2;
-  const int RW = W1 + W2;
-  uint8_t* stages = smem;
-  uint64_t* full = reinterpret_cast<uint64_t*>(smem + (size_t)p.nstage * p.stage_bytes);
-  SinkSmem sm;
-  sm.corner = reinterpret_cast<uint32_t*>(full + p.nstage);
-  sm.h1a = sm.corner + p.cr * p.cc;
-  sm.h1b = sm.h1a + p.h1a;
-  const int nhist = p.cr * p.cc + p.h1a + p.h1b;
-
-  if (tid == 0) {
-    for (int i = 0; i < p.nstage; ++i) mbar_init(full + i, 1);
-    fence_barrier_init();
-  }
-  for (int i = tid; i < nhist; i += blockDim.x) sm.corner[i] = 0;
-  __syncthreads();
-
-  // contiguous range of tiles of this CTA; a tile = tile_blocks blocks of 32 SNPs
-  const long long b0 = p.r0 / BLK, b1 = (p.r1 + BLK - 1) / BLK;  // r0 is a multiple of BLK
-  const long long ntiles = (b1 - b0 + p.tile_blocks - 1) / p.tile_blocks;
-  // tile `i` (local index) of this CTA is global tile t0 + i * tstride
-  const long long t0 = p.interleave ? blockIdx.x : ntiles * blockIdx.x / gridDim.x;
-  const long long tstride = p.interleave ? gridDim.x : 1;
-  const long long n = p.interleave ? (ntiles > blockIdx.x ? (ntiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0)
-                                   : ntiles * (blockIdx.x + 1) / gridDim.x - t0;
-  const long long block_words = (long long)RW * BLK;
-  const int depth = p.nstage / p.cwarps;  // stages per warp
-
-  ChromCache cc;
-  const int cta_group = (n > 0) ? tile_group(p, p.r0 + t0 * p.tile_blocks * BLK, cc) : -1;
-  if (warp < p.cwarps) {
-    uint8_t* my_stages = stages + (size_t)warp * depth * p.stage_bytes;
-    uint64_t* my_full = full + warp * depth;
-    auto issue = [&](long long i, int slot) {  // lane 0 only
-      const long long blk0 = b0 + (t0 + i * tstride) * p.tile_blocks;
-      const uint32_t bytes = (uint32_t)(min((long long)p.tile_blocks, b1 - blk0) * block_words * 4);
-      mbar_arrive_expect_tx(my_full + slot, bytes);
-      bulk_g2s_stream(my_stages + (size_t)slot * p.stage_bytes, p.G + blk0 * block_words, bytes, my_full + slot);
-    };
-    if (lane == 0)
-      for (int j = 0; j < depth; ++j)
-        if (warp + (long long)j * p.cwarps < n) issue(warp + (long long)j * p.cwarps, j);
-    int slot = 0;
-    uint32_t ph = 0;
-    for (long long i = warp; i < n; i += p.cwarps) {
-      const long long blk0 = b0 + (t0 + i * tstride) * p.tile_blocks;
-      const int nb = (int)min((long long)p.tile_blocks, b1 - blk0);
-      mbar_wait(my_full + slot, ph);
-      const uint32_t* tile = reinterpret_cast<const uint32_t*>(my_stages + (size_t)slot * p.stage_bytes);
-      for (int b = 0; b < nb; ++b) {
-        const long long s = (blk0 + b) * BLK + lane;
-        uint32_t T1 = 0, M1 = 0, T2 = 0, M2 = 0;
-        if (s < p.r1) {
-          const uint32_t* rowp = tile + (size_t)b * block_words + lane;
-          if (TW1 > 0 && TW1 == TW2) {
-            count_two_blocks_b32<TW1>(rowp, rowp + W1 * BLK, T1, M1, T2, M2);
-          } else {
-            count_block_b32<TW1>(rowp, W1, T1, M1);
-            count_block_b32<TW2>(rowp + W1 * BLK, W2, T2, M2);
-          }
-        }
-        if (b == nb - 1) {
-          // the stage has been read completely: refill it BEFORE the fold / record / histogram work of its last block,
-          // so that work overlaps the next load instead of delaying it
-          __syncwarp();
-          if (lane == 0) {
-            const long long nxt = i + (long long)depth * p.cwarps;
-            if (nxt < n) {
-              fence_proxy_async();  // order this warp's generic-proxy reads of the stage before the async-proxy refill
-              issue(nxt, slot);
-            }
-          }
-        }
-        if (s < p.r1) {
-          const int alt1 = (int)(T1 - M1), alt2 = (int)(T2 - M2);
-          const int ref1 = 2 * (p.ns1 - (int)M1) - alt1, ref2 = 2 * (p.ns2 - (int)M2) - alt2;
-          sink_row(p, s, ref1, alt1, ref2, alt2, cta_group, sm, cc);
-        }
-      }
-      if (++slot == depth) { slot = 0; ph ^= 1; }
-    }
-  }
-  __syncthreads();
-  sink_flush(p, sm, cta_group, tid, blockDim.x);
-}
-
-// Bandwidth probe (TDSFS_K1_PROBE=1, profiling only - produces no spectra): the ring traffic of k1_genotypes without the
-// counting, i.e. the ceiling of this access pattern.  Each lane folds one word per block into a checksum so the loads stay.
-__global__ void __launch_bounds__(K1_THREADS, 1) k1_probe_ring(const __grid_constant__ KeyParams p) {
-  extern __shared__ __align__(128) uint8_t smem[];
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int RW = p.W1 + p.W2;
-  uint8_t* stages = smem;
-  uint64_t* full = reinterpret_cast<uint64_t*>(smem + (size_t)p.nstage * p.stage_bytes);
-  if (tid == 0) {
-    for (int i = 0; i < p.nstage; ++i) mbar_init(full + i, 1);
-    fence_barrier_init();
-  }
-  __syncthreads();
-  const long long b0 = p.r0 / BLK, b1 = (p.r1 + BLK - 1) / BLK;
-  const long long ntiles = (b1 - b0 + p.tile_blocks - 1) / p.tile_blocks;
-  const long long t0 = p.interleave ? blockIdx.x : ntiles * blockIdx.x / gridDim.x;
-  const long long tstride = p.interleave ? gridDim.x : 1;
-  const long long n = p.interleave ? (ntiles > blockIdx.x ? (ntiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0)
-                                   : ntiles * (blockIdx.x + 1) / gridDim.x - t0;
-  const long long block_words = (long long)RW * BLK;
-  const int depth = p.nstage / p.cwarps;
-  uint32_t sum = 0;
-  if (warp < p.cwarps) {
-    uint8_t* my_stages = stages + (size_t)warp * depth * p.stage_bytes;
-    uint64_t* my_full = full + warp * depth;
-    auto issue = [&](long long i, int slot) {
-      const long long blk0 = b0 + (t0 + i * tstride) * p.tile_blocks;
-      const uint32_t bytes = (uint32_t)(min((long long)p.tile_blocks, b1 - blk0) * block_words * 4);
-      mbar_arrive_expect_tx(my_full + slot, bytes);
-      bulk_g2s_stream(my_stages + (size_t)slot * p.stage_bytes, p.G + blk0 * block_words, bytes, my_full + slot);
-    };
-    if (lane == 0)
-      for (int j = 0; j < depth; ++j)
-        if (warp + (long long)j * p.cwarps < n) issue(warp + (long long)j * p.cwarps, j);
-    int slot = 0;
-    uint32_t ph = 0;
-    for (long long i = warp; i < n; i += p.cwarps) {
-      mbar_wait(my_full + slot, ph);
-      sum += reinterpret_cast<const uint32_t*>(my_stages + (size_t)slot * p.stage_bytes)[lane];
-      __syncwarp();
-      if (lane == 0) {
-        const long long nxt = i + (long long)depth * p.cwarps;
-        if (nxt < n) {
-          fence_proxy_async();
-          issue(nxt, slot);
-        }
-      }
-      if (++slot == depth) { slot = 0; ph ^= 1; }
-    }
-  }
-  if (sum == 0xFFFFFFFFu) p.hist[0] = sum;  // keeps the loads alive
-}
-
-// K1 for rows wider than one ring stage (more than 4096 samples): a 32-SNP block is streamed as segments of `seg_words`
-// words (contiguous in the B32 layout); the warp carries its bit-sliced counters across the segments of a block and
-// sinks the SNPs after the last one.  Generic (runtime) geometry: the population of a word is decided per segment piece.
+// K1 for rows wider than one stage of k1_fused's ring (more than 4096 samples): a 32-SNP block is streamed as segments of
+// `seg_words` words (contiguous in the B32 layout); the warp carries its bit-sliced counters across the segments of a block
+// and sinks the SNPs after the last one.  Generic (runtime) geometry: the population of a word is decided per segment piece.
 __global__ void __launch_bounds__(K1_THREADS, 1) k1_genotypes_wide(const __grid_constant__ KeyParams p, int seg_words) {
   extern __shared__ __align__(128) uint8_t smem[];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -642,11 +453,9 @@ struct PeerParams {
   unsigned long long* flags[PEER_MAX];
   int rank, world;
   long long words;
-  unsigned long long epoch;  // barrier 1 = epoch, barrier 2 = epoch + 1
   int* err;
   long long timeout_cycles;
-  unsigned int* ticket;      // CTA arrival counter of k_peer_reduce (reset by its last CTA)
-  unsigned long long* epoch_mem;  // device copy of the last epoch used (read by k_peer_reduce_finalize)
+  unsigned int* ticket;      // CTA arrival counter of peer_exchange (reset by its last CTA)
 };
 
 __device__ __forceinline__ void st_release_sys(unsigned long long* p, unsigned long long v) {
@@ -665,65 +474,6 @@ __device__ __forceinline__ void peer_wait(const unsigned long long* flag, unsign
     if (clock64() - t0 > timeout_cycles) {
       atomicOr(err, 4);
       break;
-    }
-  }
-}
-
-// wait-only barrier (used when something other than the finalize kernel consumes the reduced histogram)
-__global__ void k_peer_wait(const unsigned long long* flags, int world, unsigned long long epoch, int* err, long long timeout_cycles) {
-  if ((int)threadIdx.x < world) peer_wait(flags + threadIdx.x, epoch, err, timeout_cycles);
-}
-
-// One launch per rank: [barrier 1: signal "my count kernel is done" (block 0), wait for every rank's signal (all blocks)]
-// -> pull slice `rank` of every histogram, sum, push the sum into every histogram -> [signal "my pushes have landed"
-// (last block)].  The matching wait is at the head of the consumer (k_finalize_counts / k_peer_wait).
-__global__ void __launch_bounds__(256) k_peer_reduce(const __grid_constant__ PeerParams p) {
-  __shared__ int s_last;
-  if ((int)threadIdx.x < p.world) {
-    if (blockIdx.x == 0) {
-      __threadfence_system();
-      st_release_sys(p.flags[threadIdx.x] + p.rank, p.epoch);
-    }
-    peer_wait(p.flags[p.rank] + threadIdx.x, p.epoch, p.err, p.timeout_cycles);
-  }
-  __syncthreads();
-  const long long n4 = p.words / 4;
-  const long long lo = n4 * p.rank / p.world, hi = n4 * (p.rank + 1) / p.world;
-  for (long long i = lo + (long long)blockIdx.x * blockDim.x + threadIdx.x; i < hi; i += (long long)gridDim.x * blockDim.x) {
-    uint4 v[8];
-#pragma unroll
-    for (int r = 0; r < 8; ++r)
-      if (r < p.world) v[r] = __ldcg(reinterpret_cast<const uint4*>(p.hist[r]) + i);
-    uint4 s = make_uint4(0, 0, 0, 0);
-#pragma unroll
-    for (int r = 0; r < 8; ++r)
-      if (r < p.world) { s.x += v[r].x; s.y += v[r].y; s.z += v[r].z; s.w += v[r].w; }
-    for (int r = 8; r < p.world; ++r) {
-      const uint4 t = __ldcg(reinterpret_cast<const uint4*>(p.hist[r]) + i);
-      s.x += t.x; s.y += t.y; s.z += t.z; s.w += t.w;
-    }
-    for (int r = 0; r < p.world; ++r) __stcg(reinterpret_cast<uint4*>(p.hist[r]) + i, s);
-  }
-  // the last (words % 4) words: one thread of the last rank
-  if (p.rank == p.world - 1 && blockIdx.x == 0 && threadIdx.x == 0)
-    for (long long w = n4 * 4; w < p.words; ++w) {
-      uint32_t s = 0;
-      for (int r = 0; r < p.world; ++r) s += __ldcg(p.hist[r] + w);
-      for (int r = 0; r < p.world; ++r) __stcg(p.hist[r] + w, s);
-    }
-  // every thread's pushes are ordered before the CTA's ticket; the last CTA tells every rank that this rank is done
-  __threadfence_system();
-  __syncthreads();
-  if (threadIdx.x == 0) s_last = atomicAdd(p.ticket, 1u) == gridDim.x - 1;
-  __syncthreads();
-  if (s_last) {
-    if ((int)threadIdx.x < p.world) {
-      __threadfence_system();
-      st_release_sys(p.flags[threadIdx.x] + p.rank, p.epoch + 1);
-    }
-    if (threadIdx.x == 0) {
-      *p.ticket = 0;
-      *p.epoch_mem = p.epoch + 1;
     }
   }
 }
@@ -775,12 +525,6 @@ struct FinParams {
   double* lb1b;  // [NG][n2+1]
   unsigned long long* Bsum;  // [NG][3] interior totals, then one word used as the CTA arrival counter; zero between launches
   double* B;                 // [NG][6] = B (2D, 1D pop1, 1D pop2) then ln B
-  // multi-GPU: wait until every rank's k_peer_reduce has pushed its slice (flags in this rank's memory)
-  const unsigned long long* wait_flags;
-  int wait_n;
-  unsigned long long wait_epoch;
-  int* err;
-  long long timeout_cycles;
 };
 
 __device__ __forceinline__ double ln_count(unsigned long long v) { return v ? log((double)v) : -INFINITY; }
@@ -853,10 +597,6 @@ __device__ __forceinline__ void finalize_totals(const FinParams& p, int ctas_tot
 }
 
 __global__ void __launch_bounds__(256) k_finalize_counts(const __grid_constant__ FinParams p) {
-  if (p.wait_n) {
-    if ((int)threadIdx.x < p.wait_n) peer_wait(p.wait_flags + threadIdx.x, p.wait_epoch, p.err, p.timeout_cycles);
-    __syncthreads();
-  }
   finalize_tables(p, blockIdx.y, blockIdx.x, gridDim.x);
   finalize_totals(p, gridDim.x * gridDim.y);
 }
@@ -875,6 +615,9 @@ struct PeerFinParams {
 // the exchange proper, by every CTA of a launch whose CTAs are all resident (they spin on the flags)
 // `stamps` (diagnostics, normally null): CTA 0 leaves clock64 after barrier 1 [3], after its pushes are fenced [4] and after
 // barrier 2 [5]
+// No wait is needed after the launch: it returns only once every rank has signalled e + 1, and a rank signals only after it
+// has read its slice from every histogram, summed it, pushed the sum and fenced (__threadfence_system).  So when the launch
+// ends no peer still reads or writes this rank's histogram, and the next count kernel may zero and refill it.
 __device__ __forceinline__ void peer_exchange(const PeerParams& p, unsigned long long* epoch_mem, unsigned long long* stamps = nullptr) {
   __shared__ int s_last2;
   auto stamp = [&](int i) { if (stamps && blockIdx.x == 0 && threadIdx.x == 0) stamps[i] = (unsigned long long)clock64(); };

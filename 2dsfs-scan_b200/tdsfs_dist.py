@@ -159,7 +159,7 @@ def check_total_snps(local_snps, group=None):
 
 def peer_setup(handle, group=None):
     """Map every rank's background histogram into every other rank (CUDA IPC over NVLink) for
-    handle.peer_allreduce_background().  Collective; the handle must hold its shard and tdsfs_background must have
+    handle.peer_reduce_finalize().  Collective; the handle must hold its shard and tdsfs_background must have
     run once (single-group mode).  Returns False, leaving the NCCL path in use, when the mapping is not possible."""
     import torch.distributed as dist
     import tdsfs_capi as T
@@ -292,22 +292,3 @@ def sharded_scan(handle, pieces, pos, size, bg_mode, device, *, snp_mode=False, 
         handle.check()  # a late or missing peer must not pass as a result
     return gather_results(localize_results(res, pieces, pos, size, snp_mode), 0, group)
 
-
-def sharded_scan_bp(handle, window_bp, bg_mode, device, group=None, chrom_base=0, peer=False):
-    """Whole-chromosome shards (shard_chromosomes), fixed-bp windows: background -> (all-reduce) -> finalize -> scan ->
-    gather.  Kept for callers that shard by chromosome themselves; sharded_scan handles split chromosomes, fixed-SNP
-    windows and a single-chromosome background."""
-    handle.plan(window_bp)  # window boundaries on a side stream: overlaps the count kernel and the all-reduce
-    handle.background(bg_mode)
-    if bg_mode == BG_GENOME:
-        if peer:
-            handle.peer_allreduce_background()
-        else:
-            allreduce_background(background_tensor(handle, device), group)
-    elif bg_mode == BG_CHROM:
-        raise ValueError("a single-chromosome background needs the chromosome's GLOBAL index: use sharded_scan(bg_chrom=...)")
-    handle.finalize_background()
-    res = handle.scan(window_bp)
-    if hasattr(handle, "check"):
-        handle.check()
-    return gather_results(res, chrom_base, group)

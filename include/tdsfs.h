@@ -142,17 +142,20 @@ int tdsfs_background_device(tdsfs_t* ctx, void** dev_ptr, int64_t* n_words, int3
  *   tdsfs_background(...)                       once, so that the histogram exists (single group: GENOME / CHROM)
  *   tdsfs_peer_export(ctx, rank, world, blob)   fills blob[TDSFS_PEER_BLOB_BYTES]; exchange blobs out of band
  *   tdsfs_peer_import(ctx, blobs)               blobs = world x TDSFS_PEER_BLOB_BYTES in rank order
- *   per scan: tdsfs_background -> tdsfs_peer_allreduce_background -> tdsfs_finalize_background -> tdsfs_scan_*
+ *   per scan: tdsfs_background -> tdsfs_peer_reduce_finalize -> tdsfs_scan_*
  *   tdsfs_peer_close(ctx)                       on every rank BEFORE any rank changes its panel or is destroyed
- * tdsfs_peer_allreduce_background is asynchronous on the handle's stream; all ranks must call it the same number
- * of times.  A rank that never arrives makes the others flag TDSFS_ERR_CUDA (tdsfs_check) after ~60 s (TDSFS_PEER_TIMEOUT_S), not hang. */
+ * The exchange is asynchronous on the handle's stream; all ranks must call it the same number of times.  A rank that
+ * never arrives makes the others flag TDSFS_ERR_CUDA (tdsfs_check) after ~60 s (TDSFS_PEER_TIMEOUT_S), not hang. */
 #define TDSFS_PEER_BLOB_BYTES 192
 #define TDSFS_PEER_MAX_RANKS 16
 int tdsfs_peer_export(tdsfs_t* ctx, int32_t rank, int32_t world, void* blob);
 int tdsfs_peer_import(tdsfs_t* ctx, const void* blobs);
+/* The same call as tdsfs_peer_reduce_finalize: besides the all-reduce it builds the ln tables, so a
+ * tdsfs_finalize_background that follows is a no-op unless tdsfs_background_device was called in between. */
 int tdsfs_peer_allreduce_background(tdsfs_t* ctx);
-/* The same exchange and tdsfs_finalize_background in ONE launch per rank: barrier, pull / sum / push of this rank's slice,
- * barrier, then the ln tables of the complete local histogram.  A tdsfs_finalize_background that follows is a no-op. */
+/* The exchange and tdsfs_finalize_background in ONE launch per rank: barrier, pull / sum / push of this rank's slice,
+ * barrier, then the ln tables of the complete local histogram.  A tdsfs_finalize_background that follows is a no-op
+ * unless tdsfs_background_device was called in between. */
 int tdsfs_peer_reduce_finalize(tdsfs_t* ctx);
 int tdsfs_peer_close(tdsfs_t* ctx);
 

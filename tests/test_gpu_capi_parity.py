@@ -346,8 +346,9 @@ def test_rows_wider_than_one_ring_stage(T, h):
 
 
 def test_peer_exchange_single_rank(T, h):
-    """The peer-memory all-reduce with world = 1 (this rank maps only itself): barrier epochs, in-place reduce and the
-    finalize kernel's wait all run, and the scan equals the plain one.  Two ranks: tests/test_gpu_multi.py."""
+    """The peer-memory all-reduce with world = 1 (this rank maps only itself): barrier epochs, in-place reduce and the ln
+    tables of the one-launch exchange (peer_allreduce_background runs peer_reduce_finalize) all run, and the scan equals the
+    plain one.  Two ranks: tests/test_gpu_multi.py."""
     rng = np.random.default_rng(31)
     n1, n2, S = 20, 16, 9000
     G, w1, w2, pos, off = random_panel(rng, S, n1, n2, 3, 120000)
@@ -367,7 +368,7 @@ def test_peer_exchange_single_rank(T, h):
     for _ in range(3):
         h.background(T.BG_GENOME)
         h.peer_allreduce_background()
-        s2, s1a, s1b = h.get_background(0)        # settles the pending wait without finalize
+        s2, s1a, s1b = h.get_background(0)        # the histogram between two exchanges
         h.peer_allreduce_background()             # sum over one rank: unchanged
         h.finalize_background()
         res = h.scan(6000)

@@ -4,5 +4,3 @@ mkdir -p gpurun_out
 for wl in config5 config4; do python bench.py --workload $wl --no-cpu --no-e2e --no-extra --verify-windows 32 --steps 20 > gpurun_out/r2m_popc_$wl.json 2> gpurun_out/r2m_popc_$wl.err; done
 python tools/show_bench.py gpurun_out/r2m_popc_config5.json gpurun_out/r2m_popc_config4.json
 python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29511 bench.py --gpus 2 --steps 30 --warmup 3 --no-cpu > gpurun_out/r2m_bench_n2.json 2> gpurun_out/r2m_bench_n2.err; tail -2 gpurun_out/r2m_bench_n2.err | cut -c1-300
-TDSFS_NO_TAIL=1 python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29512 bench.py --gpus 2 --steps 30 --warmup 3 --no-cpu --no-e2e > gpurun_out/r2m_bench_n2_notail.json 2> gpurun_out/r2m_bench_n2_notail.err
-python tools/show_bench.py gpurun_out/r2m_bench_n2.json gpurun_out/r2m_bench_n2_notail.json

@@ -22,5 +22,3 @@ done; done; done
 for w in 10 12 14 16; do for t in 1 2 4; do for d in 1 2; do
   run config4 w${w}t${t}d${d} TDSFS_K1_WARPS=$w TDSFS_K1_TILE=$t TDSFS_K1_DEPTH=$d
 done; done; done
-run config5 noplain TDSFS_NO_PLAIN=1
-run config4 noplain TDSFS_NO_PLAIN=1

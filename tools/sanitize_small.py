@@ -2,7 +2,7 @@
 """Small scans that touch every kernel of the hot path, for compute-sanitizer (one tool per gpurun call):
   compute-sanitizer --tool racecheck|synccheck|memcheck python tools/sanitize_small.py
 k1_fused (plain + generic instantiation, narrow + wide records, fixed-bp + fixed-SNP windows, chunked upload, flags),
-k3_finish (both variants), k3_score_small (G = 1, 2, 4) + k3_score_large, k2_bounds_*, k_finalize_counts, k1_counts,
+k3_finish, k3_score_small (G = 1, 2, 4) + k3_score_large, k2_bounds_*, k_finalize_counts, k1_counts,
 the Poisson walk.  Results are compared with the CPU oracle so that a sanitizer-only failure mode cannot hide."""
 import os
 import sys
@@ -27,24 +27,22 @@ def main():
                 os.environ["TDSFS_UPLOAD_CHUNK_KB"] = chunk_kb
             else:
                 os.environ.pop("TDSFS_UPLOAD_CHUNK_KB", None)
-            for stream in ("0", "1"):
-                os.environ["TDSFS_FINISH_STREAM"] = stream
-                h = T.Handle(0)
-                h.set_panel(n1, n2, True)
-                h.load_genotypes(G, S, w1, w2, n1, n2, pos, off)
-                for mode, bg in ((T.BG_GENOME, "genome"), (T.BG_PER_CHROM, "per_chrom")):
-                    h.plan(W)
-                    h.background(mode)
-                    h.finalize_background()
-                    res = h.scan(W)
-                    assert h.scan_info()[0]
-                    compare_scan(T, res, O.scan_arrays(cnt, pos, off, n1, n2, W=W, bg=bg))
-                    h.plan(N, snp_mode=True)
-                    h.background(mode)
-                    h.finalize_background()
-                    compare_scan(T, h.scan(N, snp_mode=True), O.scan_arrays(cnt, pos, off, n1, n2, N=N, bg=bg), snp_mode=True)
-                    done.append(("fused", n1, chunk_kb, stream, bg))
-                h.close()
+            h = T.Handle(0)
+            h.set_panel(n1, n2, True)
+            h.load_genotypes(G, S, w1, w2, n1, n2, pos, off)
+            for mode, bg in ((T.BG_GENOME, "genome"), (T.BG_PER_CHROM, "per_chrom")):
+                h.plan(W)
+                h.background(mode)
+                h.finalize_background()
+                res = h.scan(W)
+                assert h.scan_info()[0]
+                compare_scan(T, res, O.scan_arrays(cnt, pos, off, n1, n2, W=W, bg=bg))
+                h.plan(N, snp_mode=True)
+                h.background(mode)
+                h.finalize_background()
+                compare_scan(T, h.scan(N, snp_mode=True), O.scan_arrays(cnt, pos, off, n1, n2, N=N, bg=bg), snp_mode=True)
+                done.append(("fused", n1, chunk_kb, bg))
+            h.close()
         # table scorer (no plan), group widths, large windows, counts entry, wide records
         for g in ("1", "2", "4"):
             os.environ["TDSFS_SCORE_G"] = g
