@@ -9,14 +9,16 @@
 #include <string>
 #include <vector>
 
+#include <cub/device/device_scan.cuh>
 #include <nvtx3/nvToolsExt.h>
 
 #include "tdsfs_kernels.cuh"
 #include "tdsfs_fused.cuh"
+#include "tdsfs_diversity.cuh"
 
 using namespace tdsfs;
 
-#define TDSFS_VERSION 200
+#define TDSFS_VERSION 201
 
 static thread_local std::string g_err;
 
@@ -62,7 +64,7 @@ static long long peer_timeout_cycles() {
     if (r__) return r__;       \
   } while (0)
 
-enum { EV_BG0, EV_K1, EV_FIN0, EV_FIN1, EV_SC0, EV_K2, EV_K3S, EV_K3L, EV_X0, EV_X1, NEV };
+enum { EV_BG0, EV_K1, EV_FIN0, EV_FIN1, EV_SC0, EV_K2, EV_K3S, EV_K3L, EV_X0, EV_X1, EV_D0, EV_D1, NEV };
 
 struct Chunk {
   long long r0, r1;
@@ -172,6 +174,23 @@ struct tdsfs_ctx {
   int step_mode = -1, warm_mode = -1;
   long long step_launches = 0;
   bool step_graphs_off = false;       // capture failed once: run eagerly from then on
+  // per-window diversity (tdsfs_diversity_*): its own candidate list, boundaries, scratch and results, so that it never
+  // touches the scan's plan, window buffers or unfetched results
+  long long div_W = -1;               // (size, mode) whose candidate offsets d_div_cand_off holds
+  int div_snp = -1;
+  std::vector<long long> div_off_host;
+  long long div_cap = 0, div_part_cap = 0, div_ncand = 0;
+  size_t div_tmp_bytes = 0;
+  long long* d_div_cand_off = nullptr;
+  int32_t *d_div_wlo = nullptr, *d_div_whi = nullptr, *d_div_wchrom = nullptr, *d_div_count = nullptr, *d_div_nsites = nullptr;
+  int32_t* d_div_large = nullptr;     // never written: the diversity pass has no "large window" split
+  int* d_div_nlarge = nullptr;
+  long long *d_div_wstart = nullptr, *d_div_wend = nullptr, *d_div_nseg = nullptr, *d_div_segoff = nullptr;
+  double *d_div_pi1 = nullptr, *d_div_pi2 = nullptr, *d_div_dxy = nullptr, *d_div_fst = nullptr;
+  uint8_t* d_div_flags = nullptr;
+  DivPart* d_div_part = nullptr;
+  void* d_div_tmp = nullptr;          // CUB scan scratch
+  bool div_ready = false, div_timed = false;
   // instrumentation
   cudaEvent_t ev[NEV] = {};
   float ms[10] = {};
@@ -301,6 +320,8 @@ static void free_data(tdsfs_ctx* c) {
   c->plan_W = -1;
   c->ws_ready = false;
   c->force_wide = false;
+  c->div_W = -1;
+  c->div_ready = false;
 }
 
 extern "C" void tdsfs_destroy(tdsfs_t* c) {
@@ -327,6 +348,11 @@ extern "C" void tdsfs_destroy(tdsfs_t* c) {
   dev_free(c->r_T1b); dev_free(c->r_flags); dev_free(c->d_scratch);
   for (int i = 0; i < NEV; ++i) if (c->ev[i]) cudaEventDestroy(c->ev[i]);
   dev_free(c->d_dxI); dev_free(c->d_ws); dev_free(c->d_gridbar); dev_free(c->d_stamps);
+  dev_free(c->d_div_cand_off); dev_free(c->d_div_wlo); dev_free(c->d_div_whi); dev_free(c->d_div_wchrom); dev_free(c->d_div_count);
+  dev_free(c->d_div_nsites); dev_free(c->d_div_large); dev_free(c->d_div_nlarge); dev_free(c->d_div_wstart); dev_free(c->d_div_wend);
+  dev_free(c->d_div_nseg); dev_free(c->d_div_segoff); dev_free(c->d_div_pi1); dev_free(c->d_div_pi2); dev_free(c->d_div_dxy);
+  dev_free(c->d_div_fst); dev_free(c->d_div_flags); dev_free(c->d_div_part);
+  if (c->d_div_tmp) cudaFree(c->d_div_tmp);
   cudaStreamDestroy(c->own_stream);
   cudaStreamDestroy(c->copy_stream);
   cudaStreamDestroy(c->plan_stream);
@@ -1409,6 +1435,136 @@ extern "C" int tdsfs_window_spectra(tdsfs_t* c, int64_t window, uint64_t* s2, ui
   return 0;
 }
 
+// ------------------------------------------------------------------------------------------------ diversity (Hudson FST, pi, dxy)
+extern "C" int tdsfs_fetch_diversity(tdsfs_t* c, tdsfs_diversity_t* out, int64_t cap, int64_t* n_windows) {
+  if (!c || !out) return fail(TDSFS_ERR_ARG, "NULL argument");
+  if (!c->div_ready) return fail(TDSFS_ERR_STATE, "no diversity results (tdsfs_diversity_bp / _snp first)");
+  if (cap < c->div_ncand) return fail(TDSFS_ERR_ARG, "result capacity %lld < %lld candidate windows", (long long)cap, c->div_ncand);
+  CK(cudaSetDevice(c->device));
+  cudaStream_t st = c->stream;
+  const size_t n = (size_t)c->div_ncand;
+#define D2H(dst, src, T) \
+  if (out->dst && n) CK(cudaMemcpyAsync(out->dst, c->src, n * sizeof(T), cudaMemcpyDeviceToHost, st))
+  D2H(chrom, d_div_wchrom, int32_t);
+  D2H(start, d_div_wstart, long long);
+  D2H(end, d_div_wend, long long);
+  D2H(snp_count, d_div_count, int32_t);
+  D2H(flags, d_div_flags, uint8_t);
+  D2H(n_sites, d_div_nsites, int32_t);
+  D2H(pi_p1, d_div_pi1, double);
+  D2H(pi_p2, d_div_pi2, double);
+  D2H(dxy, d_div_dxy, double);
+  D2H(fst, d_div_fst, double);
+#undef D2H
+  CK(cudaStreamSynchronize(st));
+  if (n_windows) *n_windows = c->div_ncand;
+  return 0;
+}
+
+static int ensure_div_buffers(tdsfs_ctx* c, long long ncand, long long parts) {
+  if (ncand > c->div_cap) {
+    CK(cudaStreamSynchronize(c->stream));  // a previous asynchronous call may still use the old arrays
+    dev_free(c->d_div_wlo); dev_free(c->d_div_whi); dev_free(c->d_div_wchrom); dev_free(c->d_div_count); dev_free(c->d_div_nsites);
+    dev_free(c->d_div_wstart); dev_free(c->d_div_wend); dev_free(c->d_div_nseg); dev_free(c->d_div_segoff); dev_free(c->d_div_pi1);
+    dev_free(c->d_div_pi2); dev_free(c->d_div_dxy); dev_free(c->d_div_fst); dev_free(c->d_div_flags);
+    if (c->d_div_tmp) cudaFree(c->d_div_tmp);
+    c->d_div_tmp = nullptr;
+    CKR(dev_alloc(&c->d_div_wlo, ncand)); CKR(dev_alloc(&c->d_div_whi, ncand)); CKR(dev_alloc(&c->d_div_wchrom, ncand));
+    CKR(dev_alloc(&c->d_div_count, ncand)); CKR(dev_alloc(&c->d_div_nsites, ncand)); CKR(dev_alloc(&c->d_div_wstart, ncand));
+    CKR(dev_alloc(&c->d_div_wend, ncand)); CKR(dev_alloc(&c->d_div_nseg, ncand + 1)); CKR(dev_alloc(&c->d_div_segoff, ncand + 1));
+    CKR(dev_alloc(&c->d_div_pi1, ncand)); CKR(dev_alloc(&c->d_div_pi2, ncand)); CKR(dev_alloc(&c->d_div_dxy, ncand));
+    CKR(dev_alloc(&c->d_div_fst, ncand)); CKR(dev_alloc(&c->d_div_flags, ncand));
+    size_t tmp = 0;
+    CK(cub::DeviceScan::ExclusiveSum(nullptr, tmp, c->d_div_nseg, c->d_div_segoff, (int)(ncand + 1), c->stream));
+    CK(cudaMalloc(&c->d_div_tmp, std::max<size_t>(tmp, 16)));
+    c->div_tmp_bytes = std::max<size_t>(tmp, 16);
+    c->div_cap = ncand;
+  }
+  if (parts > c->div_part_cap) {
+    CK(cudaStreamSynchronize(c->stream));
+    dev_free(c->d_div_part);
+    CKR(dev_alloc(&c->d_div_part, parts));
+    c->div_part_cap = parts;
+  }
+  if (!c->d_div_large) {
+    CKR(dev_alloc(&c->d_div_large, 1));
+    CKR(dev_alloc(&c->d_div_nlarge, 1));
+  }
+  return 0;
+}
+
+// Per-window Hudson FST, pi and dxy over the candidate windows of (W, mode), in the order of tdsfs_scan_*: window
+// boundaries (K2 into the diversity pass's own arrays) -> segments per window -> their prefix sum (device) -> k_diversity
+// (one warp per segment of DIV_SEG rows) -> k_div_finish.  Needs loaded data only; no host round trip when out == NULL.
+static int diversity(tdsfs_ctx* c, long long W, bool snp_mode, tdsfs_diversity_t* out, int64_t cap, int64_t* n_windows) {
+  if (!c || W < 1) return fail(TDSFS_ERR_ARG, "bad argument");
+  if (!c->loaded) return fail(TDSFS_ERR_STATE, "load data first");
+  CK(cudaSetDevice(c->device));
+  NvtxRange nvtx("tdsfs:diversity (FST, pi, dxy)");
+  cudaStream_t st = c->stream;
+  if (c->div_W != W || c->div_snp != (int)snp_mode) {  // candidate offsets cached per (size, mode), apart from the scan's
+    std::vector<long long> off;
+    CKR(candidates(c, W, snp_mode, off));
+    c->div_off_host.swap(off);
+    c->div_W = -1;
+    dev_free(c->d_div_cand_off);
+    CKR(dev_alloc(&c->d_div_cand_off, c->C + 1));
+    CK(cudaMemcpyAsync(c->d_div_cand_off, c->div_off_host.data(), (size_t)(c->C + 1) * 8, cudaMemcpyHostToDevice, st));
+    c->div_W = W;
+    c->div_snp = snp_mode;
+  }
+  const long long ncand = c->div_off_host[c->C];
+  if (out && cap < ncand) return fail(TDSFS_ERR_ARG, "result capacity %lld < %lld candidate windows", (long long)cap, ncand);
+  // windows never overlap, so sum_w ceil(rows_w / SEG) <= S / SEG + ncand
+  const long long max_parts = ncand + c->S / DIV_SEG + 1;
+  CKR(ensure_div_buffers(c, ncand, max_parts));
+  c->div_ready = false;
+  c->div_ncand = ncand;
+  for (auto& ch : c->chunks) if (ch.ev) CK(cudaStreamWaitEvent(st, ch.ev, 0));  // rows of a host upload still in flight
+  if (ncand == 0) CK(cudaEventRecord(c->ev[EV_D0], st));
+  if (ncand > 0) {
+    WinParams w;
+    w.pos = c->dPos; w.chrom_off = c->d_off; w.cand_off = c->d_div_cand_off; w.C = c->C; w.W = W; w.ncand = ncand;
+    w.wlo = c->d_div_wlo; w.whi = c->d_div_whi; w.wchrom = c->d_div_wchrom; w.wstart = c->d_div_wstart; w.wend = c->d_div_wend;
+    w.large = c->d_div_large; w.nlarge = c->d_div_nlarge;
+    w.r_count = c->d_div_count; w.r_flags = c->d_div_flags;  // K2 marks empty windows; k_div_finish rewrites every entry
+    w.wcap = 0x7FFFFFFF;
+    const int g2 = (int)((ncand + 255) / 256);
+    if (snp_mode) k2_bounds_snp<<<g2, 256, 0, st>>>(w); else k2_bounds_bp<<<g2, 256, 0, st>>>(w);
+    DivParams p;
+    memset(&p, 0, sizeof p);
+    fill_key_params(c, p.k);
+    p.wlo = c->d_div_wlo; p.whi = c->d_div_whi; p.ncand = ncand; p.nseg = c->d_div_nseg; p.segoff = c->d_div_segoff;
+    p.part = c->d_div_part; p.snp_count = c->d_div_count; p.n_sites = c->d_div_nsites; p.pi1 = c->d_div_pi1; p.pi2 = c->d_div_pi2;
+    p.dxy = c->d_div_dxy; p.fst = c->d_div_fst; p.flags = c->d_div_flags;
+    k_div_nseg<<<(int)((ncand + 1 + 255) / 256), 256, 0, st>>>(p);
+    size_t tmp = c->div_tmp_bytes;
+    CK(cub::DeviceScan::ExclusiveSum(c->d_div_tmp, tmp, c->d_div_nseg, c->d_div_segoff, (int)(ncand + 1), st));
+    CK(cudaEventRecord(c->ev[EV_D0], st));
+    // one warp per segment; the grid covers the bound on the segment count and warps past the actual count return at once
+    void (*kern)(DivParams) = k_diversity<0, 0>;
+    if (c->dG && c->W1 == 32 && c->W2 == 32) kern = k_diversity<32, 32>;       // 500 + 500 diploids (BASELINE config 5)
+    else if (c->dG && c->W1 == 14 && c->W2 == 14) kern = k_diversity<14, 14>;  // 200 + 200 diploids (BASELINE config 4)
+    kern<<<(unsigned)((max_parts + DIV_WARPS - 1) / DIV_WARPS), DIV_WARPS * 32, 0, st>>>(p);
+    k_div_finish<<<(int)((ncand + 255) / 256), 256, 0, st>>>(p);
+    c->launches += 5;
+    CK(cudaGetLastError());
+  }
+  CK(cudaEventRecord(c->ev[EV_D1], st));
+  c->div_timed = true;
+  c->div_ready = true;
+  if (out) return tdsfs_fetch_diversity(c, out, cap, n_windows);
+  if (n_windows) *n_windows = ncand;
+  return finish(c);
+}
+
+extern "C" int tdsfs_diversity_bp(tdsfs_t* c, int64_t W, tdsfs_diversity_t* out, int64_t cap, int64_t* n_windows) {
+  return diversity(c, W, false, out, cap, n_windows);
+}
+extern "C" int tdsfs_diversity_snp(tdsfs_t* c, int64_t N, tdsfs_diversity_t* out, int64_t cap, int64_t* n_windows) {
+  return diversity(c, N, true, out, cap, n_windows);
+}
+
 // ------------------------------------------------------------------------------------------------ explicit likelihood
 extern "C" int tdsfs_likelihood(tdsfs_t* c, const int64_t* x, const double* b, int64_t n, double B, double* T, int32_t* flag) {
   if (!c || !T || !flag || n < 0 || (n > 0 && (!x || !b))) return fail(TDSFS_ERR_ARG, "bad argument");
@@ -1492,6 +1648,7 @@ extern "C" int tdsfs_timings(tdsfs_t* c, float* ms, int32_t n) {
   }
   c->ms[5] = c->ms[0];
   if (c->x_timed) cudaEventElapsedTime(&c->ms[8], c->ev[EV_X0], c->ev[EV_X1]);
+  if (c->div_timed) cudaEventElapsedTime(&c->ms[9], c->ev[EV_D0], c->ev[EV_D1]);
   cudaGetLastError();
   for (int i = 0; i < n && i < 10; ++i) ms[i] = c->ms[i];
   return 0;

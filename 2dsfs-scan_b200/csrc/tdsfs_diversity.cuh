@@ -1,0 +1,155 @@
+// tdsfs_diversity.cuh -- per-window Hudson FST, pi and dxy (DESIGN.md section 7, "Diversity: Hudson FST, pi, dxy").
+// Included by tdsfs.cu after tdsfs_kernels.cuh and tdsfs_fused.cuh.  No reference counterpart: the reference's users get
+// the FST column of their tables from pixy, run separately over the same VCF.
+//
+// Per SNP that passes the spectrum filters (snp_flags bit0) with n_i = ref_i + alt_i >= 2 in both populations, in fp64:
+//   pi_i = 2 ref_i alt_i / (n_i (n_i - 1)),   dxy = (ref_1 alt_2 + alt_1 ref_2) / (n_1 n_2)
+// (integer numerators and denominators, one rounded division each).  The sums of a window are taken in a fixed order that
+// depends on the window's rows alone: segments of DIV_SEG rows counted from the window's first row; inside a segment lane
+// (s - first row) mod 32 adds its SNPs in row order and a fixed xor tree combines the lanes; the segment sums are added in
+// segment order.  So the result is bitwise the same for the counts and the genotype entry, any grid and any sharding that
+// keeps windows whole.
+#pragma once
+
+namespace tdsfs {
+
+constexpr int DIV_SEG = 1024;   // rows per segment (a multiple of 32)
+constexpr int DIV_WARPS = 8;    // warps per CTA of k_diversity: one warp per segment
+
+struct DivPart {  // sums of one segment
+  double pi1, pi2, dxy;
+  int n_sites, snp_count;
+};
+
+struct DivParams {
+  KeyParams k;                 // source rows (G or cnt), sample columns, snp_flags + fix-ups (row_filters)
+  const int32_t* wlo;          // [ncand] first row of each candidate window (k2_bounds_*)
+  const int32_t* whi;          // [ncand] one past its last row
+  long long ncand;
+  long long* nseg;             // [ncand + 1] segments per window, 0 in the last slot
+  const long long* segoff;     // [ncand + 1] exclusive prefix sum of nseg: segoff[ncand] = number of segments
+  DivPart* part;               // [segments]
+  int32_t* snp_count;          // [ncand] outputs
+  int32_t* n_sites;
+  double* pi1;
+  double* pi2;
+  double* dxy;
+  double* fst;
+  uint8_t* flags;
+};
+
+__global__ void __launch_bounds__(256) k_div_nseg(const __grid_constant__ DivParams p) {
+  const long long id = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (id < p.ncand) p.nseg[id] = (__ldg(p.whi + id) - __ldg(p.wlo + id) + DIV_SEG - 1) / DIV_SEG;
+  else if (id == p.ncand) p.nseg[id] = 0;
+}
+
+// (ref1, alt1, ref2, alt2) of SNP s before the fix-ups: compile-time word counts (fully unrolled, every load of the row
+// issued together) or the runtime decode shared with k_window_hist (any width, and the counts entry)
+template <int TW1, int TW2>
+__device__ __forceinline__ void div_counts(const KeyParams& p, long long s, int& ref1, int& alt1, int& ref2, int& alt2) {
+  if constexpr (TW1 > 0 && TW2 > 0) {
+    // every word of the row is loaded before any is counted: one memory round trip per row (count_pop_planes interleaves
+    // loads and counting, and the compiler then issues the second population's loads only after the first one's arrive)
+    constexpr int P1 = TW1 / 2, P2 = TW2 / 2;
+    const uint32_t* row = p.G + (s >> 5) * (long long)((TW1 + TW2) * BLK) + (s & 31);
+    uint32_t lo1[P1], hi1[P1], lo2[P2], hi2[P2];
+#pragma unroll
+    for (int i = 0; i < P1; ++i) { lo1[i] = __ldcs(row + (2 * i) * BLK); hi1[i] = __ldcs(row + (2 * i + 1) * BLK); }
+#pragma unroll
+    for (int i = 0; i < P2; ++i) { lo2[i] = __ldcs(row + (TW1 + 2 * i) * BLK); hi2[i] = __ldcs(row + (TW1 + 2 * i + 1) * BLK); }
+    // codes 00, 01, 11, 10 = hom-ref, het, hom-alt, missing: alt = popc(lo) + popc(lo & hi), missing = popc(hi) - popc(lo & hi)
+    uint32_t b1[P1], b2[P2];
+#pragma unroll
+    for (int i = 0; i < P1; ++i) b1[i] = lo1[i] & hi1[i];
+#pragma unroll
+    for (int i = 0; i < P2; ++i) b2[i] = lo2[i] & hi2[i];
+    const int c1 = (int)popc_sum<P1>(b1), c2 = (int)popc_sum<P2>(b2);
+    alt1 = (int)popc_sum<P1>(lo1) + c1;
+    alt2 = (int)popc_sum<P2>(lo2) + c2;
+    ref1 = 2 * (p.ns1 - ((int)popc_sum<P1>(hi1) - c1)) - alt1;
+    ref2 = 2 * (p.ns2 - ((int)popc_sum<P2>(hi2) - c2)) - alt2;
+  } else {
+    source_counts(p, s, ref1, alt1, ref2, alt2);
+  }
+}
+
+// One warp per segment.  The warp walks the ALIGNED 32-row blocks that overlap its segment, so word w of a step is exactly
+// one 128-byte line (a window starting inside a block would otherwise split every line of every step in two).  Lane l loads
+// row b + l; its terms then move to the lane that owns that row in the definition, (s - r0) mod 32 = (l - r0) mod 32, which
+// receives its rows in increasing order, one per block: the sums are the definition's, bit for bit.
+template <int TW1, int TW2>
+__global__ void __launch_bounds__(DIV_WARPS * 32) k_diversity(const __grid_constant__ DivParams p) {
+  const int lane = threadIdx.x & 31;
+  const long long g = (long long)blockIdx.x * DIV_WARPS + (threadIdx.x >> 5);
+  if (g >= __ldg(p.segoff + p.ncand)) return;
+  // window of segment g: the last w with segoff[w] <= g (an empty window owns no segment, so it is never the last one)
+  long long lo = 0, hi = p.ncand;
+  while (hi - lo > 1) {
+    const long long mid = (lo + hi) >> 1;
+    if (__ldg(p.segoff + mid) <= g) lo = mid; else hi = mid;
+  }
+  const long long r0 = (long long)__ldg(p.wlo + lo) + (g - __ldg(p.segoff + lo)) * DIV_SEG;
+  const long long r1 = min(r0 + DIV_SEG, (long long)__ldg(p.whi + lo));
+  const int src = (lane + (int)(r0 & 31)) & 31;  // the lane that loads the row this lane owns
+  double pi1 = 0.0, pi2 = 0.0, dxy = 0.0;
+  int n_sites = 0, snp_count = 0;
+  for (long long b = r0 & ~31LL; b < r1; b += 32) {
+    const long long s = b + lane;
+    double t1 = 0.0, t2 = 0.0, td = 0.0;
+    int enter = 0, counted = 0;
+    if (s >= r0 && s < r1) {
+      int ref1, alt1, ref2, alt2;
+      div_counts<TW1, TW2>(p.k, s, ref1, alt1, ref2, alt2);
+      counted = p.k.flags ? (__ldg(p.k.flags + s) >> 1) & 1 : 1;
+      const bool pass = row_filters(p.k, s, ref1, alt1, ref2, alt2);
+      const long long n1 = ref1 + alt1, n2 = ref2 + alt2;
+      if (pass && n1 >= 2 && n2 >= 2) {
+        t1 = (double)(2LL * ref1 * alt1) / (double)(n1 * (n1 - 1));
+        t2 = (double)(2LL * ref2 * alt2) / (double)(n2 * (n2 - 1));
+        td = (double)((long long)ref1 * alt2 + (long long)alt1 * ref2) / (double)(n1 * n2);
+        enter = 1;
+      }
+    }
+    t1 = __shfl_sync(0xffffffffu, t1, src);
+    t2 = __shfl_sync(0xffffffffu, t2, src);
+    td = __shfl_sync(0xffffffffu, td, src);
+    enter = __shfl_sync(0xffffffffu, enter, src);
+    snp_count += __shfl_sync(0xffffffffu, counted, src);
+    if (enter) {
+      pi1 += t1; pi2 += t2; dxy += td;
+      ++n_sites;
+    }
+  }
+#pragma unroll
+  for (int o = 16; o; o >>= 1) {
+    pi1 += __shfl_xor_sync(0xffffffffu, pi1, o);
+    pi2 += __shfl_xor_sync(0xffffffffu, pi2, o);
+    dxy += __shfl_xor_sync(0xffffffffu, dxy, o);
+    n_sites += __shfl_xor_sync(0xffffffffu, n_sites, o);
+    snp_count += __shfl_xor_sync(0xffffffffu, snp_count, o);
+  }
+  if (lane == 0) p.part[g] = DivPart{pi1, pi2, dxy, n_sites, snp_count};
+}
+
+// One thread per window: its segment sums in segment order, then FST (NaN when dxy == 0).
+__global__ void __launch_bounds__(256) k_div_finish(const __grid_constant__ DivParams p) {
+  const long long id = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (id >= p.ncand) return;
+  double pi1 = 0.0, pi2 = 0.0, dxy = 0.0;
+  int n_sites = 0, snp_count = 0;
+  for (long long g = __ldg(p.segoff + id), e = __ldg(p.segoff + id + 1); g < e; ++g) {
+    const DivPart q = p.part[g];
+    pi1 += q.pi1; pi2 += q.pi2; dxy += q.dxy;
+    n_sites += q.n_sites; snp_count += q.snp_count;
+  }
+  p.snp_count[id] = snp_count;
+  p.n_sites[id] = n_sites;
+  p.pi1[id] = pi1;
+  p.pi2[id] = pi2;
+  p.dxy[id] = dxy;
+  p.fst[id] = dxy == 0.0 ? __longlong_as_double(0x7FF8000000000000LL) : 1.0 - (pi1 + pi2) / (2.0 * dxy);
+  p.flags[id] = __ldg(p.whi + id) == __ldg(p.wlo + id) ? TDSFS_F_EMPTY : 0;
+}
+
+}  // namespace tdsfs

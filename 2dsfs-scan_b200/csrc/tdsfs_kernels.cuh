@@ -1229,28 +1229,34 @@ __global__ void __launch_bounds__(LARGE_THREADS) k3_score_large(const __grid_con
   score_large_windows(p, blockIdx.x, gridDim.x);
 }
 
+// (ref1, alt1, ref2, alt2) of SNP s before the fix-ups, from the source rows: the counts entry or the B32 genotype matrix
+// with runtime word counts
+__device__ __forceinline__ void source_counts(const KeyParams& p, long long s, int& ref1, int& alt1, int& ref2, int& alt2) {
+  if (p.cnt) {
+    const uint2 v = __ldg(reinterpret_cast<const uint2*>(p.cnt) + s);
+    ref1 = v.x & 0xFFFF; alt1 = v.x >> 16; ref2 = v.y & 0xFFFF; alt2 = v.y >> 16;
+    return;
+  }
+  const int RW = p.W1 + p.W2;
+  const uint32_t* row = p.G + ((s >> 5) * RW) * BLK + (s & 31);
+  int T[2] = {0, 0}, M[2] = {0, 0};
+  for (int w = 0; w < RW; w += 2) {  // (lo plane, hi plane) of 32 samples; W1 and W2 are even
+    const uint32_t l = row[(long long)w * BLK], h = row[(long long)(w + 1) * BLK];
+    T[w >= p.W1] += __popc(l) + __popc(h);
+    M[w >= p.W1] += __popc(h & ~l);
+  }
+  alt1 = T[0] - M[0]; alt2 = T[1] - M[1];
+  ref1 = 2 * (p.ns1 - M[0]) - alt1; ref2 = 2 * (p.ns2 - M[1]) - alt2;
+}
+
 // dense spectra of one window (calculate_2d_sfs / calculate_1d_sfs on window_data): 2D bins from the stored records,
 // raw (unfolded) 1D alt counts recomputed from the source rows (counts entry or B32 genotype matrix)
 __global__ void k_window_hist(const __grid_constant__ KeyParams p, int lo, int hi, uint32_t* h2, uint32_t* h1a, uint32_t* h1b) {
-  const int RW = p.W1 + p.W2;
   for (long long s = lo + blockIdx.x * blockDim.x + threadIdx.x; s < hi; s += gridDim.x * blockDim.x) {
     const uint32_t k = load_rec(p.rec, p.fmt, s, p.n1, p.n2, p.C2).x;
     if (k) atomicAdd(h2 + k, 1u);
     int ref1, alt1, ref2, alt2;
-    if (p.cnt) {
-      const uint2 v = reinterpret_cast<const uint2*>(p.cnt)[s];
-      ref1 = v.x & 0xFFFF; alt1 = v.x >> 16; ref2 = v.y & 0xFFFF; alt2 = v.y >> 16;
-    } else {
-      const uint32_t* row = p.G + ((s >> 5) * RW) * BLK + (s & 31);
-      int T[2] = {0, 0}, M[2] = {0, 0};
-      for (int w = 0; w < RW; w += 2) {  // (lo plane, hi plane) of 32 samples; W1 and W2 are even
-        const uint32_t l = row[(long long)w * BLK], h = row[(long long)(w + 1) * BLK];
-        T[w >= p.W1] += __popc(l) + __popc(h);
-        M[w >= p.W1] += __popc(h & ~l);
-      }
-      alt1 = T[0] - M[0]; alt2 = T[1] - M[1];
-      ref1 = 2 * (p.ns1 - M[0]) - alt1; ref2 = 2 * (p.ns2 - M[1]) - alt2;
-    }
+    source_counts(p, s, ref1, alt1, ref2, alt2);
     if (row_filters(p, s, ref1, alt1, ref2, alt2)) {
       if (alt1 > 0 && alt1 < p.R1) atomicAdd(h1a + alt1, 1u);
       if (alt2 > 0 && alt2 < p.R2) atomicAdd(h1b + alt2, 1u);

@@ -22,6 +22,7 @@ EXPORTS = [
     "tdsfs_scan_snp", "tdsfs_set_poisson_background", "tdsfs_scan_poisson_bp", "tdsfs_fetch_results", "tdsfs_check", "tdsfs_run_bp", "tdsfs_step_bp", "tdsfs_window_spectra", "tdsfs_likelihood",
     "tdsfs_poisson_score", "tdsfs_peer_export", "tdsfs_peer_import", "tdsfs_peer_allreduce_background", "tdsfs_peer_reduce_finalize", "tdsfs_peer_close",
     "tdsfs_synth_genotypes", "tdsfs_timings", "tdsfs_launch_count", "tdsfs_scan_info", "tdsfs_tail_stamps", "tdsfs_version",
+    "tdsfs_diversity_bp", "tdsfs_diversity_snp", "tdsfs_fetch_diversity",
 ]
 
 
@@ -49,6 +50,14 @@ class Result(C.Structure):
 
 RESULT_DTYPES = dict(chrom=np.int32, start=np.int64, end=np.int64, snp_count=np.int32, n2d=np.int32, n1d_p1=np.int32,
                      n1d_p2=np.int32, T2D=np.float64, T1D_p1=np.float64, T1D_p2=np.float64, flags=np.uint8)
+
+class Diversity(C.Structure):
+    _fields_ = [("chrom", C.c_void_p), ("start", C.c_void_p), ("end", C.c_void_p), ("snp_count", C.c_void_p), ("flags", C.c_void_p),
+                ("n_sites", C.c_void_p), ("pi_p1", C.c_void_p), ("pi_p2", C.c_void_p), ("dxy", C.c_void_p), ("fst", C.c_void_p)]
+
+
+DIVERSITY_DTYPES = dict(chrom=np.int32, start=np.int64, end=np.int64, snp_count=np.int32, flags=np.uint8, n_sites=np.int32,
+                        pi_p1=np.float64, pi_p2=np.float64, dxy=np.float64, fst=np.float64)
 
 _lib = None
 
@@ -244,6 +253,32 @@ class Handle:
         self._check(f(self._h, C.c_int64(size), C.byref(r), C.c_int64(cap), C.byref(n)))
         return {k: v[:n.value] for k, v in arrs.items()}
 
+    def diversity(self, size, snp_mode=False, fetch=True):
+        """Per-window Hudson FST, pi and dxy over the candidate windows of (size, mode), in scan order (tdsfs_diversity_*).
+        pi_p1 / pi_p2 / dxy are sums over the variant sites that entered (n_sites), not per-bp values; fst is NaN when
+        dxy == 0.  Returns a dict of arrays (chrom / start / end / snp_count / flags as the scan's), or the candidate count
+        when fetch=False (results stay on the device: fetch_diversity)."""
+        f = self._L.tdsfs_diversity_snp if snp_mode else self._L.tdsfs_diversity_bp
+        n = C.c_int64()
+        if not fetch:
+            self._check(f(self._h, C.c_int64(size), None, C.c_int64(0), C.byref(n)))
+            return n.value
+        cap = self.candidates(size, snp_mode)
+        arrs, r = self._alloc_diversity(cap)
+        self._check(f(self._h, C.c_int64(size), C.byref(r), C.c_int64(cap), C.byref(n)))
+        return {k: v[:n.value] for k, v in arrs.items()}
+
+    @staticmethod
+    def _alloc_diversity(n):
+        arrs = {k: np.zeros(max(n, 1), dtype=dt) for k, dt in DIVERSITY_DTYPES.items()}
+        return arrs, Diversity(**{k: v.ctypes.data for k, v in arrs.items()})
+
+    def fetch_diversity(self, cap):
+        arrs, r = self._alloc_diversity(cap)
+        n = C.c_int64()
+        self._check(self._L.tdsfs_fetch_diversity(self._h, C.byref(r), C.c_int64(cap), C.byref(n)))
+        return {k: v[:n.value] for k, v in arrs.items()}
+
     def fetch_results(self, cap):
         arrs, r = self._alloc_result(cap)
         n = C.c_int64()
@@ -298,6 +333,12 @@ class Handle:
         self._check(self._L.tdsfs_timings(self._h, ms, C.c_int32(10)))
         names = ["k1_count", "finalize", "k2_bounds", "k3_small", "k3_large", "background_call", "scan_call", "pass_total", "exchange"]
         return dict(zip(names, list(ms)))
+
+    def diversity_ms(self):
+        """CUDA-event time (ms) of the segment + finish kernels of the last diversity call (tdsfs_timings slot 9)."""
+        ms = (C.c_float * 10)()
+        self._check(self._L.tdsfs_timings(self._h, ms, C.c_int32(10)))
+        return float(ms[9])
 
     def launch_count(self):
         return int(self._L.tdsfs_launch_count(self._h))

@@ -292,3 +292,12 @@ def sharded_scan(handle, pieces, pos, size, bg_mode, device, *, snp_mode=False, 
         handle.check()  # a late or missing peer must not pass as a result
     return gather_results(localize_results(res, pieces, pos, size, snp_mode), 0, group)
 
+
+
+def sharded_diversity(handle, pieces, pos, size, device, *, snp_mode=False, group=None):
+    """Per-window Hudson FST, pi and dxy of a sharded panel: the diversity counterpart of sharded_scan, for a handle that
+    already holds this rank's pieces.  The sums of a window depend on its own rows only, so no collective is needed beyond
+    the gather, and the gathered arrays equal a single-handle run bit for bit.  `device` is unused (the handle knows its
+    GPU); it keeps sharded_scan's calling convention.  Returns the gathered arrays (identical on every rank)."""
+    res = handle.diversity(size, snp_mode=snp_mode)
+    return gather_results(localize_results(res, pieces, pos, size, snp_mode), 0, group)

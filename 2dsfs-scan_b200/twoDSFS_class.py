@@ -480,6 +480,42 @@ class LikelihoodInference_jointSFS:
         keys, counts, stats, _, _ = self._scan(table, snp_window_size, True, bg_mode=T.BG_PER_CHROM)
         return self._unguarded(keys, counts, stats, with_diff=True, snp_count_fixed=snp_window_size)
 
+    # ------------------------------------------------------------------ diversity (not in the reference)
+    def _fst(self, data_dict, size, snp_mode):
+        table = self._table(data_dict)
+        if table.n == 0:
+            return {}
+        self._int_filters()
+        eng = self._eng()
+        eng.load(table, self.pop1_size, self.pop2_size, self.fold, self._flags(table))
+        res = eng.h.diversity(size, snp_mode=snp_mode)
+        live = (res["flags"] & T.F_EMPTY) == 0
+        keys = window_keys(table, res, live)
+        cols = [res[k][live].tolist() for k in ("snp_count", "n_sites", "pi_p1", "pi_p2", "dxy", "fst")]
+        return {k: {"snp_count": c, "n_sites": n, "pi_pop1": a, "pi_pop2": b, "dxy": d, "FST": None if f != f else f}
+                for k, c, n, a, b, d, f in zip(keys, *cols)}
+
+    def fst_scan(self, data_dict, window_size):
+        """Hudson FST, pi and dxy of every non-empty fixed-bp window, computed on the GPU from the same data as the scans:
+        {"{chrom} {start}-{end}": {"snp_count", "n_sites", "pi_pop1", "pi_pop2", "dxy", "FST"}}, keyed like combined_scan.
+        A SNP enters the sums iff it passes the constructor's start_position / end_position / variant_type filters and has at
+        least two called alleles in both populations.  pi_pop1 / pi_pop2 / dxy are SUMS over those n_sites variant sites, not
+        per-bp values: divide by the window's callable length for per-bp diversity.  FST = 1 - (pi_pop1 + pi_pop2) / (2 dxy)
+        (Hudson, as a ratio of averages: Bhatia et al. 2013 eq. 10; pixy --fst_type hudson), None when dxy == 0.
+        snp_count is count_snps, as in the scanners.  Not in the reference; pass the result to save_csv_stats(fst=...)."""
+        self.data_dict = data_dict
+        self.window_size = window_size
+        return self._fst(data_dict, window_size, False)
+
+    def fst_scan_bySNPs(self, data_dict, snp_window_size):
+        """fst_scan over fixed-SNP windows (full chunks of snp_window_size SNPs per chromosome, labelled like
+        scan_perChr_bySNPs).  The key set is a superset of scan_perChr_bySNPs': a chunk that scanner skips because its 2D
+        spectrum is empty has dxy == 0 here and appears with FST None.  snp_count is count_snps of the chunk (the scanner
+        reports snp_window_size instead)."""
+        self.data_dict = data_dict
+        self.snp_window_size = snp_window_size
+        return self._fst(data_dict, snp_window_size, True)
+
     # ------------------------------------------------------------------ simulations
     def get_gens(self, main_dir):
         search_strings = set()
@@ -566,18 +602,23 @@ def load_chr_ids(chromosomes_txt):
 col_names = ['chromosome', 'window_start', 'window_end', 'snp_count', 'T2D', 'T1D_p1', 'T1D_p2', 'new_term_p1', 'new_term_p2', 'T2D_diff']
 
 
-def save_csv_stats(stats_dict, output):
-    """reference :1884-1907: same columns, chromosome mapped through chr_ids, None written as ''."""
+def save_csv_stats(stats_dict, output, fst=None):
+    """reference :1884-1907: same columns, chromosome mapped through chr_ids, None written as ''.  fst (not in the
+    reference): the dict of fst_scan / fst_scan_bySNPs over the same windows adds a trailing FST column, the layout of the
+    ECB tables the reference's R post-processing writes; '' where FST is None or the window has no entry."""
     with open(output, 'w', newline='') as csvfile:
-        writer = csv.DictWriter(csvfile, fieldnames=col_names)
+        writer = csv.DictWriter(csvfile, fieldnames=col_names + (['FST'] if fst is not None else []))
         writer.writeheader()
         for window_coords, result in stats_dict.items():
             chromosome = window_coords.split(' ')[0]
             window_start, window_end = window_coords.split(' ')[1].split('-')
-            writer.writerow({'chromosome': chr_ids.get(chromosome, chromosome), 'window_start': window_start, 'window_end': window_end,
-                             'snp_count': result["snp_count"], 'T2D': result["T2D"], 'T1D_p1': result["T1D_pop1"],
-                             'T1D_p2': result["T1D_pop2"], 'new_term_p1': result["new_term_pop1"],
-                             'new_term_p2': result["new_term_pop2"], 'T2D_diff': result["T2D_diff"]})
+            row = {'chromosome': chr_ids.get(chromosome, chromosome), 'window_start': window_start, 'window_end': window_end,
+                   'snp_count': result["snp_count"], 'T2D': result["T2D"], 'T1D_p1': result["T1D_pop1"],
+                   'T1D_p2': result["T1D_pop2"], 'new_term_p1': result["new_term_pop1"],
+                   'new_term_p2': result["new_term_pop2"], 'T2D_diff': result["T2D_diff"]}
+            if fst is not None:
+                row['FST'] = fst.get(window_coords, {}).get("FST")
+            writer.writerow(row)
 
 
 def plot_2d_sfs(*args, **kwargs):

@@ -213,6 +213,33 @@ int tdsfs_step_bp(tdsfs_t* ctx, int32_t bg_mode, int64_t W);
 /* Spectra of one scanned window (calculate_2d_sfs / calculate_1d_sfs on window_data): dense outputs, any NULL. */
 int tdsfs_window_spectra(tdsfs_t* ctx, int64_t window, uint64_t* sfs2d, uint64_t* sfs1d_p1, uint64_t* sfs1d_p2);
 
+/* ---- per-window diversity: Hudson FST, pi, dxy (no reference counterpart; DESIGN.md section 7) ------------------
+ * Over the candidate windows of (size, mode), in the list and order of tdsfs_scan_* of that size, from the loaded data
+ * alone (no background, no scan).  A SNP enters a window's sums iff it passes the spectrum filters (snp_flags bit0) and
+ * n_i = ref_i + alt_i >= 2 in both populations (called alleles, fix-ups applied).  Per SNP, in fp64:
+ *   pi_i = 2 ref_i alt_i / (n_i (n_i - 1)),   dxy = (ref_1 alt_2 + alt_1 ref_2) / (n_1 n_2)
+ * pi_p1 / pi_p2 / dxy are SUMS over the entered (variant) sites, not per-bp values: dividing by a callable length is the
+ * caller's business.  fst = 1 - (pi_p1 + pi_p2) / (2 dxy), Hudson's estimator as a ratio of averages (Bhatia et al. 2013,
+ * eq. 10), NaN when dxy == 0.  The sums run in a fixed order that depends on the window's rows alone, so results are
+ * bitwise equal for the counts and the genotype entry and for any sharding that keeps windows whole.
+ * The call keeps its own window arrays and results: a pending plan, the scan's results and the step graph are untouched.
+ * out == NULL: enqueue only (honours tdsfs_set_sync(0)); tdsfs_fetch_diversity copies the results later. */
+typedef struct {            /* caller-owned host SoA, capacity >= tdsfs_candidates_bp / _snp; any member may be NULL */
+  int32_t* chrom;           /* as tdsfs_result_t */
+  int64_t* start;
+  int64_t* end;
+  int32_t* snp_count;       /* count_snps, as tdsfs_result_t */
+  uint8_t* flags;           /* TDSFS_F_EMPTY */
+  int32_t* n_sites;         /* SNPs that entered the sums */
+  double* pi_p1;
+  double* pi_p2;
+  double* dxy;
+  double* fst;              /* NaN when dxy == 0 */
+} tdsfs_diversity_t;
+int tdsfs_diversity_bp(tdsfs_t* ctx, int64_t W, tdsfs_diversity_t* out, int64_t cap, int64_t* n_windows);
+int tdsfs_diversity_snp(tdsfs_t* ctx, int64_t N, tdsfs_diversity_t* out, int64_t cap, int64_t* n_windows);
+int tdsfs_fetch_diversity(tdsfs_t* ctx, tdsfs_diversity_t* out, int64_t cap, int64_t* n_windows);
+
 /* ---- likelihood of explicit spectra ------------------------------------------------------------------------
  * calculate_likelihood_1D / _2D (:478-537, :625-684) on already-interior vectors: x[n] integer counts,
  * b[n] background values, B = sum of b as the caller's language sums it.  *flag = 1 when the reference returns
@@ -230,7 +257,8 @@ int tdsfs_synth_genotypes(tdsfs_t* ctx, void* G_dev, int64_t S, int64_t snp0, in
                           int32_t ns1, int32_t ns2, uint64_t seed, double missing_rate, double fst);
 /* CUDA-event times (ms) of the last background / finalize / scan calls (synchronises the stream):
  * [0]=count kernel (K1), [1]=finalize, [2]=boundaries (K2), [3]=score small windows (K3/K4), [4]=score large windows,
- * [5]=background call, [6]=scan call, [7]=K1 start -> last score kernel end, [8]=peer exchange kernel (n >= 9). */
+ * [5]=background call, [6]=scan call, [7]=K1 start -> last score kernel end, [8]=peer exchange kernel (n >= 9),
+ * [9]=segment + finish kernels of the last tdsfs_diversity_* call (n >= 10). */
 int tdsfs_timings(tdsfs_t* ctx, float* ms, int32_t n);
 int64_t tdsfs_launch_count(tdsfs_t* ctx); /* kernels launched by this handle so far */
 /* Which path scored the last scan: *fused = 1 when the fused pair ran (tdsfs_plan_* before tdsfs_background on the
