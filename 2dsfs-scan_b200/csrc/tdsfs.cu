@@ -18,7 +18,7 @@
 
 using namespace tdsfs;
 
-#define TDSFS_VERSION 201
+#define TDSFS_VERSION 202
 
 static thread_local std::string g_err;
 
@@ -64,11 +64,29 @@ static long long peer_timeout_cycles() {
     if (r__) return r__;       \
   } while (0)
 
-enum { EV_BG0, EV_K1, EV_FIN0, EV_FIN1, EV_SC0, EV_K2, EV_K3S, EV_K3L, EV_X0, EV_X1, EV_D0, EV_D1, NEV };
+enum { EV_BG0, EV_K1, EV_FIN0, EV_FIN1, EV_SC0, EV_K2, EV_K3S, EV_K3L, EV_X0, EV_X1, EV_D0, EV_D1, EV_N0, EV_N1, NEV };
 
 struct Chunk {
   long long r0, r1;
   cudaEvent_t ev;
+};
+
+// Workspace of one per-window pass over the candidate windows of (size, mode) (tdsfs_diversity_*, tdsfs_neutrality_*):
+// its candidate offsets, window boundaries, segment list and scan scratch.
+struct WindowPass {
+  long long W = -1;                   // (size, mode) whose candidate offsets d_cand_off holds
+  int snp = -1;
+  std::vector<long long> off_host;
+  long long cap = 0, ncand = 0;
+  size_t tmp_bytes = 0;
+  long long* d_cand_off = nullptr;
+  int32_t *d_wlo = nullptr, *d_whi = nullptr, *d_wchrom = nullptr, *d_count = nullptr;
+  int32_t* d_large = nullptr;         // never written: a per-window pass has no "large window" split
+  int* d_nlarge = nullptr;
+  long long *d_wstart = nullptr, *d_wend = nullptr, *d_nseg = nullptr, *d_segoff = nullptr;
+  uint8_t* d_flags = nullptr;
+  void* d_tmp = nullptr;              // CUB scan scratch
+  bool ready = false, timed = false;  // results of the last call are on the device / its events were recorded
 };
 
 struct tdsfs_ctx {
@@ -174,26 +192,27 @@ struct tdsfs_ctx {
   int step_mode = -1, warm_mode = -1;
   long long step_launches = 0;
   bool step_graphs_off = false;       // capture failed once: run eagerly from then on
-  // per-window diversity (tdsfs_diversity_*): its own candidate list, boundaries, scratch and results, so that it never
-  // touches the scan's plan, window buffers or unfetched results
-  long long div_W = -1;               // (size, mode) whose candidate offsets d_div_cand_off holds
-  int div_snp = -1;
-  std::vector<long long> div_off_host;
-  long long div_cap = 0, div_part_cap = 0, div_ncand = 0;
-  size_t div_tmp_bytes = 0;
-  long long* d_div_cand_off = nullptr;
-  int32_t *d_div_wlo = nullptr, *d_div_whi = nullptr, *d_div_wchrom = nullptr, *d_div_count = nullptr, *d_div_nsites = nullptr;
-  int32_t* d_div_large = nullptr;     // never written: the diversity pass has no "large window" split
-  int* d_div_nlarge = nullptr;
-  long long *d_div_wstart = nullptr, *d_div_wend = nullptr, *d_div_nseg = nullptr, *d_div_segoff = nullptr;
+  // per-window passes over the scan's candidate windows: each has its own workspace and results, so that it never touches
+  // the scan's plan, window buffers or unfetched results, nor the other pass's
+  // Hudson FST, pi, dxy (tdsfs_diversity_*)
+  WindowPass div;
+  long long div_part_cap = 0;
+  int32_t* d_div_nsites = nullptr;
   double *d_div_pi1 = nullptr, *d_div_pi2 = nullptr, *d_div_dxy = nullptr, *d_div_fst = nullptr;
-  uint8_t* d_div_flags = nullptr;
   DivPart* d_div_part = nullptr;
-  void* d_div_tmp = nullptr;          // CUB scan scratch
-  bool div_ready = false, div_timed = false;
+  // Watterson's theta, Tajima's D (tdsfs_neutrality_*)
+  WindowPass neut;
+  long long neut_part_cap = 0;
+  int32_t *d_neut_S1 = nullptr, *d_neut_S2 = nullptr, *d_neut_nmax1 = nullptr, *d_neut_nmax2 = nullptr;
+  double *d_neut_pi1 = nullptr, *d_neut_pi2 = nullptr, *d_neut_tw1 = nullptr, *d_neut_tw2 = nullptr;
+  double *d_neut_d1 = nullptr, *d_neut_d2 = nullptr;
+  NeutPart* d_neut_part = nullptr;
+  double* d_neut_tab = nullptr;       // a1(n) for n in [0, neut_tab_n], then a2(n) for the same n
+  long long neut_tab_n = -1;
+  long long n_allele_max = 0;         // the largest n_i = ref_i + alt_i a row of the loaded data can reach
   // instrumentation
   cudaEvent_t ev[NEV] = {};
-  float ms[10] = {};
+  float ms[11] = {};
   long long launches = 0;
 };
 
@@ -320,8 +339,18 @@ static void free_data(tdsfs_ctx* c) {
   c->plan_W = -1;
   c->ws_ready = false;
   c->force_wide = false;
-  c->div_W = -1;
-  c->div_ready = false;
+  for (WindowPass* w : {&c->div, &c->neut}) {
+    w->W = -1;
+    w->ready = false;
+  }
+  c->n_allele_max = 0;
+}
+
+static void free_window_pass(WindowPass& w) {
+  dev_free(w.d_cand_off); dev_free(w.d_wlo); dev_free(w.d_whi); dev_free(w.d_wchrom); dev_free(w.d_count); dev_free(w.d_large);
+  dev_free(w.d_nlarge); dev_free(w.d_wstart); dev_free(w.d_wend); dev_free(w.d_nseg); dev_free(w.d_segoff); dev_free(w.d_flags);
+  if (w.d_tmp) cudaFree(w.d_tmp);
+  w.d_tmp = nullptr;
 }
 
 extern "C" void tdsfs_destroy(tdsfs_t* c) {
@@ -348,11 +377,13 @@ extern "C" void tdsfs_destroy(tdsfs_t* c) {
   dev_free(c->r_T1b); dev_free(c->r_flags); dev_free(c->d_scratch);
   for (int i = 0; i < NEV; ++i) if (c->ev[i]) cudaEventDestroy(c->ev[i]);
   dev_free(c->d_dxI); dev_free(c->d_ws); dev_free(c->d_gridbar); dev_free(c->d_stamps);
-  dev_free(c->d_div_cand_off); dev_free(c->d_div_wlo); dev_free(c->d_div_whi); dev_free(c->d_div_wchrom); dev_free(c->d_div_count);
-  dev_free(c->d_div_nsites); dev_free(c->d_div_large); dev_free(c->d_div_nlarge); dev_free(c->d_div_wstart); dev_free(c->d_div_wend);
-  dev_free(c->d_div_nseg); dev_free(c->d_div_segoff); dev_free(c->d_div_pi1); dev_free(c->d_div_pi2); dev_free(c->d_div_dxy);
-  dev_free(c->d_div_fst); dev_free(c->d_div_flags); dev_free(c->d_div_part);
-  if (c->d_div_tmp) cudaFree(c->d_div_tmp);
+  free_window_pass(c->div);
+  dev_free(c->d_div_nsites); dev_free(c->d_div_pi1); dev_free(c->d_div_pi2); dev_free(c->d_div_dxy); dev_free(c->d_div_fst);
+  dev_free(c->d_div_part);
+  free_window_pass(c->neut);
+  dev_free(c->d_neut_S1); dev_free(c->d_neut_S2); dev_free(c->d_neut_nmax1); dev_free(c->d_neut_nmax2); dev_free(c->d_neut_pi1);
+  dev_free(c->d_neut_pi2); dev_free(c->d_neut_tw1); dev_free(c->d_neut_tw2); dev_free(c->d_neut_d1); dev_free(c->d_neut_d2);
+  dev_free(c->d_neut_part); dev_free(c->d_neut_tab);
   cudaStreamDestroy(c->own_stream);
   cudaStreamDestroy(c->copy_stream);
   cudaStreamDestroy(c->plan_stream);
@@ -480,6 +511,7 @@ extern "C" int tdsfs_load_counts(tdsfs_t* c, const uint16_t* cnt, int64_t S, con
     CKR(adopt_or_upload(c, cnt, S * 4, &c->dCnt, &c->own_cnt, &c->pool_cnt, &c->cap_cnt));
     if (((uintptr_t)c->dCnt & 7) != 0) return fail(TDSFS_ERR_ARG, "cnt must be 8-byte aligned");
   }
+  c->n_allele_max = 2 * 65535;
   c->loaded = true;
   return finish(c);
 }
@@ -498,6 +530,7 @@ extern "C" int tdsfs_load_genotypes(tdsfs_t* c, const void* G, int64_t S, int32_
   const bool has_fix = fixups && n_fixups > 0;
   CKR(load_common(c, S, pos, (const long long*)chrom_off, C, snp_flags, has_fix));
   c->W1 = words1; c->W2 = words2; c->ns1 = ns1; c->ns2 = ns2;
+  c->n_allele_max = 2LL * std::max(ns1, ns2);
   const long long RW = words1 + words2;
   if (has_fix) {
     // flag bit2 marks rows that own fix-ups; build (or extend) the flag array on the host side
@@ -513,6 +546,11 @@ extern "C" int tdsfs_load_genotypes(tdsfs_t* c, const void* G, int64_t S, int32_
     for (auto& f : hf) {
       if (f.snp < 0 || f.snp >= S || (f.pop != 0 && f.pop != 1)) return fail(TDSFS_ERR_ARG, "fixup out of range");
       hflags[(size_t)f.snp] |= 4;
+    }
+    for (size_t i = 0, j; i < hf.size(); i = j) {  // the fix-ups of one (row, population) add up
+      long long dn[2] = {0, 0};
+      for (j = i; j < hf.size() && hf[j].snp == hf[i].snp; ++j) dn[hf[j].pop] += (long long)hf[j].dref + hf[j].dalt;
+      c->n_allele_max = std::max(c->n_allele_max, 2LL * std::max(ns1, ns2) + std::max(dn[0], dn[1]));
     }
     if (!c->own_flags) {
       void* d = nullptr;
@@ -1435,21 +1473,90 @@ extern "C" int tdsfs_window_spectra(tdsfs_t* c, int64_t window, uint64_t* s2, ui
   return 0;
 }
 
+// ------------------------------------------------------------------------------------------------ per-window passes
+// The candidate windows of (W, mode) for pass w: offsets cached per (size, mode), apart from the scan's and the other pass's.
+static int pass_candidates(tdsfs_ctx* c, WindowPass& w, long long W, bool snp_mode, long long* ncand) {
+  if (w.W != W || w.snp != (int)snp_mode) {
+    std::vector<long long> off;
+    CKR(candidates(c, W, snp_mode, off));
+    w.off_host.swap(off);
+    w.W = -1;
+    dev_free(w.d_cand_off);
+    CKR(dev_alloc(&w.d_cand_off, c->C + 1));
+    CK(cudaMemcpyAsync(w.d_cand_off, w.off_host.data(), (size_t)(c->C + 1) * 8, cudaMemcpyHostToDevice, c->stream));
+    w.W = W;
+    w.snp = snp_mode;
+  }
+  *ncand = w.off_host[c->C];
+  return 0;
+}
+
+// Per-window arrays of pass w for ncand windows; *grown when they were reallocated (the pass's own per-window results
+// follow), after the stream has drained.
+static int pass_buffers(tdsfs_ctx* c, WindowPass& w, long long ncand, bool* grown) {
+  *grown = ncand > w.cap;
+  if (*grown) {
+    CK(cudaStreamSynchronize(c->stream));  // a previous asynchronous call may still use the old arrays
+    dev_free(w.d_wlo); dev_free(w.d_whi); dev_free(w.d_wchrom); dev_free(w.d_count); dev_free(w.d_wstart); dev_free(w.d_wend);
+    dev_free(w.d_nseg); dev_free(w.d_segoff); dev_free(w.d_flags);
+    if (w.d_tmp) cudaFree(w.d_tmp);
+    w.d_tmp = nullptr;
+    CKR(dev_alloc(&w.d_wlo, ncand)); CKR(dev_alloc(&w.d_whi, ncand)); CKR(dev_alloc(&w.d_wchrom, ncand));
+    CKR(dev_alloc(&w.d_count, ncand)); CKR(dev_alloc(&w.d_wstart, ncand)); CKR(dev_alloc(&w.d_wend, ncand));
+    CKR(dev_alloc(&w.d_nseg, ncand + 1)); CKR(dev_alloc(&w.d_segoff, ncand + 1)); CKR(dev_alloc(&w.d_flags, ncand));
+    size_t tmp = 0;
+    CK(cub::DeviceScan::ExclusiveSum(nullptr, tmp, w.d_nseg, w.d_segoff, (int)(ncand + 1), c->stream));
+    CK(cudaMalloc(&w.d_tmp, std::max<size_t>(tmp, 16)));
+    w.tmp_bytes = std::max<size_t>(tmp, 16);
+    w.cap = ncand;
+  }
+  if (!w.d_large) {
+    CKR(dev_alloc(&w.d_large, 1));
+    CKR(dev_alloc(&w.d_nlarge, 1));
+  }
+  return 0;
+}
+
+// After the rows of a host upload still in flight: window boundaries of pass w's w.ncand candidates (K2 into its own
+// arrays) -> segments per window (k_div_nseg) -> the segment list (exclusive scan), on the handle's stream.
+static int pass_segments(tdsfs_ctx* c, WindowPass& w, long long W, bool snp_mode) {
+  cudaStream_t st = c->stream;
+  for (auto& ch : c->chunks) if (ch.ev) CK(cudaStreamWaitEvent(st, ch.ev, 0));
+  const long long ncand = w.ncand;
+  if (ncand == 0) return 0;
+  WinParams wp;
+  wp.pos = c->dPos; wp.chrom_off = c->d_off; wp.cand_off = w.d_cand_off; wp.C = c->C; wp.W = W; wp.ncand = ncand;
+  wp.wlo = w.d_wlo; wp.whi = w.d_whi; wp.wchrom = w.d_wchrom; wp.wstart = w.d_wstart; wp.wend = w.d_wend;
+  wp.large = w.d_large; wp.nlarge = w.d_nlarge;
+  wp.r_count = w.d_count; wp.r_flags = w.d_flags;  // K2 marks empty windows; the pass's finish kernel rewrites every entry
+  wp.wcap = 0x7FFFFFFF;
+  const int g2 = (int)((ncand + 255) / 256);
+  if (snp_mode) k2_bounds_snp<<<g2, 256, 0, st>>>(wp); else k2_bounds_bp<<<g2, 256, 0, st>>>(wp);
+  DivParams p;  // k_div_nseg reads the window rows and writes nseg only
+  memset(&p, 0, sizeof p);
+  p.wlo = w.d_wlo; p.whi = w.d_whi; p.ncand = ncand; p.nseg = w.d_nseg;
+  k_div_nseg<<<(int)((ncand + 1 + 255) / 256), 256, 0, st>>>(p);
+  size_t tmp = w.tmp_bytes;
+  CK(cub::DeviceScan::ExclusiveSum(w.d_tmp, tmp, w.d_nseg, w.d_segoff, (int)(ncand + 1), st));
+  c->launches += 3;
+  return 0;
+}
+
 // ------------------------------------------------------------------------------------------------ diversity (Hudson FST, pi, dxy)
 extern "C" int tdsfs_fetch_diversity(tdsfs_t* c, tdsfs_diversity_t* out, int64_t cap, int64_t* n_windows) {
   if (!c || !out) return fail(TDSFS_ERR_ARG, "NULL argument");
-  if (!c->div_ready) return fail(TDSFS_ERR_STATE, "no diversity results (tdsfs_diversity_bp / _snp first)");
-  if (cap < c->div_ncand) return fail(TDSFS_ERR_ARG, "result capacity %lld < %lld candidate windows", (long long)cap, c->div_ncand);
+  if (!c->div.ready) return fail(TDSFS_ERR_STATE, "no diversity results (tdsfs_diversity_bp / _snp first)");
+  if (cap < c->div.ncand) return fail(TDSFS_ERR_ARG, "result capacity %lld < %lld candidate windows", (long long)cap, c->div.ncand);
   CK(cudaSetDevice(c->device));
   cudaStream_t st = c->stream;
-  const size_t n = (size_t)c->div_ncand;
+  const size_t n = (size_t)c->div.ncand;
 #define D2H(dst, src, T) \
   if (out->dst && n) CK(cudaMemcpyAsync(out->dst, c->src, n * sizeof(T), cudaMemcpyDeviceToHost, st))
-  D2H(chrom, d_div_wchrom, int32_t);
-  D2H(start, d_div_wstart, long long);
-  D2H(end, d_div_wend, long long);
-  D2H(snp_count, d_div_count, int32_t);
-  D2H(flags, d_div_flags, uint8_t);
+  D2H(chrom, div.d_wchrom, int32_t);
+  D2H(start, div.d_wstart, long long);
+  D2H(end, div.d_wend, long long);
+  D2H(snp_count, div.d_count, int32_t);
+  D2H(flags, div.d_flags, uint8_t);
   D2H(n_sites, d_div_nsites, int32_t);
   D2H(pi_p1, d_div_pi1, double);
   D2H(pi_p2, d_div_pi2, double);
@@ -1457,28 +1564,17 @@ extern "C" int tdsfs_fetch_diversity(tdsfs_t* c, tdsfs_diversity_t* out, int64_t
   D2H(fst, d_div_fst, double);
 #undef D2H
   CK(cudaStreamSynchronize(st));
-  if (n_windows) *n_windows = c->div_ncand;
+  if (n_windows) *n_windows = c->div.ncand;
   return 0;
 }
 
 static int ensure_div_buffers(tdsfs_ctx* c, long long ncand, long long parts) {
-  if (ncand > c->div_cap) {
-    CK(cudaStreamSynchronize(c->stream));  // a previous asynchronous call may still use the old arrays
-    dev_free(c->d_div_wlo); dev_free(c->d_div_whi); dev_free(c->d_div_wchrom); dev_free(c->d_div_count); dev_free(c->d_div_nsites);
-    dev_free(c->d_div_wstart); dev_free(c->d_div_wend); dev_free(c->d_div_nseg); dev_free(c->d_div_segoff); dev_free(c->d_div_pi1);
-    dev_free(c->d_div_pi2); dev_free(c->d_div_dxy); dev_free(c->d_div_fst); dev_free(c->d_div_flags);
-    if (c->d_div_tmp) cudaFree(c->d_div_tmp);
-    c->d_div_tmp = nullptr;
-    CKR(dev_alloc(&c->d_div_wlo, ncand)); CKR(dev_alloc(&c->d_div_whi, ncand)); CKR(dev_alloc(&c->d_div_wchrom, ncand));
-    CKR(dev_alloc(&c->d_div_count, ncand)); CKR(dev_alloc(&c->d_div_nsites, ncand)); CKR(dev_alloc(&c->d_div_wstart, ncand));
-    CKR(dev_alloc(&c->d_div_wend, ncand)); CKR(dev_alloc(&c->d_div_nseg, ncand + 1)); CKR(dev_alloc(&c->d_div_segoff, ncand + 1));
-    CKR(dev_alloc(&c->d_div_pi1, ncand)); CKR(dev_alloc(&c->d_div_pi2, ncand)); CKR(dev_alloc(&c->d_div_dxy, ncand));
-    CKR(dev_alloc(&c->d_div_fst, ncand)); CKR(dev_alloc(&c->d_div_flags, ncand));
-    size_t tmp = 0;
-    CK(cub::DeviceScan::ExclusiveSum(nullptr, tmp, c->d_div_nseg, c->d_div_segoff, (int)(ncand + 1), c->stream));
-    CK(cudaMalloc(&c->d_div_tmp, std::max<size_t>(tmp, 16)));
-    c->div_tmp_bytes = std::max<size_t>(tmp, 16);
-    c->div_cap = ncand;
+  bool grown;
+  CKR(pass_buffers(c, c->div, ncand, &grown));
+  if (grown) {
+    dev_free(c->d_div_nsites); dev_free(c->d_div_pi1); dev_free(c->d_div_pi2); dev_free(c->d_div_dxy); dev_free(c->d_div_fst);
+    CKR(dev_alloc(&c->d_div_nsites, ncand)); CKR(dev_alloc(&c->d_div_pi1, ncand)); CKR(dev_alloc(&c->d_div_pi2, ncand));
+    CKR(dev_alloc(&c->d_div_dxy, ncand)); CKR(dev_alloc(&c->d_div_fst, ncand));
   }
   if (parts > c->div_part_cap) {
     CK(cudaStreamSynchronize(c->stream));
@@ -1486,73 +1582,47 @@ static int ensure_div_buffers(tdsfs_ctx* c, long long ncand, long long parts) {
     CKR(dev_alloc(&c->d_div_part, parts));
     c->div_part_cap = parts;
   }
-  if (!c->d_div_large) {
-    CKR(dev_alloc(&c->d_div_large, 1));
-    CKR(dev_alloc(&c->d_div_nlarge, 1));
-  }
   return 0;
 }
 
-// Per-window Hudson FST, pi and dxy over the candidate windows of (W, mode), in the order of tdsfs_scan_*: window
-// boundaries (K2 into the diversity pass's own arrays) -> segments per window -> their prefix sum (device) -> k_diversity
-// (one warp per segment of DIV_SEG rows) -> k_div_finish.  Needs loaded data only; no host round trip when out == NULL.
+// Per-window Hudson FST, pi and dxy over the candidate windows of (W, mode), in the order of tdsfs_scan_*: the segment list
+// (pass_segments) -> k_diversity (one warp per segment of DIV_SEG rows) -> k_div_finish.  Needs loaded data only; no host
+// round trip when out == NULL.
 static int diversity(tdsfs_ctx* c, long long W, bool snp_mode, tdsfs_diversity_t* out, int64_t cap, int64_t* n_windows) {
   if (!c || W < 1) return fail(TDSFS_ERR_ARG, "bad argument");
   if (!c->loaded) return fail(TDSFS_ERR_STATE, "load data first");
   CK(cudaSetDevice(c->device));
   NvtxRange nvtx("tdsfs:diversity (FST, pi, dxy)");
   cudaStream_t st = c->stream;
-  if (c->div_W != W || c->div_snp != (int)snp_mode) {  // candidate offsets cached per (size, mode), apart from the scan's
-    std::vector<long long> off;
-    CKR(candidates(c, W, snp_mode, off));
-    c->div_off_host.swap(off);
-    c->div_W = -1;
-    dev_free(c->d_div_cand_off);
-    CKR(dev_alloc(&c->d_div_cand_off, c->C + 1));
-    CK(cudaMemcpyAsync(c->d_div_cand_off, c->div_off_host.data(), (size_t)(c->C + 1) * 8, cudaMemcpyHostToDevice, st));
-    c->div_W = W;
-    c->div_snp = snp_mode;
-  }
-  const long long ncand = c->div_off_host[c->C];
+  long long ncand;
+  CKR(pass_candidates(c, c->div, W, snp_mode, &ncand));
   if (out && cap < ncand) return fail(TDSFS_ERR_ARG, "result capacity %lld < %lld candidate windows", (long long)cap, ncand);
   // windows never overlap, so sum_w ceil(rows_w / SEG) <= S / SEG + ncand
   const long long max_parts = ncand + c->S / DIV_SEG + 1;
   CKR(ensure_div_buffers(c, ncand, max_parts));
-  c->div_ready = false;
-  c->div_ncand = ncand;
-  for (auto& ch : c->chunks) if (ch.ev) CK(cudaStreamWaitEvent(st, ch.ev, 0));  // rows of a host upload still in flight
-  if (ncand == 0) CK(cudaEventRecord(c->ev[EV_D0], st));
+  c->div.ready = false;
+  c->div.ncand = ncand;
+  CKR(pass_segments(c, c->div, W, snp_mode));
+  CK(cudaEventRecord(c->ev[EV_D0], st));
   if (ncand > 0) {
-    WinParams w;
-    w.pos = c->dPos; w.chrom_off = c->d_off; w.cand_off = c->d_div_cand_off; w.C = c->C; w.W = W; w.ncand = ncand;
-    w.wlo = c->d_div_wlo; w.whi = c->d_div_whi; w.wchrom = c->d_div_wchrom; w.wstart = c->d_div_wstart; w.wend = c->d_div_wend;
-    w.large = c->d_div_large; w.nlarge = c->d_div_nlarge;
-    w.r_count = c->d_div_count; w.r_flags = c->d_div_flags;  // K2 marks empty windows; k_div_finish rewrites every entry
-    w.wcap = 0x7FFFFFFF;
-    const int g2 = (int)((ncand + 255) / 256);
-    if (snp_mode) k2_bounds_snp<<<g2, 256, 0, st>>>(w); else k2_bounds_bp<<<g2, 256, 0, st>>>(w);
     DivParams p;
     memset(&p, 0, sizeof p);
     fill_key_params(c, p.k);
-    p.wlo = c->d_div_wlo; p.whi = c->d_div_whi; p.ncand = ncand; p.nseg = c->d_div_nseg; p.segoff = c->d_div_segoff;
-    p.part = c->d_div_part; p.snp_count = c->d_div_count; p.n_sites = c->d_div_nsites; p.pi1 = c->d_div_pi1; p.pi2 = c->d_div_pi2;
-    p.dxy = c->d_div_dxy; p.fst = c->d_div_fst; p.flags = c->d_div_flags;
-    k_div_nseg<<<(int)((ncand + 1 + 255) / 256), 256, 0, st>>>(p);
-    size_t tmp = c->div_tmp_bytes;
-    CK(cub::DeviceScan::ExclusiveSum(c->d_div_tmp, tmp, c->d_div_nseg, c->d_div_segoff, (int)(ncand + 1), st));
-    CK(cudaEventRecord(c->ev[EV_D0], st));
+    p.wlo = c->div.d_wlo; p.whi = c->div.d_whi; p.ncand = ncand; p.nseg = c->div.d_nseg; p.segoff = c->div.d_segoff;
+    p.part = c->d_div_part; p.snp_count = c->div.d_count; p.n_sites = c->d_div_nsites; p.pi1 = c->d_div_pi1; p.pi2 = c->d_div_pi2;
+    p.dxy = c->d_div_dxy; p.fst = c->d_div_fst; p.flags = c->div.d_flags;
     // one warp per segment; the grid covers the bound on the segment count and warps past the actual count return at once
     void (*kern)(DivParams) = k_diversity<0, 0>;
     if (c->dG && c->W1 == 32 && c->W2 == 32) kern = k_diversity<32, 32>;       // 500 + 500 diploids (BASELINE config 5)
     else if (c->dG && c->W1 == 14 && c->W2 == 14) kern = k_diversity<14, 14>;  // 200 + 200 diploids (BASELINE config 4)
     kern<<<(unsigned)((max_parts + DIV_WARPS - 1) / DIV_WARPS), DIV_WARPS * 32, 0, st>>>(p);
     k_div_finish<<<(int)((ncand + 255) / 256), 256, 0, st>>>(p);
-    c->launches += 5;
+    c->launches += 2;
     CK(cudaGetLastError());
   }
   CK(cudaEventRecord(c->ev[EV_D1], st));
-  c->div_timed = true;
-  c->div_ready = true;
+  c->div.timed = true;
+  c->div.ready = true;
   if (out) return tdsfs_fetch_diversity(c, out, cap, n_windows);
   if (n_windows) *n_windows = ncand;
   return finish(c);
@@ -1563,6 +1633,125 @@ extern "C" int tdsfs_diversity_bp(tdsfs_t* c, int64_t W, tdsfs_diversity_t* out,
 }
 extern "C" int tdsfs_diversity_snp(tdsfs_t* c, int64_t N, tdsfs_diversity_t* out, int64_t cap, int64_t* n_windows) {
   return diversity(c, N, true, out, cap, n_windows);
+}
+
+// ------------------------------------------------------------------------------------------------ neutrality (theta_W, Tajima's D)
+extern "C" int tdsfs_fetch_neutrality(tdsfs_t* c, tdsfs_neutrality_t* out, int64_t cap, int64_t* n_windows) {
+  if (!c || !out) return fail(TDSFS_ERR_ARG, "NULL argument");
+  if (!c->neut.ready) return fail(TDSFS_ERR_STATE, "no neutrality results (tdsfs_neutrality_bp / _snp first)");
+  if (cap < c->neut.ncand) return fail(TDSFS_ERR_ARG, "result capacity %lld < %lld candidate windows", (long long)cap, c->neut.ncand);
+  CK(cudaSetDevice(c->device));
+  cudaStream_t st = c->stream;
+  const size_t n = (size_t)c->neut.ncand;
+#define D2H(dst, src, T) \
+  if (out->dst && n) CK(cudaMemcpyAsync(out->dst, c->src, n * sizeof(T), cudaMemcpyDeviceToHost, st))
+  D2H(chrom, neut.d_wchrom, int32_t);
+  D2H(start, neut.d_wstart, long long);
+  D2H(end, neut.d_wend, long long);
+  D2H(snp_count, neut.d_count, int32_t);
+  D2H(flags, neut.d_flags, uint8_t);
+  D2H(n_seg_p1, d_neut_S1, int32_t);
+  D2H(n_seg_p2, d_neut_S2, int32_t);
+  D2H(n_max_p1, d_neut_nmax1, int32_t);
+  D2H(n_max_p2, d_neut_nmax2, int32_t);
+  D2H(theta_pi_p1, d_neut_pi1, double);
+  D2H(theta_pi_p2, d_neut_pi2, double);
+  D2H(theta_w_p1, d_neut_tw1, double);
+  D2H(theta_w_p2, d_neut_tw2, double);
+  D2H(tajima_d_p1, d_neut_d1, double);
+  D2H(tajima_d_p2, d_neut_d2, double);
+#undef D2H
+  CK(cudaStreamSynchronize(st));
+  if (n_windows) *n_windows = c->neut.ncand;
+  return 0;
+}
+
+static int ensure_neut_buffers(tdsfs_ctx* c, long long ncand, long long parts) {
+  bool grown;
+  CKR(pass_buffers(c, c->neut, ncand, &grown));
+  if (grown) {
+    dev_free(c->d_neut_S1); dev_free(c->d_neut_S2); dev_free(c->d_neut_nmax1); dev_free(c->d_neut_nmax2);
+    dev_free(c->d_neut_pi1); dev_free(c->d_neut_pi2); dev_free(c->d_neut_tw1); dev_free(c->d_neut_tw2);
+    dev_free(c->d_neut_d1); dev_free(c->d_neut_d2);
+    CKR(dev_alloc(&c->d_neut_S1, ncand)); CKR(dev_alloc(&c->d_neut_S2, ncand)); CKR(dev_alloc(&c->d_neut_nmax1, ncand));
+    CKR(dev_alloc(&c->d_neut_nmax2, ncand)); CKR(dev_alloc(&c->d_neut_pi1, ncand)); CKR(dev_alloc(&c->d_neut_pi2, ncand));
+    CKR(dev_alloc(&c->d_neut_tw1, ncand)); CKR(dev_alloc(&c->d_neut_tw2, ncand)); CKR(dev_alloc(&c->d_neut_d1, ncand));
+    CKR(dev_alloc(&c->d_neut_d2, ncand));
+  }
+  if (parts > c->neut_part_cap) {
+    CK(cudaStreamSynchronize(c->stream));
+    dev_free(c->d_neut_part);
+    CKR(dev_alloc(&c->d_neut_part, parts));
+    c->neut_part_cap = parts;
+  }
+  // a1(n) and a2(n) for every n a loaded row can reach, summed in ascending k; built again only when a load reaches a
+  // larger n (the entries of a longer table are the same numbers)
+  if (c->n_allele_max > c->neut_tab_n) {
+    const long long m = c->n_allele_max + 1;
+    std::vector<double> t((size_t)(2 * m), 0.0);
+    for (long long n = 2; n < m; ++n) {
+      const double k = (double)(n - 1);
+      t[n] = t[n - 1] + 1.0 / k;
+      t[m + n] = t[m + n - 1] + 1.0 / (k * k);
+    }
+    CK(cudaStreamSynchronize(c->stream));  // a previous asynchronous call may still read the old table
+    c->neut_tab_n = -1;
+    dev_free(c->d_neut_tab);
+    CKR(dev_alloc(&c->d_neut_tab, 2 * m));
+    CK(cudaMemcpyAsync(c->d_neut_tab, t.data(), (size_t)(2 * m) * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+    c->neut_tab_n = m - 1;
+  }
+  return 0;
+}
+
+// Per-window, per-population Watterson's theta and Tajima's D over the candidate windows of (W, mode), in the order of
+// tdsfs_scan_*: the segment list (pass_segments) -> k_neutrality (one warp per segment of DIV_SEG rows) -> k_neut_finish.
+// Needs loaded data only; no host round trip when out == NULL (past the first call after a load that needs a larger table).
+static int neutrality(tdsfs_ctx* c, long long W, bool snp_mode, tdsfs_neutrality_t* out, int64_t cap, int64_t* n_windows) {
+  if (!c || W < 1) return fail(TDSFS_ERR_ARG, "bad argument");
+  if (!c->loaded) return fail(TDSFS_ERR_STATE, "load data first");
+  CK(cudaSetDevice(c->device));
+  NvtxRange nvtx("tdsfs:neutrality (theta_W, Tajima's D)");
+  cudaStream_t st = c->stream;
+  long long ncand;
+  CKR(pass_candidates(c, c->neut, W, snp_mode, &ncand));
+  if (out && cap < ncand) return fail(TDSFS_ERR_ARG, "result capacity %lld < %lld candidate windows", (long long)cap, ncand);
+  const long long max_parts = ncand + c->S / DIV_SEG + 1;  // as in diversity()
+  CKR(ensure_neut_buffers(c, ncand, max_parts));
+  c->neut.ready = false;
+  c->neut.ncand = ncand;
+  CKR(pass_segments(c, c->neut, W, snp_mode));
+  CK(cudaEventRecord(c->ev[EV_N0], st));
+  if (ncand > 0) {
+    NeutParams p;
+    memset(&p, 0, sizeof p);
+    fill_key_params(c, p.k);
+    p.wlo = c->neut.d_wlo; p.whi = c->neut.d_whi; p.ncand = ncand; p.segoff = c->neut.d_segoff; p.part = c->d_neut_part;
+    p.a1 = c->d_neut_tab; p.a2 = c->d_neut_tab + c->neut_tab_n + 1;
+    p.snp_count = c->neut.d_count; p.S1 = c->d_neut_S1; p.S2 = c->d_neut_S2; p.nmax1 = c->d_neut_nmax1; p.nmax2 = c->d_neut_nmax2;
+    p.theta_pi1 = c->d_neut_pi1; p.theta_pi2 = c->d_neut_pi2; p.theta_w1 = c->d_neut_tw1; p.theta_w2 = c->d_neut_tw2;
+    p.tajd1 = c->d_neut_d1; p.tajd2 = c->d_neut_d2; p.flags = c->neut.d_flags;
+    void (*kern)(NeutParams) = k_neutrality<0, 0>;
+    if (c->dG && c->W1 == 32 && c->W2 == 32) kern = k_neutrality<32, 32>;
+    else if (c->dG && c->W1 == 14 && c->W2 == 14) kern = k_neutrality<14, 14>;
+    kern<<<(unsigned)((max_parts + DIV_WARPS - 1) / DIV_WARPS), DIV_WARPS * 32, 0, st>>>(p);
+    k_neut_finish<<<(int)((ncand + 255) / 256), 256, 0, st>>>(p);
+    c->launches += 2;
+    CK(cudaGetLastError());
+  }
+  CK(cudaEventRecord(c->ev[EV_N1], st));
+  c->neut.timed = true;
+  c->neut.ready = true;
+  if (out) return tdsfs_fetch_neutrality(c, out, cap, n_windows);
+  if (n_windows) *n_windows = ncand;
+  return finish(c);
+}
+
+extern "C" int tdsfs_neutrality_bp(tdsfs_t* c, int64_t W, tdsfs_neutrality_t* out, int64_t cap, int64_t* n_windows) {
+  return neutrality(c, W, false, out, cap, n_windows);
+}
+extern "C" int tdsfs_neutrality_snp(tdsfs_t* c, int64_t N, tdsfs_neutrality_t* out, int64_t cap, int64_t* n_windows) {
+  return neutrality(c, N, true, out, cap, n_windows);
 }
 
 // ------------------------------------------------------------------------------------------------ explicit likelihood
@@ -1635,7 +1824,7 @@ extern "C" int tdsfs_timings(tdsfs_t* c, float* ms, int32_t n) {
   if (!c || !ms) return fail(TDSFS_ERR_ARG, "NULL argument");
   CK(cudaSetDevice(c->device));
   CK(cudaStreamSynchronize(c->stream));
-  for (int i = 0; i < 10; ++i) c->ms[i] = 0.f;
+  for (int i = 0; i < 11; ++i) c->ms[i] = 0.f;
   if (c->keys_ready) cudaEventElapsedTime(&c->ms[0], c->ev[EV_BG0], c->ev[EV_K1]);
   if (c->fin_timed) cudaEventElapsedTime(&c->ms[1], c->ev[EV_FIN0], c->ev[EV_FIN1]);
   if (c->results_ready) {
@@ -1648,9 +1837,10 @@ extern "C" int tdsfs_timings(tdsfs_t* c, float* ms, int32_t n) {
   }
   c->ms[5] = c->ms[0];
   if (c->x_timed) cudaEventElapsedTime(&c->ms[8], c->ev[EV_X0], c->ev[EV_X1]);
-  if (c->div_timed) cudaEventElapsedTime(&c->ms[9], c->ev[EV_D0], c->ev[EV_D1]);
+  if (c->div.timed) cudaEventElapsedTime(&c->ms[9], c->ev[EV_D0], c->ev[EV_D1]);
+  if (c->neut.timed) cudaEventElapsedTime(&c->ms[10], c->ev[EV_N0], c->ev[EV_N1]);
   cudaGetLastError();
-  for (int i = 0; i < n && i < 10; ++i) ms[i] = c->ms[i];
+  for (int i = 0; i < n && i < 11; ++i) ms[i] = c->ms[i];
   return 0;
 }
 

@@ -1,6 +1,7 @@
-// tdsfs_diversity.cuh -- per-window Hudson FST, pi and dxy (DESIGN.md section 7, "Diversity: Hudson FST, pi, dxy").
-// Included by tdsfs.cu after tdsfs_kernels.cuh and tdsfs_fused.cuh.  No reference counterpart: the reference's users get
-// the FST column of their tables from pixy, run separately over the same VCF.
+// tdsfs_diversity.cuh -- per-window Hudson FST, pi and dxy, and per-population Watterson's theta and Tajima's D
+// (DESIGN.md section 7).  Included by tdsfs.cu after tdsfs_kernels.cuh and tdsfs_fused.cuh.  No reference counterpart: the
+// reference's users get the FST column of their tables from pixy, and Tajima's D from scikit-allel, run separately over
+// the same VCF.
 //
 // Per SNP that passes the spectrum filters (snp_flags bit0) with n_i = ref_i + alt_i >= 2 in both populations, in fp64:
 //   pi_i = 2 ref_i alt_i / (n_i (n_i - 1)),   dxy = (ref_1 alt_2 + alt_1 ref_2) / (n_1 n_2)
@@ -14,7 +15,7 @@
 namespace tdsfs {
 
 constexpr int DIV_SEG = 1024;   // rows per segment (a multiple of 32)
-constexpr int DIV_WARPS = 8;    // warps per CTA of k_diversity: one warp per segment
+constexpr int DIV_WARPS = 8;    // warps per CTA of k_diversity and k_neutrality: one warp per segment
 
 struct DivPart {  // sums of one segment
   double pi1, pi2, dxy;
@@ -149,6 +150,135 @@ __global__ void __launch_bounds__(256) k_div_finish(const __grid_constant__ DivP
   p.pi2[id] = pi2;
   p.dxy[id] = dxy;
   p.fst[id] = dxy == 0.0 ? __longlong_as_double(0x7FF8000000000000LL) : 1.0 - (pi1 + pi2) / (2.0 * dxy);
+  p.flags[id] = __ldg(p.whi + id) == __ldg(p.wlo + id) ? TDSFS_F_EMPTY : 0;
+}
+
+// ------------------------------------------------------------------------------------------------ neutrality
+// Per population i, over the rows that pass the spectrum filters: S_i segregating sites (ref_i > 0 and alt_i > 0),
+// n_max_i the largest n_i, theta_pi_i the sum of 2 ref_i alt_i / (n_i (n_i - 1)) over the rows with n_i >= 2 (the pi_i term
+// of the FST pass, summed in the same order, but not restricted to rows where the other population has n >= 2); then
+// Watterson's theta S_i / a1(n_max_i) and Tajima's D (Tajima 1989) at n = n_max_i.  A window's results depend on its rows
+// alone, as the FST pass's do.
+
+struct NeutPart {  // sums of one segment
+  double theta_pi1, theta_pi2;
+  int S1, S2, nmax1, nmax2, snp_count;
+};
+
+struct NeutParams {
+  KeyParams k;                 // source rows, sample columns, snp_flags + fix-ups
+  const int32_t* wlo;          // [ncand] first row of each candidate window
+  const int32_t* whi;          // [ncand] one past its last row
+  long long ncand;
+  const long long* segoff;     // [ncand + 1] the segment list (k_div_nseg + exclusive scan)
+  NeutPart* part;              // [segments]
+  const double* a1;            // [tab_n + 1] a1(n) = sum_{k=1}^{n-1} 1/k, ascending k; a1(0) = a1(1) = 0
+  const double* a2;            // [tab_n + 1] a2(n) = sum_{k=1}^{n-1} 1/k^2
+  int32_t* snp_count;          // [ncand] outputs
+  int32_t* S1;
+  int32_t* S2;
+  int32_t* nmax1;
+  int32_t* nmax2;
+  double* theta_pi1;
+  double* theta_pi2;
+  double* theta_w1;
+  double* theta_w2;
+  double* tajd1;
+  double* tajd2;
+  uint8_t* flags;
+};
+
+// One warp per segment, walking aligned 32-row blocks as k_diversity does.  Only the theta_pi terms depend on the order in
+// which they are added, so only they move to the owning lane; the integer counts and maxima are reduced at the end.
+template <int TW1, int TW2>
+__global__ void __launch_bounds__(DIV_WARPS * 32) k_neutrality(const __grid_constant__ NeutParams p) {
+  const int lane = threadIdx.x & 31;
+  const long long g = (long long)blockIdx.x * DIV_WARPS + (threadIdx.x >> 5);
+  if (g >= __ldg(p.segoff + p.ncand)) return;
+  // window of segment g, as in k_diversity
+  long long lo = 0, hi = p.ncand;
+  while (hi - lo > 1) {
+    const long long mid = (lo + hi) >> 1;
+    if (__ldg(p.segoff + mid) <= g) lo = mid; else hi = mid;
+  }
+  const long long r0 = (long long)__ldg(p.wlo + lo) + (g - __ldg(p.segoff + lo)) * DIV_SEG;
+  const long long r1 = min(r0 + DIV_SEG, (long long)__ldg(p.whi + lo));
+  const int src = (lane + (int)(r0 & 31)) & 31;  // the lane that loads the row this lane owns
+  double pi1 = 0.0, pi2 = 0.0;
+  int S1 = 0, S2 = 0, nmax1 = 0, nmax2 = 0, snp_count = 0;
+  for (long long b = r0 & ~31LL; b < r1; b += 32) {
+    const long long s = b + lane;
+    double t1 = 0.0, t2 = 0.0;
+    if (s >= r0 && s < r1) {
+      int ref1, alt1, ref2, alt2;
+      div_counts<TW1, TW2>(p.k, s, ref1, alt1, ref2, alt2);
+      snp_count += p.k.flags ? (__ldg(p.k.flags + s) >> 1) & 1 : 1;
+      if (row_filters(p.k, s, ref1, alt1, ref2, alt2)) {
+        const long long n1 = ref1 + alt1, n2 = ref2 + alt2;
+        S1 += ref1 > 0 && alt1 > 0;
+        S2 += ref2 > 0 && alt2 > 0;
+        nmax1 = max(nmax1, (int)n1);
+        nmax2 = max(nmax2, (int)n2);
+        if (n1 >= 2) t1 = (double)(2LL * ref1 * alt1) / (double)(n1 * (n1 - 1));
+        if (n2 >= 2) t2 = (double)(2LL * ref2 * alt2) / (double)(n2 * (n2 - 1));
+      }
+    }
+    // a row that adds no term adds +0.0, which leaves the (never negative zero) sum bitwise unchanged
+    pi1 += __shfl_sync(0xffffffffu, t1, src);
+    pi2 += __shfl_sync(0xffffffffu, t2, src);
+  }
+#pragma unroll
+  for (int o = 16; o; o >>= 1) {
+    pi1 += __shfl_xor_sync(0xffffffffu, pi1, o);
+    pi2 += __shfl_xor_sync(0xffffffffu, pi2, o);
+  }
+  S1 = __reduce_add_sync(0xffffffffu, S1);
+  S2 = __reduce_add_sync(0xffffffffu, S2);
+  snp_count = __reduce_add_sync(0xffffffffu, snp_count);
+  nmax1 = __reduce_max_sync(0xffffffffu, nmax1);
+  nmax2 = __reduce_max_sync(0xffffffffu, nmax2);
+  if (lane == 0) p.part[g] = NeutPart{pi1, pi2, S1, S2, nmax1, nmax2, snp_count};
+}
+
+// Watterson's theta and Tajima's D of one population from (theta_pi, S, n_max); NaN where undefined.
+__device__ __forceinline__ void tajima(const NeutParams& p, double pi, int S, int n, double& theta_w, double& d) {
+  const double nan = __longlong_as_double(0x7FF8000000000000LL);
+  theta_w = nan;
+  d = nan;
+  if (n < 2) return;
+  const double a1 = __ldg(p.a1 + n), a2 = __ldg(p.a2 + n), nn = n, s = S;
+  theta_w = s / a1;
+  if (S < 3) return;
+  const double b1 = (nn + 1.0) / (3.0 * (nn - 1.0));
+  const double b2 = 2.0 * (nn * nn + nn + 3.0) / (9.0 * nn * (nn - 1.0));
+  const double c1 = b1 - 1.0 / a1;
+  const double c2 = b2 - (nn + 2.0) / (a1 * nn) + a2 / (a1 * a1);
+  const double e1 = c1 / a1, e2 = c2 / (a1 * a1 + a2);
+  const double var = e1 * s + e2 * s * (s - 1.0);
+  if (var > 0.0) d = (pi - theta_w) / sqrt(var);
+}
+
+// One thread per window: its segment parts in segment order (maxima for n_max), then theta_W and Tajima's D.
+__global__ void __launch_bounds__(256) k_neut_finish(const __grid_constant__ NeutParams p) {
+  const long long id = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (id >= p.ncand) return;
+  double pi1 = 0.0, pi2 = 0.0;
+  int S1 = 0, S2 = 0, nmax1 = 0, nmax2 = 0, snp_count = 0;
+  for (long long g = __ldg(p.segoff + id), e = __ldg(p.segoff + id + 1); g < e; ++g) {
+    const NeutPart q = p.part[g];
+    pi1 += q.theta_pi1; pi2 += q.theta_pi2;
+    S1 += q.S1; S2 += q.S2; snp_count += q.snp_count;
+    nmax1 = max(nmax1, q.nmax1); nmax2 = max(nmax2, q.nmax2);
+  }
+  double tw1, tw2, d1, d2;
+  tajima(p, pi1, S1, nmax1, tw1, d1);
+  tajima(p, pi2, S2, nmax2, tw2, d2);
+  p.snp_count[id] = snp_count;
+  p.S1[id] = S1; p.S2[id] = S2;
+  p.nmax1[id] = nmax1; p.nmax2[id] = nmax2;
+  p.theta_pi1[id] = pi1; p.theta_pi2[id] = pi2;
+  p.theta_w1[id] = tw1; p.theta_w2[id] = tw2;
+  p.tajd1[id] = d1; p.tajd2[id] = d2;
   p.flags[id] = __ldg(p.whi + id) == __ldg(p.wlo + id) ? TDSFS_F_EMPTY : 0;
 }
 

@@ -23,6 +23,7 @@ EXPORTS = [
     "tdsfs_poisson_score", "tdsfs_peer_export", "tdsfs_peer_import", "tdsfs_peer_allreduce_background", "tdsfs_peer_reduce_finalize", "tdsfs_peer_close",
     "tdsfs_synth_genotypes", "tdsfs_timings", "tdsfs_launch_count", "tdsfs_scan_info", "tdsfs_tail_stamps", "tdsfs_version",
     "tdsfs_diversity_bp", "tdsfs_diversity_snp", "tdsfs_fetch_diversity",
+    "tdsfs_neutrality_bp", "tdsfs_neutrality_snp", "tdsfs_fetch_neutrality",
 ]
 
 
@@ -58,6 +59,18 @@ class Diversity(C.Structure):
 
 DIVERSITY_DTYPES = dict(chrom=np.int32, start=np.int64, end=np.int64, snp_count=np.int32, flags=np.uint8, n_sites=np.int32,
                         pi_p1=np.float64, pi_p2=np.float64, dxy=np.float64, fst=np.float64)
+
+
+class Neutrality(C.Structure):
+    _fields_ = [(k, C.c_void_p) for k in ("chrom", "start", "end", "snp_count", "flags", "n_seg_p1", "n_seg_p2", "n_max_p1",
+                                          "n_max_p2", "theta_pi_p1", "theta_pi_p2", "theta_w_p1", "theta_w_p2",
+                                          "tajima_d_p1", "tajima_d_p2")]
+
+
+NEUTRALITY_DTYPES = dict(chrom=np.int32, start=np.int64, end=np.int64, snp_count=np.int32, flags=np.uint8, n_seg_p1=np.int32,
+                         n_seg_p2=np.int32, n_max_p1=np.int32, n_max_p2=np.int32, theta_pi_p1=np.float64,
+                         theta_pi_p2=np.float64, theta_w_p1=np.float64, theta_w_p2=np.float64, tajima_d_p1=np.float64,
+                         tajima_d_p2=np.float64)
 
 _lib = None
 
@@ -279,6 +292,33 @@ class Handle:
         self._check(self._L.tdsfs_fetch_diversity(self._h, C.byref(r), C.c_int64(cap), C.byref(n)))
         return {k: v[:n.value] for k, v in arrs.items()}
 
+    def neutrality(self, size, snp_mode=False, fetch=True):
+        """Per-window, per-population Watterson's theta and Tajima's D over the candidate windows of (size, mode), in scan
+        order (tdsfs_neutrality_*): n_seg_p* segregating sites, n_max_p* the largest called-allele count, theta_pi_p* /
+        theta_w_p* absolute (not per-bp) estimators, tajima_d_p* at n = n_max_p* (NaN with fewer than 3 segregating sites).
+        Returns a dict of arrays (chrom / start / end / snp_count / flags as the scan's), or the candidate count when
+        fetch=False (results stay on the device: fetch_neutrality)."""
+        f = self._L.tdsfs_neutrality_snp if snp_mode else self._L.tdsfs_neutrality_bp
+        n = C.c_int64()
+        if not fetch:
+            self._check(f(self._h, C.c_int64(size), None, C.c_int64(0), C.byref(n)))
+            return n.value
+        cap = self.candidates(size, snp_mode)
+        arrs, r = self._alloc_neutrality(cap)
+        self._check(f(self._h, C.c_int64(size), C.byref(r), C.c_int64(cap), C.byref(n)))
+        return {k: v[:n.value] for k, v in arrs.items()}
+
+    @staticmethod
+    def _alloc_neutrality(n):
+        arrs = {k: np.zeros(max(n, 1), dtype=dt) for k, dt in NEUTRALITY_DTYPES.items()}
+        return arrs, Neutrality(**{k: v.ctypes.data for k, v in arrs.items()})
+
+    def fetch_neutrality(self, cap):
+        arrs, r = self._alloc_neutrality(cap)
+        n = C.c_int64()
+        self._check(self._L.tdsfs_fetch_neutrality(self._h, C.byref(r), C.c_int64(cap), C.byref(n)))
+        return {k: v[:n.value] for k, v in arrs.items()}
+
     def fetch_results(self, cap):
         arrs, r = self._alloc_result(cap)
         n = C.c_int64()
@@ -339,6 +379,12 @@ class Handle:
         ms = (C.c_float * 10)()
         self._check(self._L.tdsfs_timings(self._h, ms, C.c_int32(10)))
         return float(ms[9])
+
+    def neutrality_ms(self):
+        """CUDA-event time (ms) of the segment + finish kernels of the last neutrality call (tdsfs_timings slot 10)."""
+        ms = (C.c_float * 11)()
+        self._check(self._L.tdsfs_timings(self._h, ms, C.c_int32(11)))
+        return float(ms[10])
 
     def launch_count(self):
         return int(self._L.tdsfs_launch_count(self._h))

@@ -301,3 +301,12 @@ def sharded_diversity(handle, pieces, pos, size, device, *, snp_mode=False, grou
     GPU); it keeps sharded_scan's calling convention.  Returns the gathered arrays (identical on every rank)."""
     res = handle.diversity(size, snp_mode=snp_mode)
     return gather_results(localize_results(res, pieces, pos, size, snp_mode), 0, group)
+
+
+def sharded_neutrality(handle, pieces, pos, size, device, *, snp_mode=False, group=None):
+    """Per-window Watterson's theta and Tajima's D of a sharded panel: the neutrality counterpart of sharded_diversity,
+    with the same calling convention.  Every result of a window depends on its own rows only (n is the window's largest
+    called-allele count), so the gathered arrays equal a single-handle run bit for bit.  Returns the gathered arrays
+    (identical on every rank)."""
+    res = handle.neutrality(size, snp_mode=snp_mode)
+    return gather_results(localize_results(res, pieces, pos, size, snp_mode), 0, group)

@@ -480,18 +480,25 @@ class LikelihoodInference_jointSFS:
         keys, counts, stats, _, _ = self._scan(table, snp_window_size, True, bg_mode=T.BG_PER_CHROM)
         return self._unguarded(keys, counts, stats, with_diff=True, snp_count_fixed=snp_window_size)
 
-    # ------------------------------------------------------------------ diversity (not in the reference)
-    def _fst(self, data_dict, size, snp_mode):
+    # ------------------------------------------------------------------ diversity and neutrality (not in the reference)
+    def _window_pass(self, data_dict, size, snp_mode, neutrality):
+        """Keys and result columns (lists) of the non-empty windows of (size, mode) from the diversity or the neutrality
+        pass over data_dict."""
         table = self._table(data_dict)
         if table.n == 0:
-            return {}
+            return [], {}
         self._int_filters()
         eng = self._eng()
         eng.load(table, self.pop1_size, self.pop2_size, self.fold, self._flags(table))
-        res = eng.h.diversity(size, snp_mode=snp_mode)
+        res = (eng.h.neutrality if neutrality else eng.h.diversity)(size, snp_mode=snp_mode)
         live = (res["flags"] & T.F_EMPTY) == 0
-        keys = window_keys(table, res, live)
-        cols = [res[k][live].tolist() for k in ("snp_count", "n_sites", "pi_p1", "pi_p2", "dxy", "fst")]
+        return window_keys(table, res, live), {k: v[live].tolist() for k, v in res.items()}
+
+    def _fst(self, data_dict, size, snp_mode):
+        keys, res = self._window_pass(data_dict, size, snp_mode, False)
+        if not keys:
+            return {}
+        cols = [res[k] for k in ("snp_count", "n_sites", "pi_p1", "pi_p2", "dxy", "fst")]
         return {k: {"snp_count": c, "n_sites": n, "pi_pop1": a, "pi_pop2": b, "dxy": d, "FST": None if f != f else f}
                 for k, c, n, a, b, d, f in zip(keys, *cols)}
 
@@ -515,6 +522,38 @@ class LikelihoodInference_jointSFS:
         self.data_dict = data_dict
         self.snp_window_size = snp_window_size
         return self._fst(data_dict, snp_window_size, True)
+
+    _TAJIMA_COLS = dict(snp_count="snp_count", S_pop1="n_seg_p1", S_pop2="n_seg_p2", n_max_pop1="n_max_p1",
+                        n_max_pop2="n_max_p2", theta_pi_pop1="theta_pi_p1", theta_pi_pop2="theta_pi_p2",
+                        theta_w_pop1="theta_w_p1", theta_w_pop2="theta_w_p2", TajimaD_pop1="tajima_d_p1",
+                        TajimaD_pop2="tajima_d_p2")
+
+    def _tajima(self, data_dict, size, snp_mode):
+        keys, res = self._window_pass(data_dict, size, snp_mode, True)
+        if not keys:
+            return {}
+        cols = [res[c] for c in self._TAJIMA_COLS.values()]
+        return {k: {name: None if v != v else v for name, v in zip(self._TAJIMA_COLS, row)} for k, row in zip(keys, zip(*cols))}
+
+    def tajima_scan(self, data_dict, window_size):
+        """Watterson's theta and Tajima's D of each population in every non-empty fixed-bp window, computed on the GPU from
+        the same data as the scans: {"{chrom} {start}-{end}": {"snp_count", "S_pop1", "S_pop2", "n_max_pop1", "n_max_pop2",
+        "theta_pi_pop1", "theta_pi_pop2", "theta_w_pop1", "theta_w_pop2", "TajimaD_pop1", "TajimaD_pop2"}}, keyed like
+        fst_scan.  Per population, over the SNPs that pass the constructor's filters: S the segregating sites, n_max the
+        largest number of called alleles, theta_pi the summed pairwise differences, theta_w = S / a1(n_max); Tajima's D is
+        scikit-allel's tajima_d of the window's SNPs at n = n_max.  theta values are absolute, not per bp.  None where
+        undefined: theta_w when n_max < 2, TajimaD when S < 3 or n_max == 2.  Negative D: an excess of rare variants
+        (sweep, expansion); positive D: an excess of intermediate ones (balancing selection, structure).  Not in the
+        reference; pass the result to save_csv_stats(tajima=...)."""
+        self.data_dict = data_dict
+        self.window_size = window_size
+        return self._tajima(data_dict, window_size, False)
+
+    def tajima_scan_bySNPs(self, data_dict, snp_window_size):
+        """tajima_scan over fixed-SNP windows, with the windows and keys of fst_scan_bySNPs."""
+        self.data_dict = data_dict
+        self.snp_window_size = snp_window_size
+        return self._tajima(data_dict, snp_window_size, True)
 
     # ------------------------------------------------------------------ simulations
     def get_gens(self, main_dir):
@@ -602,12 +641,14 @@ def load_chr_ids(chromosomes_txt):
 col_names = ['chromosome', 'window_start', 'window_end', 'snp_count', 'T2D', 'T1D_p1', 'T1D_p2', 'new_term_p1', 'new_term_p2', 'T2D_diff']
 
 
-def save_csv_stats(stats_dict, output, fst=None):
+def save_csv_stats(stats_dict, output, fst=None, tajima=None):
     """reference :1884-1907: same columns, chromosome mapped through chr_ids, None written as ''.  fst (not in the
     reference): the dict of fst_scan / fst_scan_bySNPs over the same windows adds a trailing FST column, the layout of the
-    ECB tables the reference's R post-processing writes; '' where FST is None or the window has no entry."""
+    ECB tables the reference's R post-processing writes; '' where FST is None or the window has no entry.  tajima (not in
+    the reference): the dict of tajima_scan / tajima_scan_bySNPs adds TajimaD_p1, TajimaD_p2 after it, '' likewise."""
     with open(output, 'w', newline='') as csvfile:
-        writer = csv.DictWriter(csvfile, fieldnames=col_names + (['FST'] if fst is not None else []))
+        writer = csv.DictWriter(csvfile, fieldnames=col_names + (['FST'] if fst is not None else [])
+                                + (['TajimaD_p1', 'TajimaD_p2'] if tajima is not None else []))
         writer.writeheader()
         for window_coords, result in stats_dict.items():
             chromosome = window_coords.split(' ')[0]
@@ -618,6 +659,9 @@ def save_csv_stats(stats_dict, output, fst=None):
                    'new_term_p2': result["new_term_pop2"], 'T2D_diff': result["T2D_diff"]}
             if fst is not None:
                 row['FST'] = fst.get(window_coords, {}).get("FST")
+            if tajima is not None:
+                t = tajima.get(window_coords, {})
+                row['TajimaD_p1'], row['TajimaD_p2'] = t.get("TajimaD_pop1"), t.get("TajimaD_pop2")
             writer.writerow(row)
 
 

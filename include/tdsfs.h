@@ -240,6 +240,46 @@ int tdsfs_diversity_bp(tdsfs_t* ctx, int64_t W, tdsfs_diversity_t* out, int64_t 
 int tdsfs_diversity_snp(tdsfs_t* ctx, int64_t N, tdsfs_diversity_t* out, int64_t cap, int64_t* n_windows);
 int tdsfs_fetch_diversity(tdsfs_t* ctx, tdsfs_diversity_t* out, int64_t cap, int64_t* n_windows);
 
+/* ---- per-window neutrality: Watterson's theta, Tajima's D per population (no reference counterpart; DESIGN.md 7) ---
+ * Same windows, spectrum filter (snp_flags bit0) and counts (n_i = ref_i + alt_i called alleles, fix-ups applied) as
+ * tdsfs_diversity_*.  Per window and population i, over the rows that pass the filter:
+ *   n_seg_p<i>     S_i, rows with ref_i > 0 and alt_i > 0: segregating in population i, whatever the other population has;
+ *   n_max_p<i>     the largest n_i (0 when no row passes);
+ *   theta_pi_p<i>  the sum over rows with n_i >= 2 of 2 ref_i alt_i / (n_i (n_i - 1)) (fp64, exact integer numerator and
+ *                  denominator, one rounded division), in the summation order of tdsfs_diversity_*.  It differs from that
+ *                  call's pi_p<i> only on rows where the other population has n < 2, which pi_p<i> leaves out;
+ *   theta_w_p<i>   S_i / a1(n_max_i), a1(n) = sum_{k=1}^{n-1} 1/k summed in ascending k; NaN when n_max_i < 2;
+ *   tajima_d_p<i>  (theta_pi - theta_w) / sqrt(e1 S + e2 S (S - 1)), Tajima's (1989) constants at n = n_max_i:
+ *                  a2 = sum_{k=1}^{n-1} 1/k^2, b1 = (n+1) / (3(n-1)), b2 = 2(n^2+n+3) / (9n(n-1)), c1 = b1 - 1/a1,
+ *                  c2 = b2 - (n+2)/(a1 n) + a2/a1^2, e1 = c1/a1, e2 = c2/(a1^2 + a2); NaN when S_i < 3 or the variance
+ *                  term is not > 0 (n_max = 2 makes e1 = e2 = 0).
+ * This is scikit-allel's tajima_d (min_sites = 3) on the window's rows, with absolute theta: dividing by a callable length
+ * is the caller's business.  The per-window n keeps results a function of the window's rows alone (bitwise equal for the
+ * counts and the genotype entry and for any sharding that keeps windows whole); a caller who wants another n recomputes D
+ * from n_seg, n_max and theta_pi.  Own window arrays and results, as tdsfs_diversity_*: neither call, a pending plan, the
+ * scan's results nor the step graph disturbs the other.
+ * out == NULL: enqueue only (honours tdsfs_set_sync(0)); tdsfs_fetch_neutrality copies the results later. */
+typedef struct {            /* caller-owned host SoA, capacity >= tdsfs_candidates_bp / _snp; any member may be NULL */
+  int32_t* chrom;           /* as tdsfs_result_t */
+  int64_t* start;
+  int64_t* end;
+  int32_t* snp_count;       /* count_snps, as tdsfs_result_t */
+  uint8_t* flags;           /* TDSFS_F_EMPTY */
+  int32_t* n_seg_p1;        /* S_1 */
+  int32_t* n_seg_p2;        /* S_2 */
+  int32_t* n_max_p1;
+  int32_t* n_max_p2;
+  double* theta_pi_p1;
+  double* theta_pi_p2;
+  double* theta_w_p1;       /* NaN when n_max_p1 < 2 */
+  double* theta_w_p2;
+  double* tajima_d_p1;      /* NaN when S_1 < 3 or the variance term is not > 0 */
+  double* tajima_d_p2;
+} tdsfs_neutrality_t;
+int tdsfs_neutrality_bp(tdsfs_t* ctx, int64_t W, tdsfs_neutrality_t* out, int64_t cap, int64_t* n_windows);
+int tdsfs_neutrality_snp(tdsfs_t* ctx, int64_t N, tdsfs_neutrality_t* out, int64_t cap, int64_t* n_windows);
+int tdsfs_fetch_neutrality(tdsfs_t* ctx, tdsfs_neutrality_t* out, int64_t cap, int64_t* n_windows);
+
 /* ---- likelihood of explicit spectra ------------------------------------------------------------------------
  * calculate_likelihood_1D / _2D (:478-537, :625-684) on already-interior vectors: x[n] integer counts,
  * b[n] background values, B = sum of b as the caller's language sums it.  *flag = 1 when the reference returns
@@ -258,7 +298,8 @@ int tdsfs_synth_genotypes(tdsfs_t* ctx, void* G_dev, int64_t S, int64_t snp0, in
 /* CUDA-event times (ms) of the last background / finalize / scan calls (synchronises the stream):
  * [0]=count kernel (K1), [1]=finalize, [2]=boundaries (K2), [3]=score small windows (K3/K4), [4]=score large windows,
  * [5]=background call, [6]=scan call, [7]=K1 start -> last score kernel end, [8]=peer exchange kernel (n >= 9),
- * [9]=segment + finish kernels of the last tdsfs_diversity_* call (n >= 10). */
+ * [9]=segment + finish kernels of the last tdsfs_diversity_* call (n >= 10),
+ * [10]=segment + finish kernels of the last tdsfs_neutrality_* call (n >= 11). */
 int tdsfs_timings(tdsfs_t* ctx, float* ms, int32_t n);
 int64_t tdsfs_launch_count(tdsfs_t* ctx); /* kernels launched by this handle so far */
 /* Which path scored the last scan: *fused = 1 when the fused pair ran (tdsfs_plan_* before tdsfs_background on the

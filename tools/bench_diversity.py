@@ -1,6 +1,7 @@
 #!/usr/bin/env python
-"""Time the per-window diversity pass (Hudson FST, pi, dxy: tdsfs_diversity_bp) on bench.py's config 5 and config 4 panels,
-built in HBM by the same device generator, over the same 20 kb windows.
+"""Time the per-window diversity pass (Hudson FST, pi, dxy: tdsfs_diversity_bp) and the neutrality pass (Watterson's theta,
+Tajima's D: tdsfs_neutrality_bp) on bench.py's config 5 and config 4 panels, built in HBM by the same device generator, over
+the same 20 kb windows.
 
   python tools/bench_diversity.py [--calls 30] [--warmup 5] [--out DIR]
 
@@ -11,7 +12,9 @@ Per workload it reports
   * the algorithmic bytes S (n1 + n2) / 4 (2-bit calls; each read once), the achieved GB/s over kernel_ms and call_ms, and
     their fraction of 6,544 GB/s (the copy rate measured for this project on a B200) and of the 7.7 TB/s data sheet;
   * copy_gbs: a device-to-device copy of the same genotype matrix timed in the same process, read + write bytes over time;
-  * the card's name and power limit, read in the same process.
+  * the card's name and power limit, read in the same process;
+  * the same call / kernel times, GB/s and fractions for the neutrality pass under neutrality_* keys (same panel, same
+    windows, same algorithmic bytes), and neutrality_over_fst_kernel, the ratio of the two kernel medians.
 One JSON line per workload on stdout; with --out, also DIR/bench_diversity.json.
 """
 import argparse
@@ -79,6 +82,23 @@ def measure(name, cfg, args, h, T, torch, stream):
     h.set_sync(True)
     res = h.fetch_diversity(h.candidates(W))
 
+    # the neutrality pass over the same windows, timed the same way
+    for _ in range(args.warmup):
+        h.neutrality(W, fetch=False)
+    nkernel = []
+    for _ in range(args.calls):
+        h.neutrality(W, fetch=False)
+        nkernel.append(h.neutrality_ms())
+    h.set_sync(False)
+    ev0.record(stream)
+    for _ in range(args.calls):
+        h.neutrality(W, fetch=False)
+    ev1.record(stream)
+    torch.cuda.synchronize()
+    ncall_ms = ev0.elapsed_time(ev1) / args.calls
+    h.set_sync(True)
+    nres = h.fetch_neutrality(h.candidates(W))
+
     # same-process reference: device-to-device copy of the genotype matrix
     dst = torch.empty_like(G)
     for _ in range(3):
@@ -103,7 +123,18 @@ def measure(name, cfg, args, h, T, torch, stream):
            "checks": {"snp_count_sum_equals_S": bool(int(res["snp_count"].sum()) == S),
                       "n_sites": int(res["n_sites"].sum()), "windows_with_fst": int(np.isfinite(res["fst"][live]).sum()),
                       "mean_fst": float(np.nanmean(res["fst"][live]))}}
-    for k in ("kernel", "call"):
+    nk_ms = float(np.median(nkernel))
+    nlive = (nres["flags"] & T.F_EMPTY) == 0
+    out.update({"neutrality_call_ms": ncall_ms, "neutrality_kernel_ms_median": nk_ms,
+                "neutrality_kernel_ms_min": float(np.min(nkernel)), "neutrality_kernel_ms_max": float(np.max(nkernel)),
+                "neutrality_kernel_gbs": algo / (nk_ms * 1e-3) / 1e9, "neutrality_call_gbs": algo / (ncall_ms * 1e-3) / 1e9,
+                "neutrality_over_fst_kernel": nk_ms / k_ms,
+                "neutrality_checks": {"snp_count_sum_equals_S": bool(int(nres["snp_count"].sum()) == S),
+                                      "n_seg_p1": int(nres["n_seg_p1"].sum()), "n_seg_p2": int(nres["n_seg_p2"].sum()),
+                                      "windows_with_tajima_d_p1": int(np.isfinite(nres["tajima_d_p1"][nlive]).sum()),
+                                      "mean_tajima_d_p1": float(np.nanmean(nres["tajima_d_p1"][nlive])),
+                                      "mean_tajima_d_p2": float(np.nanmean(nres["tajima_d_p2"][nlive]))}})
+    for k in ("kernel", "call", "neutrality_kernel", "neutrality_call"):
         out[k + "_frac_of_copy_peak"] = out[k + "_gbs"] / COPY_PEAK_GBS
         out[k + "_frac_of_sheet"] = out[k + "_gbs"] / SHEET_GBS
     del G, pos_dev
