@@ -64,29 +64,48 @@ static long long peer_timeout_cycles() {
     if (r__) return r__;       \
   } while (0)
 
-enum { EV_BG0, EV_K1, EV_FIN0, EV_FIN1, EV_SC0, EV_K2, EV_K3S, EV_K3L, EV_X0, EV_X1, EV_D0, EV_D1, EV_N0, EV_N1, NEV };
+enum { EV_BG0, EV_K1, EV_FIN0, EV_FIN1, EV_SC0, EV_K2, EV_K3S, EV_K3L, EV_X0, EV_X1, NEV };
 
 struct Chunk {
   long long r0, r1;
   cudaEvent_t ev;
 };
 
-// Workspace of one per-window pass over the candidate windows of (size, mode) (tdsfs_diversity_*, tdsfs_neutrality_*):
-// its candidate offsets, window boundaries, segment list and scan scratch.
-struct WindowPass {
-  long long W = -1;                   // (size, mode) whose candidate offsets d_cand_off holds
+// Candidate-window offsets per chromosome of one (size, mode), on the host and the device (cached_candidates): computed
+// and uploaded again only when (size, mode) changes, so that a steady-state call needs no host round trip.
+struct CandCache {
+  long long W = -1;                   // (size, mode) the offsets are of; -1: none
   int snp = -1;
-  std::vector<long long> off_host;
-  long long cap = 0, ncand = 0;
+  std::vector<long long> off;         // [C + 1]
+  long long* d_off = nullptr;
+  bool holds(long long size, bool snp_mode) const { return W == size && snp == (int)snp_mode; }
+};
+
+// Workspace and results of one per-window pass over the candidate windows of (size, mode) (tdsfs_diversity_*,
+// tdsfs_neutrality_*): its candidate offsets, window boundaries, segment list, scan scratch, per-segment sums, per-window
+// results and events.
+struct WindowPass {
+  WindowPass(const char* name, size_t part_bytes, int n_i32, int n_f64)
+      : name(name), part_bytes(part_bytes), n_i32(n_i32), n_f64(n_f64) {}
+  const char* name;                   // NVTX range of a call
+  size_t part_bytes;                  // size of the pass's per-segment sums (DivPart, NeutPart)
+  int n_i32, n_f64;                   // result columns of the pass in d_i32 / d_f64
+  CandCache cand;
+  long long cap = 0, ncand = 0;       // windows the per-window arrays hold / of the last call
   size_t tmp_bytes = 0;
-  long long* d_cand_off = nullptr;
   int32_t *d_wlo = nullptr, *d_whi = nullptr, *d_wchrom = nullptr, *d_count = nullptr;
   int32_t* d_large = nullptr;         // never written: a per-window pass has no "large window" split
   int* d_nlarge = nullptr;
   long long *d_wstart = nullptr, *d_wend = nullptr, *d_nseg = nullptr, *d_segoff = nullptr;
   uint8_t* d_flags = nullptr;
   void* d_tmp = nullptr;              // CUB scan scratch
+  int32_t* d_i32[4] = {};             // [cap] the pass's int32 and fp64 result columns, each in the order of its result
+  double* d_f64[6] = {};              // struct in include/tdsfs.h
+  void* d_part = nullptr;             // [part_cap] per-segment sums
+  long long part_cap = 0;
+  cudaEvent_t ev0 = nullptr, ev1 = nullptr;  // around the segment and finish kernels (tdsfs_timings)
   bool ready = false, timed = false;  // results of the last call are on the device / its events were recorded
+  SegList segs() const { return SegList{d_wlo, d_whi, ncand, d_segoff}; }
 };
 
 struct tdsfs_ctx {
@@ -162,9 +181,7 @@ struct tdsfs_ctx {
   bool peer_ready = false;
   // windows / results
   long long ncand = 0, cand_cap = 0;
-  std::vector<long long> cand_off_host;  // cached candidate offsets of (cand_W, cand_snp)
-  long long cand_W = -1;
-  int cand_snp = -1;
+  CandCache cand;
   int groups_mode = -1, groups_chrom = -1;  // what d_bg_group / d_score_group currently hold
   // window plan launched ahead of the scan on a side stream (tdsfs_plan_bp / _snp)
   cudaStream_t plan_stream = nullptr;
@@ -172,7 +189,6 @@ struct tdsfs_ctx {
   long long plan_W = -1;
   int plan_snp = -1;
   bool planned_last = false;
-  long long* d_cand_off = nullptr;
   int32_t *d_wlo = nullptr, *d_whi = nullptr, *d_wchrom = nullptr, *d_large = nullptr;
   long long *d_wstart = nullptr, *d_wend = nullptr;
   int* d_nlarge = nullptr;
@@ -194,19 +210,8 @@ struct tdsfs_ctx {
   bool step_graphs_off = false;       // capture failed once: run eagerly from then on
   // per-window passes over the scan's candidate windows: each has its own workspace and results, so that it never touches
   // the scan's plan, window buffers or unfetched results, nor the other pass's
-  // Hudson FST, pi, dxy (tdsfs_diversity_*)
-  WindowPass div;
-  long long div_part_cap = 0;
-  int32_t* d_div_nsites = nullptr;
-  double *d_div_pi1 = nullptr, *d_div_pi2 = nullptr, *d_div_dxy = nullptr, *d_div_fst = nullptr;
-  DivPart* d_div_part = nullptr;
-  // Watterson's theta, Tajima's D (tdsfs_neutrality_*)
-  WindowPass neut;
-  long long neut_part_cap = 0;
-  int32_t *d_neut_S1 = nullptr, *d_neut_S2 = nullptr, *d_neut_nmax1 = nullptr, *d_neut_nmax2 = nullptr;
-  double *d_neut_pi1 = nullptr, *d_neut_pi2 = nullptr, *d_neut_tw1 = nullptr, *d_neut_tw2 = nullptr;
-  double *d_neut_d1 = nullptr, *d_neut_d2 = nullptr;
-  NeutPart* d_neut_part = nullptr;
+  WindowPass div{"tdsfs:diversity (FST, pi, dxy)", sizeof(DivPart), 1, 4};                 // tdsfs_diversity_*
+  WindowPass neut{"tdsfs:neutrality (theta_W, Tajima's D)", sizeof(NeutPart), 4, 6};      // tdsfs_neutrality_*
   double* d_neut_tab = nullptr;       // a1(n) for n in [0, neut_tab_n], then a2(n) for the same n
   long long neut_tab_n = -1;
   long long n_allele_max = 0;         // the largest n_i = ref_i + alt_i a row of the loaded data can reach
@@ -281,6 +286,10 @@ extern "C" int tdsfs_create(int device, tdsfs_t** out) {
   CK(cudaEventCreate(&c->ev_plan0));
   c->stream = c->own_stream;
   for (int i = 0; i < NEV; ++i) CK(cudaEventCreate(&c->ev[i]));
+  for (WindowPass* w : {&c->div, &c->neut}) {
+    CK(cudaEventCreate(&w->ev0));
+    CK(cudaEventCreate(&w->ev1));
+  }
   CKR(dev_alloc(&c->d_err, 1));
   CKR(dev_alloc(&c->d_nlarge, 1));
   CKR(dev_alloc(&c->d_lnI, LN_TABLE));
@@ -334,23 +343,31 @@ static void free_data(tdsfs_ctx* c) {
   for (auto& ch : c->chunks) if (ch.ev) cudaEventDestroy(ch.ev);
   c->chunks.clear();
   c->keys_ready = c->tables_ready = c->results_ready = false;
-  c->cand_W = -1;
+  c->cand.W = -1;
   c->groups_mode = -1;
   c->plan_W = -1;
   c->ws_ready = false;
   c->force_wide = false;
   for (WindowPass* w : {&c->div, &c->neut}) {
-    w->W = -1;
+    w->cand.W = -1;
     w->ready = false;
   }
   c->n_allele_max = 0;
 }
 
+// the per-window arrays of pass w
+static void free_pass_windows(WindowPass& w) {
+  dev_free(w.d_wlo); dev_free(w.d_whi); dev_free(w.d_wchrom); dev_free(w.d_count); dev_free(w.d_wstart); dev_free(w.d_wend);
+  dev_free(w.d_nseg); dev_free(w.d_segoff); dev_free(w.d_flags); dev_free(w.d_tmp);
+  for (int32_t*& a : w.d_i32) dev_free(a);
+  for (double*& a : w.d_f64) dev_free(a);
+}
+
 static void free_window_pass(WindowPass& w) {
-  dev_free(w.d_cand_off); dev_free(w.d_wlo); dev_free(w.d_whi); dev_free(w.d_wchrom); dev_free(w.d_count); dev_free(w.d_large);
-  dev_free(w.d_nlarge); dev_free(w.d_wstart); dev_free(w.d_wend); dev_free(w.d_nseg); dev_free(w.d_segoff); dev_free(w.d_flags);
-  if (w.d_tmp) cudaFree(w.d_tmp);
-  w.d_tmp = nullptr;
+  free_pass_windows(w);
+  dev_free(w.cand.d_off); dev_free(w.d_large); dev_free(w.d_nlarge); dev_free(w.d_part);
+  if (w.ev0) cudaEventDestroy(w.ev0);
+  if (w.ev1) cudaEventDestroy(w.ev1);
 }
 
 extern "C" void tdsfs_destroy(tdsfs_t* c) {
@@ -371,19 +388,15 @@ extern "C" void tdsfs_destroy(tdsfs_t* c) {
   if (c->d_rec) cudaFree(c->d_rec);
   dev_free(c->d_hist); dev_free(c->d_bg_group); dev_free(c->d_score_group);
   dev_free(c->d_lb2); dev_free(c->d_lb1a); dev_free(c->d_lb1b); dev_free(c->d_B); dev_free(c->d_Bsum); dev_free(c->d_lnI);
-  dev_free(c->d_err); dev_free(c->d_cand_off); dev_free(c->d_wlo); dev_free(c->d_whi); dev_free(c->d_wchrom);
+  dev_free(c->d_err); dev_free(c->cand.d_off); dev_free(c->d_wlo); dev_free(c->d_whi); dev_free(c->d_wchrom);
   dev_free(c->d_large); dev_free(c->d_wstart); dev_free(c->d_wend); dev_free(c->d_nlarge);
   dev_free(c->r_count); dev_free(c->r_n2); dev_free(c->r_n1a); dev_free(c->r_n1b); dev_free(c->r_T2); dev_free(c->r_T1a);
   dev_free(c->r_T1b); dev_free(c->r_flags); dev_free(c->d_scratch);
   for (int i = 0; i < NEV; ++i) if (c->ev[i]) cudaEventDestroy(c->ev[i]);
   dev_free(c->d_dxI); dev_free(c->d_ws); dev_free(c->d_gridbar); dev_free(c->d_stamps);
   free_window_pass(c->div);
-  dev_free(c->d_div_nsites); dev_free(c->d_div_pi1); dev_free(c->d_div_pi2); dev_free(c->d_div_dxy); dev_free(c->d_div_fst);
-  dev_free(c->d_div_part);
   free_window_pass(c->neut);
-  dev_free(c->d_neut_S1); dev_free(c->d_neut_S2); dev_free(c->d_neut_nmax1); dev_free(c->d_neut_nmax2); dev_free(c->d_neut_pi1);
-  dev_free(c->d_neut_pi2); dev_free(c->d_neut_tw1); dev_free(c->d_neut_tw2); dev_free(c->d_neut_d1); dev_free(c->d_neut_d2);
-  dev_free(c->d_neut_part); dev_free(c->d_neut_tab);
+  dev_free(c->d_neut_tab);
   cudaStreamDestroy(c->own_stream);
   cudaStreamDestroy(c->copy_stream);
   cudaStreamDestroy(c->plan_stream);
@@ -759,7 +772,7 @@ extern "C" int tdsfs_background(tdsfs_t* c, int32_t mode, int32_t bg_chrom, int6
       q.wmode = fuse ? (c->plan_snp ? 2 : 1) : 0;
       q.tab_words = fuse ? tab_words : 0;
       if (fuse) {
-        const long long ncand = c->cand_off_host[c->C];
+        const long long ncand = c->cand.off[c->C];
         if (ncand > c->ws_cap) {
           CK(cudaStreamSynchronize(st));
           dev_free(c->d_ws);
@@ -768,7 +781,7 @@ extern "C" int tdsfs_background(tdsfs_t* c, int32_t mode, int32_t bg_chrom, int6
         }
         q.W = (uint32_t)c->plan_W;
         q.Wmagic = (uint32_t)std::min<unsigned long long>(0xFFFFFFFFull, (1ull << 32) / (unsigned long long)c->plan_W);
-        q.cand_off = c->d_cand_off;
+        q.cand_off = c->cand.d_off;
         q.ncand = ncand;
         q.ws = c->d_ws;
         q.dxI = c->d_dxI;
@@ -1116,20 +1129,27 @@ static int candidates(tdsfs_ctx* c, long long W, bool snp_mode, std::vector<long
   return 0;
 }
 
-extern "C" int tdsfs_candidates_bp(tdsfs_t* c, int64_t W, int64_t* n) {
+static int count_candidates(tdsfs_ctx* c, long long W, bool snp_mode, int64_t* n) {
   if (!c || !n || W < 1) return fail(TDSFS_ERR_ARG, "bad argument");
   if (!c->dPos) return fail(TDSFS_ERR_STATE, "load data first");
   std::vector<long long> off;
-  CKR(candidates(c, W, false, off));
+  CKR(candidates(c, W, snp_mode, off));
   *n = off[c->C];
   return 0;
 }
-extern "C" int tdsfs_candidates_snp(tdsfs_t* c, int64_t N, int64_t* n) {
-  if (!c || !n || N < 1) return fail(TDSFS_ERR_ARG, "bad argument");
-  if (!c->dPos) return fail(TDSFS_ERR_STATE, "load data first");
-  std::vector<long long> off;
-  CKR(candidates(c, N, true, off));
-  *n = off[c->C];
+extern "C" int tdsfs_candidates_bp(tdsfs_t* c, int64_t W, int64_t* n) { return count_candidates(c, W, false, n); }
+extern "C" int tdsfs_candidates_snp(tdsfs_t* c, int64_t N, int64_t* n) { return count_candidates(c, N, true, n); }
+
+// The offsets of (W, mode) in k, uploaded on stream st when they change.
+static int cached_candidates(tdsfs_ctx* c, CandCache& k, long long W, bool snp_mode, cudaStream_t st) {
+  if (k.holds(W, snp_mode)) return 0;
+  k.W = -1;  // until the device copy matches
+  CKR(candidates(c, W, snp_mode, k.off));
+  dev_free(k.d_off);
+  CKR(dev_alloc(&k.d_off, c->C + 1));
+  CK(cudaMemcpyAsync(k.d_off, k.off.data(), (size_t)(c->C + 1) * 8, cudaMemcpyHostToDevice, st));
+  k.W = W;
+  k.snp = snp_mode;
   return 0;
 }
 
@@ -1149,56 +1169,52 @@ static int ensure_windows(tdsfs_ctx* c, long long n) {
   return 0;
 }
 
+// n windows of one per-window result: host destination (NULL: not wanted), device source
+struct Column {
+  template <typename H, typename D>
+  Column(H* dst, const D* src) : dst(dst), src(src), size(sizeof(D)) { static_assert(sizeof(H) == sizeof(D), "element size"); }
+  void* dst;
+  const void* src;
+  size_t size;
+};
+
+// Copies n windows of each wanted column to the host on the handle's stream (its device current), then waits for them.
+static int fetch_columns(tdsfs_ctx* c, long long n, std::initializer_list<Column> cols, int64_t* n_windows) {
+  for (const Column& k : cols)
+    if (k.dst && n) CK(cudaMemcpyAsync(k.dst, k.src, (size_t)n * k.size, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  if (n_windows) *n_windows = n;
+  return 0;
+}
+
 extern "C" int tdsfs_fetch_results(tdsfs_t* c, tdsfs_result_t* out, int64_t cap, int64_t* n_windows) {
   if (!c || !out) return fail(TDSFS_ERR_ARG, "NULL argument");
   if (!c->results_ready) return fail(TDSFS_ERR_STATE, "no scan results");
   if (cap < c->ncand) return fail(TDSFS_ERR_ARG, "result capacity %lld < %lld candidate windows", (long long)cap, c->ncand);
   CK(cudaSetDevice(c->device));
-  cudaStream_t st = c->stream;
-  const size_t n = (size_t)c->ncand;
-#define D2H(dst, src, T) \
-  if (out->dst && n) CK(cudaMemcpyAsync(out->dst, c->src, n * sizeof(T), cudaMemcpyDeviceToHost, st))
-  D2H(chrom, d_wchrom, int32_t);
-  D2H(start, d_wstart, long long);
-  D2H(end, d_wend, long long);
-  D2H(snp_count, r_count, int32_t);
-  D2H(n2d, r_n2, int32_t);
-  D2H(n1d_p1, r_n1a, int32_t);
-  D2H(n1d_p2, r_n1b, int32_t);
-  D2H(T2D, r_T2, double);
-  D2H(T1D_p1, r_T1a, double);
-  D2H(T1D_p2, r_T1b, double);
-  D2H(flags, r_flags, uint8_t);
-#undef D2H
-  int err = 0;
-  CK(cudaMemcpyAsync(&err, c->d_err, sizeof err, cudaMemcpyDeviceToHost, st));
-  CK(cudaStreamSynchronize(st));
-  if (n_windows) *n_windows = c->ncand;
+  int err = 0;  // read in the same round trip as the results
+  CK(cudaMemcpyAsync(&err, c->d_err, sizeof err, cudaMemcpyDeviceToHost, c->stream));
+  CKR(fetch_columns(c, c->ncand, {{out->chrom, c->d_wchrom}, {out->start, c->d_wstart}, {out->end, c->d_wend},
+                                  {out->snp_count, c->r_count}, {out->n2d, c->r_n2}, {out->n1d_p1, c->r_n1a},
+                                  {out->n1d_p2, c->r_n1b}, {out->T2D, c->r_T2}, {out->T1D_p1, c->r_T1a},
+                                  {out->T1D_p2, c->r_T1b}, {out->flags, c->r_flags}}, n_windows));
   return deferred_error(c, err);
 }
 
 // candidate list of (W, mode) on the device + K2 launch on stream `st`
 static int ensure_candidates(tdsfs_ctx* c, long long W, bool snp_mode, cudaStream_t st) {
-  if (c->cand_W != W || c->cand_snp != (int)snp_mode) {  // candidate offsets cached per (size, mode): no sync in steady state
-    CKR(candidates(c, W, snp_mode, c->cand_off_host));
-    CKR(ensure_windows(c, c->cand_off_host[c->C]));
-    dev_free(c->d_cand_off);
-    CKR(dev_alloc(&c->d_cand_off, c->C + 1));
-    CK(cudaMemcpyAsync(c->d_cand_off, c->cand_off_host.data(), (size_t)(c->C + 1) * 8, cudaMemcpyHostToDevice, st));
-    c->cand_W = W;
-    c->cand_snp = snp_mode;
-    c->ws_ready = false;
-  }
-  return 0;
+  if (!c->cand.holds(W, snp_mode)) c->ws_ready = false;  // the count kernel's window sums are of other windows
+  CKR(cached_candidates(c, c->cand, W, snp_mode, st));
+  return ensure_windows(c, c->cand.off[c->C]);
 }
 
 static int launch_bounds(tdsfs_ctx* c, long long W, bool snp_mode, cudaStream_t st) {
   CKR(ensure_candidates(c, W, snp_mode, st));
-  const long long ncand = c->cand_off_host[c->C];
+  const long long ncand = c->cand.off[c->C];
   if (ncand > 0) {
     CK(cudaMemsetAsync(c->d_nlarge, 0, sizeof(int), st));
     WinParams w;
-    w.pos = c->dPos; w.chrom_off = c->d_off; w.cand_off = c->d_cand_off; w.C = c->C; w.W = W; w.ncand = ncand;
+    w.pos = c->dPos; w.chrom_off = c->d_off; w.cand_off = c->cand.d_off; w.C = c->C; w.W = W; w.ncand = ncand;
     w.wlo = c->d_wlo; w.whi = c->d_whi; w.wchrom = c->d_wchrom; w.wstart = c->d_wstart; w.wend = c->d_wend;
     w.large = c->d_large; w.nlarge = c->d_nlarge;
     w.r_count = c->r_count; w.r_flags = c->r_flags;
@@ -1247,7 +1263,7 @@ static int scan(tdsfs_ctx* c, long long W, bool snp_mode, tdsfs_result_t* out, i
   if (planned) CK(cudaStreamWaitEvent(st, c->ev_plan, 0));   // K2 already ran (or is running) on the side stream
   else CKR(launch_bounds(c, W, snp_mode, st));
   c->planned_last = planned;
-  const long long ncand = c->cand_off_host[c->C];
+  const long long ncand = c->cand.off[c->C];
   if (out && cap < ncand) return fail(TDSFS_ERR_ARG, "result capacity %lld < %lld candidate windows", (long long)cap, ncand);
   c->ncand = ncand;
   CK(cudaEventRecord(c->ev[EV_K2], st));
@@ -1474,41 +1490,27 @@ extern "C" int tdsfs_window_spectra(tdsfs_t* c, int64_t window, uint64_t* s2, ui
 }
 
 // ------------------------------------------------------------------------------------------------ per-window passes
-// The candidate windows of (W, mode) for pass w: offsets cached per (size, mode), apart from the scan's and the other pass's.
-static int pass_candidates(tdsfs_ctx* c, WindowPass& w, long long W, bool snp_mode, long long* ncand) {
-  if (w.W != W || w.snp != (int)snp_mode) {
-    std::vector<long long> off;
-    CKR(candidates(c, W, snp_mode, off));
-    w.off_host.swap(off);
-    w.W = -1;
-    dev_free(w.d_cand_off);
-    CKR(dev_alloc(&w.d_cand_off, c->C + 1));
-    CK(cudaMemcpyAsync(w.d_cand_off, w.off_host.data(), (size_t)(c->C + 1) * 8, cudaMemcpyHostToDevice, c->stream));
-    w.W = W;
-    w.snp = snp_mode;
-  }
-  *ncand = w.off_host[c->C];
-  return 0;
-}
-
-// Per-window arrays of pass w for ncand windows; *grown when they were reallocated (the pass's own per-window results
-// follow), after the stream has drained.
-static int pass_buffers(tdsfs_ctx* c, WindowPass& w, long long ncand, bool* grown) {
-  *grown = ncand > w.cap;
-  if (*grown) {
-    CK(cudaStreamSynchronize(c->stream));  // a previous asynchronous call may still use the old arrays
-    dev_free(w.d_wlo); dev_free(w.d_whi); dev_free(w.d_wchrom); dev_free(w.d_count); dev_free(w.d_wstart); dev_free(w.d_wend);
-    dev_free(w.d_nseg); dev_free(w.d_segoff); dev_free(w.d_flags);
-    if (w.d_tmp) cudaFree(w.d_tmp);
-    w.d_tmp = nullptr;
+// Arrays of pass w for ncand windows and `parts` segments, grown after the stream has drained (a previous asynchronous
+// call may still use the old ones).
+static int pass_buffers(tdsfs_ctx* c, WindowPass& w, long long ncand, long long parts) {
+  if (ncand > w.cap || parts > w.part_cap) CK(cudaStreamSynchronize(c->stream));
+  if (ncand > w.cap) {
+    free_pass_windows(w);
     CKR(dev_alloc(&w.d_wlo, ncand)); CKR(dev_alloc(&w.d_whi, ncand)); CKR(dev_alloc(&w.d_wchrom, ncand));
     CKR(dev_alloc(&w.d_count, ncand)); CKR(dev_alloc(&w.d_wstart, ncand)); CKR(dev_alloc(&w.d_wend, ncand));
     CKR(dev_alloc(&w.d_nseg, ncand + 1)); CKR(dev_alloc(&w.d_segoff, ncand + 1)); CKR(dev_alloc(&w.d_flags, ncand));
+    for (int i = 0; i < w.n_i32; ++i) CKR(dev_alloc(&w.d_i32[i], ncand));
+    for (int i = 0; i < w.n_f64; ++i) CKR(dev_alloc(&w.d_f64[i], ncand));
     size_t tmp = 0;
     CK(cub::DeviceScan::ExclusiveSum(nullptr, tmp, w.d_nseg, w.d_segoff, (int)(ncand + 1), c->stream));
     CK(cudaMalloc(&w.d_tmp, std::max<size_t>(tmp, 16)));
     w.tmp_bytes = std::max<size_t>(tmp, 16);
     w.cap = ncand;
+  }
+  if (parts > w.part_cap) {
+    dev_free(w.d_part);
+    CK(cudaMalloc(&w.d_part, (size_t)parts * w.part_bytes));
+    w.part_cap = parts;
   }
   if (!w.d_large) {
     CKR(dev_alloc(&w.d_large, 1));
@@ -1525,107 +1527,95 @@ static int pass_segments(tdsfs_ctx* c, WindowPass& w, long long W, bool snp_mode
   const long long ncand = w.ncand;
   if (ncand == 0) return 0;
   WinParams wp;
-  wp.pos = c->dPos; wp.chrom_off = c->d_off; wp.cand_off = w.d_cand_off; wp.C = c->C; wp.W = W; wp.ncand = ncand;
+  wp.pos = c->dPos; wp.chrom_off = c->d_off; wp.cand_off = w.cand.d_off; wp.C = c->C; wp.W = W; wp.ncand = ncand;
   wp.wlo = w.d_wlo; wp.whi = w.d_whi; wp.wchrom = w.d_wchrom; wp.wstart = w.d_wstart; wp.wend = w.d_wend;
   wp.large = w.d_large; wp.nlarge = w.d_nlarge;
   wp.r_count = w.d_count; wp.r_flags = w.d_flags;  // K2 marks empty windows; the pass's finish kernel rewrites every entry
   wp.wcap = 0x7FFFFFFF;
   const int g2 = (int)((ncand + 255) / 256);
   if (snp_mode) k2_bounds_snp<<<g2, 256, 0, st>>>(wp); else k2_bounds_bp<<<g2, 256, 0, st>>>(wp);
-  DivParams p;  // k_div_nseg reads the window rows and writes nseg only
-  memset(&p, 0, sizeof p);
-  p.wlo = w.d_wlo; p.whi = w.d_whi; p.ncand = ncand; p.nseg = w.d_nseg;
-  k_div_nseg<<<(int)((ncand + 1 + 255) / 256), 256, 0, st>>>(p);
+  k_div_nseg<<<(int)((ncand + 1 + 255) / 256), 256, 0, st>>>(w.d_wlo, w.d_whi, ncand, w.d_nseg);
   size_t tmp = w.tmp_bytes;
   CK(cub::DeviceScan::ExclusiveSum(w.d_tmp, tmp, w.d_nseg, w.d_segoff, (int)(ncand + 1), st));
   c->launches += 3;
   return 0;
 }
 
-// ------------------------------------------------------------------------------------------------ diversity (Hudson FST, pi, dxy)
-extern "C" int tdsfs_fetch_diversity(tdsfs_t* c, tdsfs_diversity_t* out, int64_t cap, int64_t* n_windows) {
-  if (!c || !out) return fail(TDSFS_ERR_ARG, "NULL argument");
-  if (!c->div.ready) return fail(TDSFS_ERR_STATE, "no diversity results (tdsfs_diversity_bp / _snp first)");
-  if (cap < c->div.ncand) return fail(TDSFS_ERR_ARG, "result capacity %lld < %lld candidate windows", (long long)cap, c->div.ncand);
-  CK(cudaSetDevice(c->device));
-  cudaStream_t st = c->stream;
-  const size_t n = (size_t)c->div.ncand;
-#define D2H(dst, src, T) \
-  if (out->dst && n) CK(cudaMemcpyAsync(out->dst, c->src, n * sizeof(T), cudaMemcpyDeviceToHost, st))
-  D2H(chrom, div.d_wchrom, int32_t);
-  D2H(start, div.d_wstart, long long);
-  D2H(end, div.d_wend, long long);
-  D2H(snp_count, div.d_count, int32_t);
-  D2H(flags, div.d_flags, uint8_t);
-  D2H(n_sites, d_div_nsites, int32_t);
-  D2H(pi_p1, d_div_pi1, double);
-  D2H(pi_p2, d_div_pi2, double);
-  D2H(dxy, d_div_dxy, double);
-  D2H(fst, d_div_fst, double);
-#undef D2H
-  CK(cudaStreamSynchronize(st));
-  if (n_windows) *n_windows = c->div.ncand;
-  return 0;
+// A pass's segment kernel for the loaded rows: compile-time word counts for the genotype entry's 500 + 500 and 200 + 200
+// diploid panels (BASELINE configs 5 and 4), the runtime decode for any other width and for the counts entry.
+template <typename P>
+static auto segment_kernel(const tdsfs_ctx* c, void (*k32)(P), void (*k14)(P), void (*k0)(P)) -> void (*)(P) {
+  if (c->dG && c->W1 == 32 && c->W2 == 32) return k32;
+  if (c->dG && c->W1 == 14 && c->W2 == 14) return k14;
+  return k0;
 }
 
-static int ensure_div_buffers(tdsfs_ctx* c, long long ncand, long long parts) {
-  bool grown;
-  CKR(pass_buffers(c, c->div, ncand, &grown));
-  if (grown) {
-    dev_free(c->d_div_nsites); dev_free(c->d_div_pi1); dev_free(c->d_div_pi2); dev_free(c->d_div_dxy); dev_free(c->d_div_fst);
-    CKR(dev_alloc(&c->d_div_nsites, ncand)); CKR(dev_alloc(&c->d_div_pi1, ncand)); CKR(dev_alloc(&c->d_div_pi2, ncand));
-    CKR(dev_alloc(&c->d_div_dxy, ncand)); CKR(dev_alloc(&c->d_div_fst, ncand));
-  }
-  if (parts > c->div_part_cap) {
-    CK(cudaStreamSynchronize(c->stream));
-    dev_free(c->d_div_part);
-    CKR(dev_alloc(&c->d_div_part, parts));
-    c->div_part_cap = parts;
-  }
-  return 0;
-}
-
-// Per-window Hudson FST, pi and dxy over the candidate windows of (W, mode), in the order of tdsfs_scan_*: the segment list
-// (pass_segments) -> k_diversity (one warp per segment of DIV_SEG rows) -> k_div_finish.  Needs loaded data only; no host
-// round trip when out == NULL.
-static int diversity(tdsfs_ctx* c, long long W, bool snp_mode, tdsfs_diversity_t* out, int64_t cap, int64_t* n_windows) {
+// One per-window pass over the candidate windows of (W, mode), in the order of tdsfs_scan_*: the segment list
+// (pass_segments), then launch(c, grid): the pass's params, its segment kernel on `grid` CTAs (one warp per segment of
+// DIV_SEG rows; warps past the actual count return at once) and its finish kernel.  prepare (NULL: none) sets up what else
+// those kernels read, before the timed range.  Needs loaded data only, and no host round trip when !fetch; when fetch, the
+// caller fetches the results.
+static int window_pass(tdsfs_ctx* c, WindowPass tdsfs_ctx::*pass, long long W, bool snp_mode, bool fetch, int64_t cap,
+                       int64_t* n_windows, int (*prepare)(tdsfs_ctx*), void (*launch)(tdsfs_ctx*, unsigned)) {
   if (!c || W < 1) return fail(TDSFS_ERR_ARG, "bad argument");
   if (!c->loaded) return fail(TDSFS_ERR_STATE, "load data first");
+  WindowPass& w = c->*pass;
   CK(cudaSetDevice(c->device));
-  NvtxRange nvtx("tdsfs:diversity (FST, pi, dxy)");
+  NvtxRange nvtx(w.name);
   cudaStream_t st = c->stream;
-  long long ncand;
-  CKR(pass_candidates(c, c->div, W, snp_mode, &ncand));
-  if (out && cap < ncand) return fail(TDSFS_ERR_ARG, "result capacity %lld < %lld candidate windows", (long long)cap, ncand);
+  CKR(cached_candidates(c, w.cand, W, snp_mode, st));
+  const long long ncand = w.cand.off[c->C];
+  if (fetch && cap < ncand) return fail(TDSFS_ERR_ARG, "result capacity %lld < %lld candidate windows", (long long)cap, ncand);
   // windows never overlap, so sum_w ceil(rows_w / SEG) <= S / SEG + ncand
   const long long max_parts = ncand + c->S / DIV_SEG + 1;
-  CKR(ensure_div_buffers(c, ncand, max_parts));
-  c->div.ready = false;
-  c->div.ncand = ncand;
-  CKR(pass_segments(c, c->div, W, snp_mode));
-  CK(cudaEventRecord(c->ev[EV_D0], st));
+  CKR(pass_buffers(c, w, ncand, max_parts));
+  if (prepare) CKR(prepare(c));
+  w.ready = false;
+  w.ncand = ncand;
+  CKR(pass_segments(c, w, W, snp_mode));
+  CK(cudaEventRecord(w.ev0, st));
   if (ncand > 0) {
-    DivParams p;
-    memset(&p, 0, sizeof p);
-    fill_key_params(c, p.k);
-    p.wlo = c->div.d_wlo; p.whi = c->div.d_whi; p.ncand = ncand; p.nseg = c->div.d_nseg; p.segoff = c->div.d_segoff;
-    p.part = c->d_div_part; p.snp_count = c->div.d_count; p.n_sites = c->d_div_nsites; p.pi1 = c->d_div_pi1; p.pi2 = c->d_div_pi2;
-    p.dxy = c->d_div_dxy; p.fst = c->d_div_fst; p.flags = c->div.d_flags;
-    // one warp per segment; the grid covers the bound on the segment count and warps past the actual count return at once
-    void (*kern)(DivParams) = k_diversity<0, 0>;
-    if (c->dG && c->W1 == 32 && c->W2 == 32) kern = k_diversity<32, 32>;       // 500 + 500 diploids (BASELINE config 5)
-    else if (c->dG && c->W1 == 14 && c->W2 == 14) kern = k_diversity<14, 14>;  // 200 + 200 diploids (BASELINE config 4)
-    kern<<<(unsigned)((max_parts + DIV_WARPS - 1) / DIV_WARPS), DIV_WARPS * 32, 0, st>>>(p);
-    k_div_finish<<<(int)((ncand + 255) / 256), 256, 0, st>>>(p);
+    launch(c, (unsigned)((max_parts + DIV_WARPS - 1) / DIV_WARPS));
     c->launches += 2;
     CK(cudaGetLastError());
   }
-  CK(cudaEventRecord(c->ev[EV_D1], st));
-  c->div.timed = true;
-  c->div.ready = true;
-  if (out) return tdsfs_fetch_diversity(c, out, cap, n_windows);
+  CK(cudaEventRecord(w.ev1, st));
+  w.timed = true;
+  w.ready = true;
+  if (fetch) return 0;
   if (n_windows) *n_windows = ncand;
   return finish(c);
+}
+
+// ------------------------------------------------------------------------------------------------ diversity (Hudson FST, pi, dxy)
+extern "C" int tdsfs_fetch_diversity(tdsfs_t* c, tdsfs_diversity_t* out, int64_t cap, int64_t* n_windows) {
+  if (!c || !out) return fail(TDSFS_ERR_ARG, "NULL argument");
+  const WindowPass& w = c->div;
+  if (!w.ready) return fail(TDSFS_ERR_STATE, "no diversity results (tdsfs_diversity_bp / _snp first)");
+  if (cap < w.ncand) return fail(TDSFS_ERR_ARG, "result capacity %lld < %lld candidate windows", (long long)cap, w.ncand);
+  CK(cudaSetDevice(c->device));
+  return fetch_columns(c, w.ncand, {{out->chrom, w.d_wchrom}, {out->start, w.d_wstart}, {out->end, w.d_wend},
+                                    {out->snp_count, w.d_count}, {out->flags, w.d_flags}, {out->n_sites, w.d_i32[0]},
+                                    {out->pi_p1, w.d_f64[0]}, {out->pi_p2, w.d_f64[1]}, {out->dxy, w.d_f64[2]},
+                                    {out->fst, w.d_f64[3]}}, n_windows);
+}
+
+static void launch_diversity(tdsfs_ctx* c, unsigned grid) {
+  const WindowPass& w = c->div;
+  DivParams p;
+  memset(&p, 0, sizeof p);
+  fill_key_params(c, p.k);
+  p.seg = w.segs(); p.part = (DivPart*)w.d_part; p.snp_count = w.d_count; p.flags = w.d_flags; p.n_sites = w.d_i32[0];
+  p.pi1 = w.d_f64[0]; p.pi2 = w.d_f64[1]; p.dxy = w.d_f64[2]; p.fst = w.d_f64[3];
+  const auto kern = segment_kernel(c, k_diversity<32, 32>, k_diversity<14, 14>, k_diversity<0, 0>);
+  kern<<<grid, DIV_WARPS * 32, 0, c->stream>>>(p);
+  k_div_finish<<<(int)((w.ncand + 255) / 256), 256, 0, c->stream>>>(p);
+}
+
+// Per-window Hudson FST, pi and dxy: k_diversity -> k_div_finish.
+static int diversity(tdsfs_ctx* c, long long W, bool snp_mode, tdsfs_diversity_t* out, int64_t cap, int64_t* n_windows) {
+  CKR(window_pass(c, &tdsfs_ctx::div, W, snp_mode, out != nullptr, cap, n_windows, nullptr, launch_diversity));
+  return out ? tdsfs_fetch_diversity(c, out, cap, n_windows) : 0;
 }
 
 extern "C" int tdsfs_diversity_bp(tdsfs_t* c, int64_t W, tdsfs_diversity_t* out, int64_t cap, int64_t* n_windows) {
@@ -1638,113 +1628,58 @@ extern "C" int tdsfs_diversity_snp(tdsfs_t* c, int64_t N, tdsfs_diversity_t* out
 // ------------------------------------------------------------------------------------------------ neutrality (theta_W, Tajima's D)
 extern "C" int tdsfs_fetch_neutrality(tdsfs_t* c, tdsfs_neutrality_t* out, int64_t cap, int64_t* n_windows) {
   if (!c || !out) return fail(TDSFS_ERR_ARG, "NULL argument");
-  if (!c->neut.ready) return fail(TDSFS_ERR_STATE, "no neutrality results (tdsfs_neutrality_bp / _snp first)");
-  if (cap < c->neut.ncand) return fail(TDSFS_ERR_ARG, "result capacity %lld < %lld candidate windows", (long long)cap, c->neut.ncand);
+  const WindowPass& w = c->neut;
+  if (!w.ready) return fail(TDSFS_ERR_STATE, "no neutrality results (tdsfs_neutrality_bp / _snp first)");
+  if (cap < w.ncand) return fail(TDSFS_ERR_ARG, "result capacity %lld < %lld candidate windows", (long long)cap, w.ncand);
   CK(cudaSetDevice(c->device));
-  cudaStream_t st = c->stream;
-  const size_t n = (size_t)c->neut.ncand;
-#define D2H(dst, src, T) \
-  if (out->dst && n) CK(cudaMemcpyAsync(out->dst, c->src, n * sizeof(T), cudaMemcpyDeviceToHost, st))
-  D2H(chrom, neut.d_wchrom, int32_t);
-  D2H(start, neut.d_wstart, long long);
-  D2H(end, neut.d_wend, long long);
-  D2H(snp_count, neut.d_count, int32_t);
-  D2H(flags, neut.d_flags, uint8_t);
-  D2H(n_seg_p1, d_neut_S1, int32_t);
-  D2H(n_seg_p2, d_neut_S2, int32_t);
-  D2H(n_max_p1, d_neut_nmax1, int32_t);
-  D2H(n_max_p2, d_neut_nmax2, int32_t);
-  D2H(theta_pi_p1, d_neut_pi1, double);
-  D2H(theta_pi_p2, d_neut_pi2, double);
-  D2H(theta_w_p1, d_neut_tw1, double);
-  D2H(theta_w_p2, d_neut_tw2, double);
-  D2H(tajima_d_p1, d_neut_d1, double);
-  D2H(tajima_d_p2, d_neut_d2, double);
-#undef D2H
-  CK(cudaStreamSynchronize(st));
-  if (n_windows) *n_windows = c->neut.ncand;
+  return fetch_columns(c, w.ncand, {{out->chrom, w.d_wchrom}, {out->start, w.d_wstart}, {out->end, w.d_wend},
+                                    {out->snp_count, w.d_count}, {out->flags, w.d_flags}, {out->n_seg_p1, w.d_i32[0]},
+                                    {out->n_seg_p2, w.d_i32[1]}, {out->n_max_p1, w.d_i32[2]}, {out->n_max_p2, w.d_i32[3]},
+                                    {out->theta_pi_p1, w.d_f64[0]}, {out->theta_pi_p2, w.d_f64[1]},
+                                    {out->theta_w_p1, w.d_f64[2]}, {out->theta_w_p2, w.d_f64[3]},
+                                    {out->tajima_d_p1, w.d_f64[4]}, {out->tajima_d_p2, w.d_f64[5]}}, n_windows);
+}
+
+// a1(n) and a2(n) for every n a loaded row can reach, summed in ascending k; built again only when a load reaches a
+// larger n (the entries of a longer table are the same numbers)
+static int neut_table(tdsfs_ctx* c) {
+  if (c->n_allele_max <= c->neut_tab_n) return 0;
+  const long long m = c->n_allele_max + 1;
+  std::vector<double> t((size_t)(2 * m), 0.0);
+  for (long long n = 2; n < m; ++n) {
+    const double k = (double)(n - 1);
+    t[n] = t[n - 1] + 1.0 / k;
+    t[m + n] = t[m + n - 1] + 1.0 / (k * k);
+  }
+  CK(cudaStreamSynchronize(c->stream));  // a previous asynchronous call may still read the old table
+  c->neut_tab_n = -1;
+  dev_free(c->d_neut_tab);
+  CKR(dev_alloc(&c->d_neut_tab, 2 * m));
+  CK(cudaMemcpyAsync(c->d_neut_tab, t.data(), (size_t)(2 * m) * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+  c->neut_tab_n = m - 1;
   return 0;
 }
 
-static int ensure_neut_buffers(tdsfs_ctx* c, long long ncand, long long parts) {
-  bool grown;
-  CKR(pass_buffers(c, c->neut, ncand, &grown));
-  if (grown) {
-    dev_free(c->d_neut_S1); dev_free(c->d_neut_S2); dev_free(c->d_neut_nmax1); dev_free(c->d_neut_nmax2);
-    dev_free(c->d_neut_pi1); dev_free(c->d_neut_pi2); dev_free(c->d_neut_tw1); dev_free(c->d_neut_tw2);
-    dev_free(c->d_neut_d1); dev_free(c->d_neut_d2);
-    CKR(dev_alloc(&c->d_neut_S1, ncand)); CKR(dev_alloc(&c->d_neut_S2, ncand)); CKR(dev_alloc(&c->d_neut_nmax1, ncand));
-    CKR(dev_alloc(&c->d_neut_nmax2, ncand)); CKR(dev_alloc(&c->d_neut_pi1, ncand)); CKR(dev_alloc(&c->d_neut_pi2, ncand));
-    CKR(dev_alloc(&c->d_neut_tw1, ncand)); CKR(dev_alloc(&c->d_neut_tw2, ncand)); CKR(dev_alloc(&c->d_neut_d1, ncand));
-    CKR(dev_alloc(&c->d_neut_d2, ncand));
-  }
-  if (parts > c->neut_part_cap) {
-    CK(cudaStreamSynchronize(c->stream));
-    dev_free(c->d_neut_part);
-    CKR(dev_alloc(&c->d_neut_part, parts));
-    c->neut_part_cap = parts;
-  }
-  // a1(n) and a2(n) for every n a loaded row can reach, summed in ascending k; built again only when a load reaches a
-  // larger n (the entries of a longer table are the same numbers)
-  if (c->n_allele_max > c->neut_tab_n) {
-    const long long m = c->n_allele_max + 1;
-    std::vector<double> t((size_t)(2 * m), 0.0);
-    for (long long n = 2; n < m; ++n) {
-      const double k = (double)(n - 1);
-      t[n] = t[n - 1] + 1.0 / k;
-      t[m + n] = t[m + n - 1] + 1.0 / (k * k);
-    }
-    CK(cudaStreamSynchronize(c->stream));  // a previous asynchronous call may still read the old table
-    c->neut_tab_n = -1;
-    dev_free(c->d_neut_tab);
-    CKR(dev_alloc(&c->d_neut_tab, 2 * m));
-    CK(cudaMemcpyAsync(c->d_neut_tab, t.data(), (size_t)(2 * m) * sizeof(double), cudaMemcpyHostToDevice, c->stream));
-    c->neut_tab_n = m - 1;
-  }
-  return 0;
+static void launch_neutrality(tdsfs_ctx* c, unsigned grid) {
+  const WindowPass& w = c->neut;
+  NeutParams p;
+  memset(&p, 0, sizeof p);
+  fill_key_params(c, p.k);
+  p.seg = w.segs(); p.part = (NeutPart*)w.d_part; p.snp_count = w.d_count; p.flags = w.d_flags;
+  p.a1 = c->d_neut_tab; p.a2 = c->d_neut_tab + c->neut_tab_n + 1;
+  p.S1 = w.d_i32[0]; p.S2 = w.d_i32[1]; p.nmax1 = w.d_i32[2]; p.nmax2 = w.d_i32[3];
+  p.theta_pi1 = w.d_f64[0]; p.theta_pi2 = w.d_f64[1]; p.theta_w1 = w.d_f64[2]; p.theta_w2 = w.d_f64[3];
+  p.tajd1 = w.d_f64[4]; p.tajd2 = w.d_f64[5];
+  const auto kern = segment_kernel(c, k_neutrality<32, 32>, k_neutrality<14, 14>, k_neutrality<0, 0>);
+  kern<<<grid, DIV_WARPS * 32, 0, c->stream>>>(p);
+  k_neut_finish<<<(int)((w.ncand + 255) / 256), 256, 0, c->stream>>>(p);
 }
 
-// Per-window, per-population Watterson's theta and Tajima's D over the candidate windows of (W, mode), in the order of
-// tdsfs_scan_*: the segment list (pass_segments) -> k_neutrality (one warp per segment of DIV_SEG rows) -> k_neut_finish.
-// Needs loaded data only; no host round trip when out == NULL (past the first call after a load that needs a larger table).
+// Per-window, per-population Watterson's theta and Tajima's D: k_neutrality -> k_neut_finish.  The first call after a load
+// that needs a larger a1 / a2 table waits for the stream once.
 static int neutrality(tdsfs_ctx* c, long long W, bool snp_mode, tdsfs_neutrality_t* out, int64_t cap, int64_t* n_windows) {
-  if (!c || W < 1) return fail(TDSFS_ERR_ARG, "bad argument");
-  if (!c->loaded) return fail(TDSFS_ERR_STATE, "load data first");
-  CK(cudaSetDevice(c->device));
-  NvtxRange nvtx("tdsfs:neutrality (theta_W, Tajima's D)");
-  cudaStream_t st = c->stream;
-  long long ncand;
-  CKR(pass_candidates(c, c->neut, W, snp_mode, &ncand));
-  if (out && cap < ncand) return fail(TDSFS_ERR_ARG, "result capacity %lld < %lld candidate windows", (long long)cap, ncand);
-  const long long max_parts = ncand + c->S / DIV_SEG + 1;  // as in diversity()
-  CKR(ensure_neut_buffers(c, ncand, max_parts));
-  c->neut.ready = false;
-  c->neut.ncand = ncand;
-  CKR(pass_segments(c, c->neut, W, snp_mode));
-  CK(cudaEventRecord(c->ev[EV_N0], st));
-  if (ncand > 0) {
-    NeutParams p;
-    memset(&p, 0, sizeof p);
-    fill_key_params(c, p.k);
-    p.wlo = c->neut.d_wlo; p.whi = c->neut.d_whi; p.ncand = ncand; p.segoff = c->neut.d_segoff; p.part = c->d_neut_part;
-    p.a1 = c->d_neut_tab; p.a2 = c->d_neut_tab + c->neut_tab_n + 1;
-    p.snp_count = c->neut.d_count; p.S1 = c->d_neut_S1; p.S2 = c->d_neut_S2; p.nmax1 = c->d_neut_nmax1; p.nmax2 = c->d_neut_nmax2;
-    p.theta_pi1 = c->d_neut_pi1; p.theta_pi2 = c->d_neut_pi2; p.theta_w1 = c->d_neut_tw1; p.theta_w2 = c->d_neut_tw2;
-    p.tajd1 = c->d_neut_d1; p.tajd2 = c->d_neut_d2; p.flags = c->neut.d_flags;
-    void (*kern)(NeutParams) = k_neutrality<0, 0>;
-    if (c->dG && c->W1 == 32 && c->W2 == 32) kern = k_neutrality<32, 32>;
-    else if (c->dG && c->W1 == 14 && c->W2 == 14) kern = k_neutrality<14, 14>;
-    kern<<<(unsigned)((max_parts + DIV_WARPS - 1) / DIV_WARPS), DIV_WARPS * 32, 0, st>>>(p);
-    k_neut_finish<<<(int)((ncand + 255) / 256), 256, 0, st>>>(p);
-    c->launches += 2;
-    CK(cudaGetLastError());
-  }
-  CK(cudaEventRecord(c->ev[EV_N1], st));
-  c->neut.timed = true;
-  c->neut.ready = true;
-  if (out) return tdsfs_fetch_neutrality(c, out, cap, n_windows);
-  if (n_windows) *n_windows = ncand;
-  return finish(c);
+  CKR(window_pass(c, &tdsfs_ctx::neut, W, snp_mode, out != nullptr, cap, n_windows, neut_table, launch_neutrality));
+  return out ? tdsfs_fetch_neutrality(c, out, cap, n_windows) : 0;
 }
 
 extern "C" int tdsfs_neutrality_bp(tdsfs_t* c, int64_t W, tdsfs_neutrality_t* out, int64_t cap, int64_t* n_windows) {
@@ -1837,8 +1772,8 @@ extern "C" int tdsfs_timings(tdsfs_t* c, float* ms, int32_t n) {
   }
   c->ms[5] = c->ms[0];
   if (c->x_timed) cudaEventElapsedTime(&c->ms[8], c->ev[EV_X0], c->ev[EV_X1]);
-  if (c->div.timed) cudaEventElapsedTime(&c->ms[9], c->ev[EV_D0], c->ev[EV_D1]);
-  if (c->neut.timed) cudaEventElapsedTime(&c->ms[10], c->ev[EV_N0], c->ev[EV_N1]);
+  if (c->div.timed) cudaEventElapsedTime(&c->ms[9], c->div.ev0, c->div.ev1);
+  if (c->neut.timed) cudaEventElapsedTime(&c->ms[10], c->neut.ev0, c->neut.ev1);
   cudaGetLastError();
   for (int i = 0; i < n && i < 11; ++i) ms[i] = c->ms[i];
   return 0;

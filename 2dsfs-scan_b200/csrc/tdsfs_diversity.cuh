@@ -17,32 +17,20 @@ namespace tdsfs {
 constexpr int DIV_SEG = 1024;   // rows per segment (a multiple of 32)
 constexpr int DIV_WARPS = 8;    // warps per CTA of k_diversity and k_neutrality: one warp per segment
 
-struct DivPart {  // sums of one segment
-  double pi1, pi2, dxy;
-  int n_sites, snp_count;
-};
-
-struct DivParams {
-  KeyParams k;                 // source rows (G or cnt), sample columns, snp_flags + fix-ups (row_filters)
+// The segment list of a pass's candidate windows: window w owns segments [segoff[w], segoff[w + 1]), DIV_SEG rows each
+// counted from its first row (the last one shorter).
+struct SegList {
   const int32_t* wlo;          // [ncand] first row of each candidate window (k2_bounds_*)
   const int32_t* whi;          // [ncand] one past its last row
   long long ncand;
-  long long* nseg;             // [ncand + 1] segments per window, 0 in the last slot
-  const long long* segoff;     // [ncand + 1] exclusive prefix sum of nseg: segoff[ncand] = number of segments
-  DivPart* part;               // [segments]
-  int32_t* snp_count;          // [ncand] outputs
-  int32_t* n_sites;
-  double* pi1;
-  double* pi2;
-  double* dxy;
-  double* fst;
-  uint8_t* flags;
+  const long long* segoff;     // [ncand + 1] exclusive prefix sum of k_div_nseg's counts: segoff[ncand] = number of segments
 };
 
-__global__ void __launch_bounds__(256) k_div_nseg(const __grid_constant__ DivParams p) {
+// Segments per window, 0 in the last slot [ncand]: the exclusive scan of nseg is the segment list's segoff.
+__global__ void __launch_bounds__(256) k_div_nseg(const int32_t* wlo, const int32_t* whi, long long ncand, long long* nseg) {
   const long long id = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (id < p.ncand) p.nseg[id] = (__ldg(p.whi + id) - __ldg(p.wlo + id) + DIV_SEG - 1) / DIV_SEG;
-  else if (id == p.ncand) p.nseg[id] = 0;
+  if (id < ncand) nseg[id] = (__ldg(whi + id) - __ldg(wlo + id) + DIV_SEG - 1) / DIV_SEG;
+  else if (id == ncand) nseg[id] = 0;
 }
 
 // (ref1, alt1, ref2, alt2) of SNP s before the fix-ups: compile-time word counts (fully unrolled, every load of the row
@@ -75,71 +63,107 @@ __device__ __forceinline__ void div_counts(const KeyParams& p, long long s, int&
   }
 }
 
-// One warp per segment.  The warp walks the ALIGNED 32-row blocks that overlap its segment, so word w of a step is exactly
-// one 128-byte line (a window starting inside a block would otherwise split every line of every step in two).  Lane l loads
-// row b + l; its terms then move to the lane that owns that row in the definition, (s - r0) mod 32 = (l - r0) mod 32, which
-// receives its rows in increasing order, one per block: the sums are the definition's, bit for bit.
-template <int TW1, int TW2>
-__global__ void __launch_bounds__(DIV_WARPS * 32) k_diversity(const __grid_constant__ DivParams p) {
-  const int lane = threadIdx.x & 31;
-  const long long g = (long long)blockIdx.x * DIV_WARPS + (threadIdx.x >> 5);
-  if (g >= __ldg(p.segoff + p.ncand)) return;
-  // window of segment g: the last w with segoff[w] <= g (an empty window owns no segment, so it is never the last one)
-  long long lo = 0, hi = p.ncand;
+// Rows [r0, r1) of segment g: segment g - segoff[w] of window w, the last w with segoff[w] <= g (an empty window owns no
+// segment, so it is never the last one).  False for a warp past the last segment: the grid covers a bound on their number.
+__device__ __forceinline__ bool segment_rows(const SegList& seg, long long g, long long& r0, long long& r1) {
+  if (g >= __ldg(seg.segoff + seg.ncand)) return false;
+  long long lo = 0, hi = seg.ncand;
   while (hi - lo > 1) {
     const long long mid = (lo + hi) >> 1;
-    if (__ldg(p.segoff + mid) <= g) lo = mid; else hi = mid;
+    if (__ldg(seg.segoff + mid) <= g) lo = mid; else hi = mid;
   }
-  const long long r0 = (long long)__ldg(p.wlo + lo) + (g - __ldg(p.segoff + lo)) * DIV_SEG;
-  const long long r1 = min(r0 + DIV_SEG, (long long)__ldg(p.whi + lo));
+  r0 = (long long)__ldg(seg.wlo + lo) + (g - __ldg(seg.segoff + lo)) * DIV_SEG;
+  r1 = min(r0 + DIV_SEG, (long long)__ldg(seg.whi + lo));
+  return true;
+}
+
+// The NF fp sums of the segment [r0, r1), taken by one warp in the order that defines them (top of this file).  The warp
+// walks the ALIGNED 32-row blocks that overlap its segment, so word w of a step is exactly one 128-byte line (a window
+// starting inside a block would otherwise split every line of every step in two).  Lane l loads row s = b + l, and
+// row(s, ref1, alt1, ref2, alt2, t) sets that row's terms t[] and adds the pass's integer statistics to the lane's own
+// registers: integers, so the kernel reduces them over the warp at the end in any order.  The terms move to the lane that
+// owns row s in the definition, (s - r0) mod 32 = (l - r0) mod 32, which receives its rows in increasing order, one per
+// block, and a fixed xor tree combines the lanes: the sums are the definition's, bit for bit.
+//
+// Every lane adds a term in every block, +0.0 for a row outside the segment or one that adds no term.  That leaves a sum
+// bitwise unchanged because no term is negative (each is a non-negative integer over a positive one): every sum starts at
+// +0.0, so none is ever -0.0, and x + (+0.0) is x bit for bit for any x but -0.0.  A term that can be negative breaks this.
+template <int TW1, int TW2, int NF, typename Row>
+__device__ __forceinline__ void segment_sums(const KeyParams& k, long long r0, long long r1, double (&sum)[NF], Row row) {
+  const int lane = threadIdx.x & 31;
   const int src = (lane + (int)(r0 & 31)) & 31;  // the lane that loads the row this lane owns
-  double pi1 = 0.0, pi2 = 0.0, dxy = 0.0;
-  int n_sites = 0, snp_count = 0;
+#pragma unroll
+  for (int i = 0; i < NF; ++i) sum[i] = 0.0;
   for (long long b = r0 & ~31LL; b < r1; b += 32) {
     const long long s = b + lane;
-    double t1 = 0.0, t2 = 0.0, td = 0.0;
-    int enter = 0, counted = 0;
+    double t[NF];
+#pragma unroll
+    for (int i = 0; i < NF; ++i) t[i] = 0.0;
     if (s >= r0 && s < r1) {
       int ref1, alt1, ref2, alt2;
-      div_counts<TW1, TW2>(p.k, s, ref1, alt1, ref2, alt2);
-      counted = p.k.flags ? (__ldg(p.k.flags + s) >> 1) & 1 : 1;
-      const bool pass = row_filters(p.k, s, ref1, alt1, ref2, alt2);
-      const long long n1 = ref1 + alt1, n2 = ref2 + alt2;
-      if (pass && n1 >= 2 && n2 >= 2) {
-        t1 = (double)(2LL * ref1 * alt1) / (double)(n1 * (n1 - 1));
-        t2 = (double)(2LL * ref2 * alt2) / (double)(n2 * (n2 - 1));
-        td = (double)((long long)ref1 * alt2 + (long long)alt1 * ref2) / (double)(n1 * n2);
-        enter = 1;
-      }
+      div_counts<TW1, TW2>(k, s, ref1, alt1, ref2, alt2);
+      row(s, ref1, alt1, ref2, alt2, t);
     }
-    t1 = __shfl_sync(0xffffffffu, t1, src);
-    t2 = __shfl_sync(0xffffffffu, t2, src);
-    td = __shfl_sync(0xffffffffu, td, src);
-    enter = __shfl_sync(0xffffffffu, enter, src);
-    snp_count += __shfl_sync(0xffffffffu, counted, src);
-    if (enter) {
-      pi1 += t1; pi2 += t2; dxy += td;
-      ++n_sites;
-    }
+#pragma unroll
+    for (int i = 0; i < NF; ++i) sum[i] += __shfl_sync(0xffffffffu, t[i], src);
   }
 #pragma unroll
   for (int o = 16; o; o >>= 1) {
-    pi1 += __shfl_xor_sync(0xffffffffu, pi1, o);
-    pi2 += __shfl_xor_sync(0xffffffffu, pi2, o);
-    dxy += __shfl_xor_sync(0xffffffffu, dxy, o);
-    n_sites += __shfl_xor_sync(0xffffffffu, n_sites, o);
-    snp_count += __shfl_xor_sync(0xffffffffu, snp_count, o);
+#pragma unroll
+    for (int i = 0; i < NF; ++i) sum[i] += __shfl_xor_sync(0xffffffffu, sum[i], o);
   }
-  if (lane == 0) p.part[g] = DivPart{pi1, pi2, dxy, n_sites, snp_count};
+}
+
+// ------------------------------------------------------------------------------------------------ Hudson FST, pi, dxy
+struct DivPart {  // sums of one segment
+  double pi1, pi2, dxy;
+  int n_sites, snp_count;
+};
+
+struct DivParams {
+  KeyParams k;                 // source rows (G or cnt), sample columns, snp_flags + fix-ups (row_filters)
+  SegList seg;
+  DivPart* part;               // [segments]
+  int32_t* snp_count;          // [ncand] outputs
+  int32_t* n_sites;
+  double* pi1;
+  double* pi2;
+  double* dxy;
+  double* fst;
+  uint8_t* flags;
+};
+
+// One warp per segment: its pi_1, pi_2 and dxy sums, SNPs that entered them and SNPs counted.
+template <int TW1, int TW2>
+__global__ void __launch_bounds__(DIV_WARPS * 32) k_diversity(const __grid_constant__ DivParams p) {
+  const long long g = (long long)blockIdx.x * DIV_WARPS + (threadIdx.x >> 5);
+  long long r0, r1;
+  if (!segment_rows(p.seg, g, r0, r1)) return;
+  double sum[3];  // pi1, pi2, dxy
+  int n_sites = 0, snp_count = 0;
+  segment_sums<TW1, TW2>(p.k, r0, r1, sum, [&](long long s, int ref1, int alt1, int ref2, int alt2, double (&t)[3]) {
+    snp_count += p.k.flags ? (__ldg(p.k.flags + s) >> 1) & 1 : 1;
+    const bool pass = row_filters(p.k, s, ref1, alt1, ref2, alt2);
+    const long long n1 = ref1 + alt1, n2 = ref2 + alt2;
+    if (pass && n1 >= 2 && n2 >= 2) {
+      t[0] = (double)(2LL * ref1 * alt1) / (double)(n1 * (n1 - 1));
+      t[1] = (double)(2LL * ref2 * alt2) / (double)(n2 * (n2 - 1));
+      t[2] = (double)((long long)ref1 * alt2 + (long long)alt1 * ref2) / (double)(n1 * n2);
+      ++n_sites;
+    }
+  });
+  n_sites = __reduce_add_sync(0xffffffffu, n_sites);
+  snp_count = __reduce_add_sync(0xffffffffu, snp_count);
+  if ((threadIdx.x & 31) == 0) p.part[g] = DivPart{sum[0], sum[1], sum[2], n_sites, snp_count};
 }
 
 // One thread per window: its segment sums in segment order, then FST (NaN when dxy == 0).
 __global__ void __launch_bounds__(256) k_div_finish(const __grid_constant__ DivParams p) {
   const long long id = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (id >= p.ncand) return;
+  if (id >= p.seg.ncand) return;
   double pi1 = 0.0, pi2 = 0.0, dxy = 0.0;
   int n_sites = 0, snp_count = 0;
-  for (long long g = __ldg(p.segoff + id), e = __ldg(p.segoff + id + 1); g < e; ++g) {
+  for (long long g = __ldg(p.seg.segoff + id), e = __ldg(p.seg.segoff + id + 1); g < e; ++g) {
     const DivPart q = p.part[g];
     pi1 += q.pi1; pi2 += q.pi2; dxy += q.dxy;
     n_sites += q.n_sites; snp_count += q.snp_count;
@@ -150,7 +174,7 @@ __global__ void __launch_bounds__(256) k_div_finish(const __grid_constant__ DivP
   p.pi2[id] = pi2;
   p.dxy[id] = dxy;
   p.fst[id] = dxy == 0.0 ? __longlong_as_double(0x7FF8000000000000LL) : 1.0 - (pi1 + pi2) / (2.0 * dxy);
-  p.flags[id] = __ldg(p.whi + id) == __ldg(p.wlo + id) ? TDSFS_F_EMPTY : 0;
+  p.flags[id] = __ldg(p.seg.whi + id) == __ldg(p.seg.wlo + id) ? TDSFS_F_EMPTY : 0;
 }
 
 // ------------------------------------------------------------------------------------------------ neutrality
@@ -167,10 +191,7 @@ struct NeutPart {  // sums of one segment
 
 struct NeutParams {
   KeyParams k;                 // source rows, sample columns, snp_flags + fix-ups
-  const int32_t* wlo;          // [ncand] first row of each candidate window
-  const int32_t* whi;          // [ncand] one past its last row
-  long long ncand;
-  const long long* segoff;     // [ncand + 1] the segment list (k_div_nseg + exclusive scan)
+  SegList seg;
   NeutPart* part;              // [segments]
   const double* a1;            // [tab_n + 1] a1(n) = sum_{k=1}^{n-1} 1/k, ascending k; a1(0) = a1(1) = 0
   const double* a2;            // [tab_n + 1] a2(n) = sum_{k=1}^{n-1} 1/k^2
@@ -188,56 +209,32 @@ struct NeutParams {
   uint8_t* flags;
 };
 
-// One warp per segment, walking aligned 32-row blocks as k_diversity does.  Only the theta_pi terms depend on the order in
-// which they are added, so only they move to the owning lane; the integer counts and maxima are reduced at the end.
+// One warp per segment: its theta_pi sums, segregating sites, largest n and SNPs counted, per population.
 template <int TW1, int TW2>
 __global__ void __launch_bounds__(DIV_WARPS * 32) k_neutrality(const __grid_constant__ NeutParams p) {
-  const int lane = threadIdx.x & 31;
   const long long g = (long long)blockIdx.x * DIV_WARPS + (threadIdx.x >> 5);
-  if (g >= __ldg(p.segoff + p.ncand)) return;
-  // window of segment g, as in k_diversity
-  long long lo = 0, hi = p.ncand;
-  while (hi - lo > 1) {
-    const long long mid = (lo + hi) >> 1;
-    if (__ldg(p.segoff + mid) <= g) lo = mid; else hi = mid;
-  }
-  const long long r0 = (long long)__ldg(p.wlo + lo) + (g - __ldg(p.segoff + lo)) * DIV_SEG;
-  const long long r1 = min(r0 + DIV_SEG, (long long)__ldg(p.whi + lo));
-  const int src = (lane + (int)(r0 & 31)) & 31;  // the lane that loads the row this lane owns
-  double pi1 = 0.0, pi2 = 0.0;
+  long long r0, r1;
+  if (!segment_rows(p.seg, g, r0, r1)) return;
+  double sum[2];  // theta_pi1, theta_pi2
   int S1 = 0, S2 = 0, nmax1 = 0, nmax2 = 0, snp_count = 0;
-  for (long long b = r0 & ~31LL; b < r1; b += 32) {
-    const long long s = b + lane;
-    double t1 = 0.0, t2 = 0.0;
-    if (s >= r0 && s < r1) {
-      int ref1, alt1, ref2, alt2;
-      div_counts<TW1, TW2>(p.k, s, ref1, alt1, ref2, alt2);
-      snp_count += p.k.flags ? (__ldg(p.k.flags + s) >> 1) & 1 : 1;
-      if (row_filters(p.k, s, ref1, alt1, ref2, alt2)) {
-        const long long n1 = ref1 + alt1, n2 = ref2 + alt2;
-        S1 += ref1 > 0 && alt1 > 0;
-        S2 += ref2 > 0 && alt2 > 0;
-        nmax1 = max(nmax1, (int)n1);
-        nmax2 = max(nmax2, (int)n2);
-        if (n1 >= 2) t1 = (double)(2LL * ref1 * alt1) / (double)(n1 * (n1 - 1));
-        if (n2 >= 2) t2 = (double)(2LL * ref2 * alt2) / (double)(n2 * (n2 - 1));
-      }
+  segment_sums<TW1, TW2>(p.k, r0, r1, sum, [&](long long s, int ref1, int alt1, int ref2, int alt2, double (&t)[2]) {
+    snp_count += p.k.flags ? (__ldg(p.k.flags + s) >> 1) & 1 : 1;
+    if (row_filters(p.k, s, ref1, alt1, ref2, alt2)) {
+      const long long n1 = ref1 + alt1, n2 = ref2 + alt2;
+      S1 += ref1 > 0 && alt1 > 0;
+      S2 += ref2 > 0 && alt2 > 0;
+      nmax1 = max(nmax1, (int)n1);
+      nmax2 = max(nmax2, (int)n2);
+      if (n1 >= 2) t[0] = (double)(2LL * ref1 * alt1) / (double)(n1 * (n1 - 1));
+      if (n2 >= 2) t[1] = (double)(2LL * ref2 * alt2) / (double)(n2 * (n2 - 1));
     }
-    // a row that adds no term adds +0.0, which leaves the (never negative zero) sum bitwise unchanged
-    pi1 += __shfl_sync(0xffffffffu, t1, src);
-    pi2 += __shfl_sync(0xffffffffu, t2, src);
-  }
-#pragma unroll
-  for (int o = 16; o; o >>= 1) {
-    pi1 += __shfl_xor_sync(0xffffffffu, pi1, o);
-    pi2 += __shfl_xor_sync(0xffffffffu, pi2, o);
-  }
+  });
   S1 = __reduce_add_sync(0xffffffffu, S1);
   S2 = __reduce_add_sync(0xffffffffu, S2);
   snp_count = __reduce_add_sync(0xffffffffu, snp_count);
   nmax1 = __reduce_max_sync(0xffffffffu, nmax1);
   nmax2 = __reduce_max_sync(0xffffffffu, nmax2);
-  if (lane == 0) p.part[g] = NeutPart{pi1, pi2, S1, S2, nmax1, nmax2, snp_count};
+  if ((threadIdx.x & 31) == 0) p.part[g] = NeutPart{sum[0], sum[1], S1, S2, nmax1, nmax2, snp_count};
 }
 
 // Watterson's theta and Tajima's D of one population from (theta_pi, S, n_max); NaN where undefined.
@@ -261,10 +258,10 @@ __device__ __forceinline__ void tajima(const NeutParams& p, double pi, int S, in
 // One thread per window: its segment parts in segment order (maxima for n_max), then theta_W and Tajima's D.
 __global__ void __launch_bounds__(256) k_neut_finish(const __grid_constant__ NeutParams p) {
   const long long id = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (id >= p.ncand) return;
+  if (id >= p.seg.ncand) return;
   double pi1 = 0.0, pi2 = 0.0;
   int S1 = 0, S2 = 0, nmax1 = 0, nmax2 = 0, snp_count = 0;
-  for (long long g = __ldg(p.segoff + id), e = __ldg(p.segoff + id + 1); g < e; ++g) {
+  for (long long g = __ldg(p.seg.segoff + id), e = __ldg(p.seg.segoff + id + 1); g < e; ++g) {
     const NeutPart q = p.part[g];
     pi1 += q.theta_pi1; pi2 += q.theta_pi2;
     S1 += q.S1; S2 += q.S2; snp_count += q.snp_count;
@@ -279,7 +276,7 @@ __global__ void __launch_bounds__(256) k_neut_finish(const __grid_constant__ Neu
   p.theta_pi1[id] = pi1; p.theta_pi2[id] = pi2;
   p.theta_w1[id] = tw1; p.theta_w2[id] = tw2;
   p.tajd1[id] = d1; p.tajd2[id] = d2;
-  p.flags[id] = __ldg(p.whi + id) == __ldg(p.wlo + id) ? TDSFS_F_EMPTY : 0;
+  p.flags[id] = __ldg(p.seg.whi + id) == __ldg(p.seg.wlo + id) ? TDSFS_F_EMPTY : 0;
 }
 
 }  // namespace tdsfs

@@ -28,6 +28,8 @@ EXPORTS = [
 
 
 PEER_BLOB_BYTES = 192  # TDSFS_PEER_BLOB_BYTES
+TIMING_NAMES = ("k1_count", "finalize", "k2_bounds", "k3_small", "k3_large", "background_call", "scan_call", "pass_total",
+                "exchange", "diversity", "neutrality")  # the slots of tdsfs_timings
 
 
 class TdsfsError(RuntimeError):
@@ -43,34 +45,29 @@ class Fixup(C.Structure):
 FIXUP_DTYPE = np.dtype([("snp", "<i8"), ("pop", "<i4"), ("dref", "<i4"), ("dalt", "<i4")], align=True)
 
 
-class Result(C.Structure):
-    _fields_ = [("chrom", C.c_void_p), ("start", C.c_void_p), ("end", C.c_void_p), ("snp_count", C.c_void_p),
-                ("n2d", C.c_void_p), ("n1d_p1", C.c_void_p), ("n1d_p2", C.c_void_p), ("T2D", C.c_void_p),
-                ("T1D_p1", C.c_void_p), ("T1D_p2", C.c_void_p), ("flags", C.c_void_p)]
-
-
+# Per-window result columns in the member order of tdsfs_result_t, tdsfs_diversity_t and tdsfs_neutrality_t: each of
+# those structs holds one host pointer per column.
 RESULT_DTYPES = dict(chrom=np.int32, start=np.int64, end=np.int64, snp_count=np.int32, n2d=np.int32, n1d_p1=np.int32,
                      n1d_p2=np.int32, T2D=np.float64, T1D_p1=np.float64, T1D_p2=np.float64, flags=np.uint8)
-
-class Diversity(C.Structure):
-    _fields_ = [("chrom", C.c_void_p), ("start", C.c_void_p), ("end", C.c_void_p), ("snp_count", C.c_void_p), ("flags", C.c_void_p),
-                ("n_sites", C.c_void_p), ("pi_p1", C.c_void_p), ("pi_p2", C.c_void_p), ("dxy", C.c_void_p), ("fst", C.c_void_p)]
-
-
 DIVERSITY_DTYPES = dict(chrom=np.int32, start=np.int64, end=np.int64, snp_count=np.int32, flags=np.uint8, n_sites=np.int32,
                         pi_p1=np.float64, pi_p2=np.float64, dxy=np.float64, fst=np.float64)
-
-
-class Neutrality(C.Structure):
-    _fields_ = [(k, C.c_void_p) for k in ("chrom", "start", "end", "snp_count", "flags", "n_seg_p1", "n_seg_p2", "n_max_p1",
-                                          "n_max_p2", "theta_pi_p1", "theta_pi_p2", "theta_w_p1", "theta_w_p2",
-                                          "tajima_d_p1", "tajima_d_p2")]
-
-
 NEUTRALITY_DTYPES = dict(chrom=np.int32, start=np.int64, end=np.int64, snp_count=np.int32, flags=np.uint8, n_seg_p1=np.int32,
                          n_seg_p2=np.int32, n_max_p1=np.int32, n_max_p2=np.int32, theta_pi_p1=np.float64,
                          theta_pi_p2=np.float64, theta_w_p1=np.float64, theta_w_p2=np.float64, tajima_d_p1=np.float64,
                          tajima_d_p2=np.float64)
+
+
+class Result(C.Structure):
+    _fields_ = [(k, C.c_void_p) for k in RESULT_DTYPES]
+
+
+class Diversity(C.Structure):
+    _fields_ = [(k, C.c_void_p) for k in DIVERSITY_DTYPES]
+
+
+class Neutrality(C.Structure):
+    _fields_ = [(k, C.c_void_p) for k in NEUTRALITY_DTYPES]
+
 
 _lib = None
 
@@ -227,11 +224,8 @@ class Handle:
 
     def scan_poisson(self, window_bp):
         """Poisson composite score of every fixed-bp window: dict of arrays, T2D = the score."""
-        cap = self.candidates(window_bp, False)
-        arrs, r = self._alloc_result(cap)
-        n = C.c_int64()
-        self._check(self._L.tdsfs_scan_poisson_bp(self._h, C.c_int64(window_bp), C.byref(r), C.c_int64(cap), C.byref(n)))
-        return {k: v[:n.value] for k, v in arrs.items()}
+        return self._into(self._alloc_result, self.candidates(window_bp, False), self._L.tdsfs_scan_poisson_bp,
+                          C.c_int64(window_bp))
 
     def finalize_background(self):
         self._check(self._L.tdsfs_finalize_background(self._h))
@@ -249,48 +243,53 @@ class Handle:
         return n.value
 
     @staticmethod
+    def _alloc(dtypes, struct, n):
+        """Zeroed host arrays for n windows (at least one) and the result struct pointing at them."""
+        arrs = {k: np.zeros(max(n, 1), dtype=dt) for k, dt in dtypes.items()}
+        return arrs, struct(**{k: v.ctypes.data for k, v in arrs.items()})
+
+    @staticmethod
     def _alloc_result(n):
-        arrs = {k: np.zeros(max(n, 1), dtype=dt) for k, dt in RESULT_DTYPES.items()}
-        r = Result(**{k: v.ctypes.data for k, v in arrs.items()})
-        return arrs, r
+        return Handle._alloc(RESULT_DTYPES, Result, n)
+
+    @staticmethod
+    def _alloc_diversity(n):
+        return Handle._alloc(DIVERSITY_DTYPES, Diversity, n)
+
+    @staticmethod
+    def _alloc_neutrality(n):
+        return Handle._alloc(NEUTRALITY_DTYPES, Neutrality, n)
+
+    def _into(self, alloc, cap, f, *args):
+        """f(handle, *args, out, cap, &n) into the arrays alloc(cap) allocates: dict of their first n entries."""
+        arrs, r = alloc(cap)
+        n = C.c_int64()
+        self._check(f(self._h, *args, C.byref(r), C.c_int64(cap), C.byref(n)))
+        return {k: v[:n.value] for k, v in arrs.items()}
+
+    def _run(self, entry, alloc, size, snp_mode, fetch):
+        """Run tdsfs_<entry>_bp / _snp over the candidate windows of (size, mode): a dict of arrays, or the candidate count
+        when fetch=False (the results stay on the device)."""
+        f = getattr(self._L, f"tdsfs_{entry}_{'snp' if snp_mode else 'bp'}")
+        if not fetch:
+            n = C.c_int64()
+            self._check(f(self._h, C.c_int64(size), None, C.c_int64(0), C.byref(n)))
+            return n.value
+        return self._into(alloc, self.candidates(size, snp_mode), f, C.c_int64(size))
 
     def scan(self, size, snp_mode=False, fetch=True):
         """Run K2 + K3/K4.  Returns dict of numpy arrays (one entry per candidate window) or the candidate count."""
-        f = self._L.tdsfs_scan_snp if snp_mode else self._L.tdsfs_scan_bp
-        n = C.c_int64()
-        if not fetch:
-            self._check(f(self._h, C.c_int64(size), None, C.c_int64(0), C.byref(n)))
-            return n.value
-        cap = self.candidates(size, snp_mode)
-        arrs, r = self._alloc_result(cap)
-        self._check(f(self._h, C.c_int64(size), C.byref(r), C.c_int64(cap), C.byref(n)))
-        return {k: v[:n.value] for k, v in arrs.items()}
+        return self._run("scan", self._alloc_result, size, snp_mode, fetch)
 
     def diversity(self, size, snp_mode=False, fetch=True):
         """Per-window Hudson FST, pi and dxy over the candidate windows of (size, mode), in scan order (tdsfs_diversity_*).
         pi_p1 / pi_p2 / dxy are sums over the variant sites that entered (n_sites), not per-bp values; fst is NaN when
         dxy == 0.  Returns a dict of arrays (chrom / start / end / snp_count / flags as the scan's), or the candidate count
         when fetch=False (results stay on the device: fetch_diversity)."""
-        f = self._L.tdsfs_diversity_snp if snp_mode else self._L.tdsfs_diversity_bp
-        n = C.c_int64()
-        if not fetch:
-            self._check(f(self._h, C.c_int64(size), None, C.c_int64(0), C.byref(n)))
-            return n.value
-        cap = self.candidates(size, snp_mode)
-        arrs, r = self._alloc_diversity(cap)
-        self._check(f(self._h, C.c_int64(size), C.byref(r), C.c_int64(cap), C.byref(n)))
-        return {k: v[:n.value] for k, v in arrs.items()}
-
-    @staticmethod
-    def _alloc_diversity(n):
-        arrs = {k: np.zeros(max(n, 1), dtype=dt) for k, dt in DIVERSITY_DTYPES.items()}
-        return arrs, Diversity(**{k: v.ctypes.data for k, v in arrs.items()})
+        return self._run("diversity", self._alloc_diversity, size, snp_mode, fetch)
 
     def fetch_diversity(self, cap):
-        arrs, r = self._alloc_diversity(cap)
-        n = C.c_int64()
-        self._check(self._L.tdsfs_fetch_diversity(self._h, C.byref(r), C.c_int64(cap), C.byref(n)))
-        return {k: v[:n.value] for k, v in arrs.items()}
+        return self._into(self._alloc_diversity, cap, self._L.tdsfs_fetch_diversity)
 
     def neutrality(self, size, snp_mode=False, fetch=True):
         """Per-window, per-population Watterson's theta and Tajima's D over the candidate windows of (size, mode), in scan
@@ -298,42 +297,21 @@ class Handle:
         theta_w_p* absolute (not per-bp) estimators, tajima_d_p* at n = n_max_p* (NaN with fewer than 3 segregating sites).
         Returns a dict of arrays (chrom / start / end / snp_count / flags as the scan's), or the candidate count when
         fetch=False (results stay on the device: fetch_neutrality)."""
-        f = self._L.tdsfs_neutrality_snp if snp_mode else self._L.tdsfs_neutrality_bp
-        n = C.c_int64()
-        if not fetch:
-            self._check(f(self._h, C.c_int64(size), None, C.c_int64(0), C.byref(n)))
-            return n.value
-        cap = self.candidates(size, snp_mode)
-        arrs, r = self._alloc_neutrality(cap)
-        self._check(f(self._h, C.c_int64(size), C.byref(r), C.c_int64(cap), C.byref(n)))
-        return {k: v[:n.value] for k, v in arrs.items()}
-
-    @staticmethod
-    def _alloc_neutrality(n):
-        arrs = {k: np.zeros(max(n, 1), dtype=dt) for k, dt in NEUTRALITY_DTYPES.items()}
-        return arrs, Neutrality(**{k: v.ctypes.data for k, v in arrs.items()})
+        return self._run("neutrality", self._alloc_neutrality, size, snp_mode, fetch)
 
     def fetch_neutrality(self, cap):
-        arrs, r = self._alloc_neutrality(cap)
-        n = C.c_int64()
-        self._check(self._L.tdsfs_fetch_neutrality(self._h, C.byref(r), C.c_int64(cap), C.byref(n)))
-        return {k: v[:n.value] for k, v in arrs.items()}
+        return self._into(self._alloc_neutrality, cap, self._L.tdsfs_fetch_neutrality)
 
     def fetch_results(self, cap):
-        arrs, r = self._alloc_result(cap)
-        n = C.c_int64()
-        self._check(self._L.tdsfs_fetch_results(self._h, C.byref(r), C.c_int64(cap), C.byref(n)))
-        return {k: v[:n.value] for k, v in arrs.items()}
+        return self._into(self._alloc_result, cap, self._L.tdsfs_fetch_results)
 
     def run_bp(self, bg_mode, W, fetch=True):
-        n = C.c_int64()
         if not fetch:
+            n = C.c_int64()
             self._check(self._L.tdsfs_run_bp(self._h, C.c_int32(bg_mode), C.c_int64(W), None, C.c_int64(0), C.byref(n)))
             return n.value
-        cap = self.candidates(W, False)
-        arrs, r = self._alloc_result(cap)
-        self._check(self._L.tdsfs_run_bp(self._h, C.c_int32(bg_mode), C.c_int64(W), C.byref(r), C.c_int64(cap), C.byref(n)))
-        return {k: v[:n.value] for k, v in arrs.items()}
+        return self._into(self._alloc_result, self.candidates(W, False), self._L.tdsfs_run_bp, C.c_int32(bg_mode),
+                          C.c_int64(W))
 
     def step_bp(self, bg_mode, W):
         """One whole asynchronous pass (CUDA graph after the first two calls); results stay on the device."""
@@ -369,22 +347,17 @@ class Handle:
                                                   C.c_double(missing_rate), C.c_double(fst)))
 
     def timings(self):
-        ms = (C.c_float * 10)()
-        self._check(self._L.tdsfs_timings(self._h, ms, C.c_int32(10)))
-        names = ["k1_count", "finalize", "k2_bounds", "k3_small", "k3_large", "background_call", "scan_call", "pass_total", "exchange"]
-        return dict(zip(names, list(ms)))
+        ms = (C.c_float * len(TIMING_NAMES))()
+        self._check(self._L.tdsfs_timings(self._h, ms, C.c_int32(len(ms))))
+        return dict(zip(TIMING_NAMES, list(ms)))
 
     def diversity_ms(self):
         """CUDA-event time (ms) of the segment + finish kernels of the last diversity call (tdsfs_timings slot 9)."""
-        ms = (C.c_float * 10)()
-        self._check(self._L.tdsfs_timings(self._h, ms, C.c_int32(10)))
-        return float(ms[9])
+        return self.timings()["diversity"]
 
     def neutrality_ms(self):
         """CUDA-event time (ms) of the segment + finish kernels of the last neutrality call (tdsfs_timings slot 10)."""
-        ms = (C.c_float * 11)()
-        self._check(self._L.tdsfs_timings(self._h, ms, C.c_int32(11)))
-        return float(ms[10])
+        return self.timings()["neutrality"]
 
     def launch_count(self):
         return int(self._L.tdsfs_launch_count(self._h))
