@@ -18,7 +18,7 @@
 
 using namespace tdsfs;
 
-#define TDSFS_VERSION 202
+#define TDSFS_VERSION 203
 
 static thread_local std::string g_err;
 
@@ -82,13 +82,13 @@ struct CandCache {
 };
 
 // Workspace and results of one per-window pass over the candidate windows of (size, mode) (tdsfs_diversity_*,
-// tdsfs_neutrality_*): its candidate offsets, window boundaries, segment list, scan scratch, per-segment sums, per-window
+// tdsfs_neutrality_*, tdsfs_wcfst_*): its candidate offsets, window boundaries, segment list, scan scratch, per-segment sums, per-window
 // results and events.
 struct WindowPass {
   WindowPass(const char* name, size_t part_bytes, int n_i32, int n_f64)
       : name(name), part_bytes(part_bytes), n_i32(n_i32), n_f64(n_f64) {}
   const char* name;                   // NVTX range of a call
-  size_t part_bytes;                  // size of the pass's per-segment sums (DivPart, NeutPart)
+  size_t part_bytes;                  // size of the pass's per-segment sums (DivPart, NeutPart, WcPart)
   int n_i32, n_f64;                   // result columns of the pass in d_i32 / d_f64
   CandCache cand;
   long long cap = 0, ncand = 0;       // windows the per-window arrays hold / of the last call
@@ -128,6 +128,7 @@ struct tdsfs_ctx {
   const int32_t* dPos = nullptr;
   bool own_pos = false;
   bool loaded = false;     // a (possibly empty) data set is loaded
+  bool genotypes = false;  // ... through tdsfs_load_genotypes: the 2-bit calls are on the device
   const uint8_t* dFlags = nullptr;
   bool own_flags = false;
   tdsfs_fixup_t* dFix = nullptr;
@@ -212,12 +213,13 @@ struct tdsfs_ctx {
   // the scan's plan, window buffers or unfetched results, nor the other pass's
   WindowPass div{"tdsfs:diversity (FST, pi, dxy)", sizeof(DivPart), 1, 4};                 // tdsfs_diversity_*
   WindowPass neut{"tdsfs:neutrality (theta_W, Tajima's D)", sizeof(NeutPart), 4, 6};      // tdsfs_neutrality_*
+  WindowPass wc{"tdsfs:Weir and Cockerham FST", sizeof(WcPart), 1, 4};                    // tdsfs_wcfst_*
   double* d_neut_tab = nullptr;       // a1(n) for n in [0, neut_tab_n], then a2(n) for the same n
   long long neut_tab_n = -1;
   long long n_allele_max = 0;         // the largest n_i = ref_i + alt_i a row of the loaded data can reach
   // instrumentation
   cudaEvent_t ev[NEV] = {};
-  float ms[11] = {};
+  float ms[12] = {};
   long long launches = 0;
 };
 
@@ -286,7 +288,7 @@ extern "C" int tdsfs_create(int device, tdsfs_t** out) {
   CK(cudaEventCreate(&c->ev_plan0));
   c->stream = c->own_stream;
   for (int i = 0; i < NEV; ++i) CK(cudaEventCreate(&c->ev[i]));
-  for (WindowPass* w : {&c->div, &c->neut}) {
+  for (WindowPass* w : {&c->div, &c->neut, &c->wc}) {
     CK(cudaEventCreate(&w->ev0));
     CK(cudaEventCreate(&w->ev1));
   }
@@ -336,7 +338,7 @@ static void free_data(tdsfs_ctx* c) {
   if (c->plan_W >= 0 && c->ev_plan) cudaStreamWaitEvent(c->stream, c->ev_plan, 0);
   c->dG = nullptr; c->dCnt = nullptr; c->dPos = nullptr; c->dFlags = nullptr;
   c->own_G = c->own_cnt = c->own_pos = c->own_flags = false;
-  c->loaded = false;
+  c->loaded = c->genotypes = false;
   dev_free(c->dFix);
   c->nfix = 0;
   c->d_off = nullptr;  // pooled (pool_off)
@@ -348,7 +350,7 @@ static void free_data(tdsfs_ctx* c) {
   c->plan_W = -1;
   c->ws_ready = false;
   c->force_wide = false;
-  for (WindowPass* w : {&c->div, &c->neut}) {
+  for (WindowPass* w : {&c->div, &c->neut, &c->wc}) {
     w->cand.W = -1;
     w->ready = false;
   }
@@ -396,6 +398,7 @@ extern "C" void tdsfs_destroy(tdsfs_t* c) {
   dev_free(c->d_dxI); dev_free(c->d_ws); dev_free(c->d_gridbar); dev_free(c->d_stamps);
   free_window_pass(c->div);
   free_window_pass(c->neut);
+  free_window_pass(c->wc);
   dev_free(c->d_neut_tab);
   cudaStreamDestroy(c->own_stream);
   cudaStreamDestroy(c->copy_stream);
@@ -543,6 +546,7 @@ extern "C" int tdsfs_load_genotypes(tdsfs_t* c, const void* G, int64_t S, int32_
   const bool has_fix = fixups && n_fixups > 0;
   CKR(load_common(c, S, pos, (const long long*)chrom_off, C, snp_flags, has_fix));
   c->W1 = words1; c->W2 = words2; c->ns1 = ns1; c->ns2 = ns2;
+  c->genotypes = true;
   c->n_allele_max = 2LL * std::max(ns1, ns2);
   const long long RW = words1 + words2;
   if (has_fix) {
@@ -1553,8 +1557,8 @@ static auto segment_kernel(const tdsfs_ctx* c, void (*k32)(P), void (*k14)(P), v
 // One per-window pass over the candidate windows of (W, mode), in the order of tdsfs_scan_*: the segment list
 // (pass_segments), then launch(c, grid): the pass's params, its segment kernel on `grid` CTAs (one warp per segment of
 // DIV_SEG rows; warps past the actual count return at once) and its finish kernel.  prepare (NULL: none) sets up what else
-// those kernels read, before the timed range.  Needs loaded data only, and no host round trip when !fetch; when fetch, the
-// caller fetches the results.
+// those kernels read, before the timed range, or rejects the loaded data.  Needs loaded data only, and no host round trip
+// when !fetch; when fetch, the caller fetches the results.
 static int window_pass(tdsfs_ctx* c, WindowPass tdsfs_ctx::*pass, long long W, bool snp_mode, bool fetch, int64_t cap,
                        int64_t* n_windows, int (*prepare)(tdsfs_ctx*), void (*launch)(tdsfs_ctx*, unsigned)) {
   if (!c || W < 1) return fail(TDSFS_ERR_ARG, "bad argument");
@@ -1689,6 +1693,55 @@ extern "C" int tdsfs_neutrality_snp(tdsfs_t* c, int64_t N, tdsfs_neutrality_t* o
   return neutrality(c, N, true, out, cap, n_windows);
 }
 
+// ------------------------------------------------------------------------------------------------ Weir and Cockerham's FST
+extern "C" int tdsfs_fetch_wcfst(tdsfs_t* c, tdsfs_wcfst_t* out, int64_t cap, int64_t* n_windows) {
+  if (!c || !out) return fail(TDSFS_ERR_ARG, "NULL argument");
+  const WindowPass& w = c->wc;
+  if (!w.ready) return fail(TDSFS_ERR_STATE, "no Weir and Cockerham FST results (tdsfs_wcfst_bp / _snp first)");
+  if (cap < w.ncand) return fail(TDSFS_ERR_ARG, "result capacity %lld < %lld candidate windows", (long long)cap, w.ncand);
+  CK(cudaSetDevice(c->device));
+  return fetch_columns(c, w.ncand, {{out->chrom, w.d_wchrom}, {out->start, w.d_wstart}, {out->end, w.d_wend},
+                                    {out->snp_count, w.d_count}, {out->flags, w.d_flags}, {out->n_sites, w.d_i32[0]},
+                                    {out->a, w.d_f64[0]}, {out->b, w.d_f64[1]}, {out->c, w.d_f64[2]},
+                                    {out->fst, w.d_f64[3]}}, n_windows);
+}
+
+// The pass reads heterozygote counts, which only the 2-bit calls hold, and its int64 terms are exact up to WC_MAX_SAMPLES
+// samples per population.
+static int wc_check(tdsfs_ctx* c) {
+  if (!c->genotypes)
+    return fail(TDSFS_ERR_STATE, "Weir and Cockerham FST needs genotype calls (tdsfs_load_genotypes): the counts entry has no heterozygote counts");
+  if (c->ns1 > WC_MAX_SAMPLES || c->ns2 > WC_MAX_SAMPLES)
+    return fail(TDSFS_ERR_ARG, "Weir and Cockerham FST takes at most %d samples per population (%d + %d loaded): its int64 terms would overflow",
+                WC_MAX_SAMPLES, c->ns1, c->ns2);
+  return 0;
+}
+
+static void launch_wcfst(tdsfs_ctx* c, unsigned grid) {
+  const WindowPass& w = c->wc;
+  WcParams p;
+  memset(&p, 0, sizeof p);
+  fill_key_params(c, p.k);
+  p.seg = w.segs(); p.part = (WcPart*)w.d_part; p.snp_count = w.d_count; p.flags = w.d_flags; p.n_sites = w.d_i32[0];
+  p.a = w.d_f64[0]; p.b = w.d_f64[1]; p.c = w.d_f64[2]; p.fst = w.d_f64[3];
+  const auto kern = segment_kernel(c, k_wcfst<32, 32>, k_wcfst<14, 14>, k_wcfst<0, 0>);
+  kern<<<grid, DIV_WARPS * 32, 0, c->stream>>>(p);
+  k_wc_finish<<<(int)((w.ncand + 255) / 256), 256, 0, c->stream>>>(p);
+}
+
+// Per-window Weir and Cockerham FST from the genotype calls: k_wcfst -> k_wc_finish.
+static int wcfst(tdsfs_ctx* c, long long W, bool snp_mode, tdsfs_wcfst_t* out, int64_t cap, int64_t* n_windows) {
+  CKR(window_pass(c, &tdsfs_ctx::wc, W, snp_mode, out != nullptr, cap, n_windows, wc_check, launch_wcfst));
+  return out ? tdsfs_fetch_wcfst(c, out, cap, n_windows) : 0;
+}
+
+extern "C" int tdsfs_wcfst_bp(tdsfs_t* c, int64_t W, tdsfs_wcfst_t* out, int64_t cap, int64_t* n_windows) {
+  return wcfst(c, W, false, out, cap, n_windows);
+}
+extern "C" int tdsfs_wcfst_snp(tdsfs_t* c, int64_t N, tdsfs_wcfst_t* out, int64_t cap, int64_t* n_windows) {
+  return wcfst(c, N, true, out, cap, n_windows);
+}
+
 // ------------------------------------------------------------------------------------------------ explicit likelihood
 extern "C" int tdsfs_likelihood(tdsfs_t* c, const int64_t* x, const double* b, int64_t n, double B, double* T, int32_t* flag) {
   if (!c || !T || !flag || n < 0 || (n > 0 && (!x || !b))) return fail(TDSFS_ERR_ARG, "bad argument");
@@ -1759,7 +1812,7 @@ extern "C" int tdsfs_timings(tdsfs_t* c, float* ms, int32_t n) {
   if (!c || !ms) return fail(TDSFS_ERR_ARG, "NULL argument");
   CK(cudaSetDevice(c->device));
   CK(cudaStreamSynchronize(c->stream));
-  for (int i = 0; i < 11; ++i) c->ms[i] = 0.f;
+  for (int i = 0; i < 12; ++i) c->ms[i] = 0.f;
   if (c->keys_ready) cudaEventElapsedTime(&c->ms[0], c->ev[EV_BG0], c->ev[EV_K1]);
   if (c->fin_timed) cudaEventElapsedTime(&c->ms[1], c->ev[EV_FIN0], c->ev[EV_FIN1]);
   if (c->results_ready) {
@@ -1774,8 +1827,9 @@ extern "C" int tdsfs_timings(tdsfs_t* c, float* ms, int32_t n) {
   if (c->x_timed) cudaEventElapsedTime(&c->ms[8], c->ev[EV_X0], c->ev[EV_X1]);
   if (c->div.timed) cudaEventElapsedTime(&c->ms[9], c->div.ev0, c->div.ev1);
   if (c->neut.timed) cudaEventElapsedTime(&c->ms[10], c->neut.ev0, c->neut.ev1);
+  if (c->wc.timed) cudaEventElapsedTime(&c->ms[11], c->wc.ev0, c->wc.ev1);
   cudaGetLastError();
-  for (int i = 0; i < n && i < 11; ++i) ms[i] = c->ms[i];
+  for (int i = 0; i < n && i < 12; ++i) ms[i] = c->ms[i];
   return 0;
 }
 

@@ -1,7 +1,7 @@
-// tdsfs_diversity.cuh -- per-window Hudson FST, pi and dxy, and per-population Watterson's theta and Tajima's D
-// (DESIGN.md section 7).  Included by tdsfs.cu after tdsfs_kernels.cuh and tdsfs_fused.cuh.  No reference counterpart: the
-// reference's users get the FST column of their tables from pixy, and Tajima's D from scikit-allel, run separately over
-// the same VCF.
+// tdsfs_diversity.cuh -- per-window Hudson FST, pi and dxy, per-population Watterson's theta and Tajima's D, and Weir and
+// Cockerham's FST (DESIGN.md section 7).  Included by tdsfs.cu after tdsfs_kernels.cuh and tdsfs_fused.cuh.  No reference
+// counterpart: the reference's users get the FST column of their tables from pixy, and Tajima's D from scikit-allel, run
+// separately over the same VCF.
 //
 // Per SNP that passes the spectrum filters (snp_flags bit0) with n_i = ref_i + alt_i >= 2 in both populations, in fp64:
 //   pi_i = 2 ref_i alt_i / (n_i (n_i - 1)),   dxy = (ref_1 alt_2 + alt_1 ref_2) / (n_1 n_2)
@@ -15,7 +15,7 @@
 namespace tdsfs {
 
 constexpr int DIV_SEG = 1024;   // rows per segment (a multiple of 32)
-constexpr int DIV_WARPS = 8;    // warps per CTA of k_diversity and k_neutrality: one warp per segment
+constexpr int DIV_WARPS = 8;    // warps per CTA of k_diversity, k_neutrality and k_wcfst: one warp per segment
 
 // The segment list of a pass's candidate windows: window w owns segments [segoff[w], segoff[w + 1]), DIV_SEG rows each
 // counted from its first row (the last one shorter).
@@ -33,10 +33,12 @@ __global__ void __launch_bounds__(256) k_div_nseg(const int32_t* wlo, const int3
   else if (id == ncand) nseg[id] = 0;
 }
 
-// (ref1, alt1, ref2, alt2) of SNP s before the fix-ups: compile-time word counts (fully unrolled, every load of the row
-// issued together) or the runtime decode shared with k_window_hist (any width, and the counts entry)
+// (ref1, alt1, ref2, alt2) of SNP s before the fix-ups and its heterozygous calls (het1, het2): compile-time word counts
+// (fully unrolled, every load of the row issued together) or the runtime decode shared with k_window_hist (any width, and
+// the counts entry, whose het counts are 0).  A pass that does not read het1 / het2 compiles to the same code without them.
 template <int TW1, int TW2>
-__device__ __forceinline__ void div_counts(const KeyParams& p, long long s, int& ref1, int& alt1, int& ref2, int& alt2) {
+__device__ __forceinline__ void div_counts(const KeyParams& p, long long s, int& ref1, int& alt1, int& ref2, int& alt2,
+                                           int& het1, int& het2) {
   if constexpr (TW1 > 0 && TW2 > 0) {
     // every word of the row is loaded before any is counted: one memory round trip per row (count_pop_planes interleaves
     // loads and counting, and the compiler then issues the second population's loads only after the first one's arrive)
@@ -47,7 +49,8 @@ __device__ __forceinline__ void div_counts(const KeyParams& p, long long s, int&
     for (int i = 0; i < P1; ++i) { lo1[i] = __ldcs(row + (2 * i) * BLK); hi1[i] = __ldcs(row + (2 * i + 1) * BLK); }
 #pragma unroll
     for (int i = 0; i < P2; ++i) { lo2[i] = __ldcs(row + (TW1 + 2 * i) * BLK); hi2[i] = __ldcs(row + (TW1 + 2 * i + 1) * BLK); }
-    // codes 00, 01, 11, 10 = hom-ref, het, hom-alt, missing: alt = popc(lo) + popc(lo & hi), missing = popc(hi) - popc(lo & hi)
+    // codes 00, 01, 11, 10 = hom-ref, het, hom-alt, missing: alt = popc(lo) + popc(lo & hi), missing = popc(hi) - popc(lo & hi),
+    // het = popc(lo & ~hi) = popc(lo) - popc(lo & hi) = alt - 2 popc(lo & hi)
     uint32_t b1[P1], b2[P2];
 #pragma unroll
     for (int i = 0; i < P1; ++i) b1[i] = lo1[i] & hi1[i];
@@ -58,8 +61,10 @@ __device__ __forceinline__ void div_counts(const KeyParams& p, long long s, int&
     alt2 = (int)popc_sum<P2>(lo2) + c2;
     ref1 = 2 * (p.ns1 - ((int)popc_sum<P1>(hi1) - c1)) - alt1;
     ref2 = 2 * (p.ns2 - ((int)popc_sum<P2>(hi2) - c2)) - alt2;
+    het1 = alt1 - 2 * c1;
+    het2 = alt2 - 2 * c2;
   } else {
-    source_counts(p, s, ref1, alt1, ref2, alt2);
+    source_counts(p, s, ref1, alt1, ref2, alt2, het1, het2);
   }
 }
 
@@ -80,14 +85,17 @@ __device__ __forceinline__ bool segment_rows(const SegList& seg, long long g, lo
 // The NF fp sums of the segment [r0, r1), taken by one warp in the order that defines them (top of this file).  The warp
 // walks the ALIGNED 32-row blocks that overlap its segment, so word w of a step is exactly one 128-byte line (a window
 // starting inside a block would otherwise split every line of every step in two).  Lane l loads row s = b + l, and
-// row(s, ref1, alt1, ref2, alt2, t) sets that row's terms t[] and adds the pass's integer statistics to the lane's own
-// registers: integers, so the kernel reduces them over the warp at the end in any order.  The terms move to the lane that
-// owns row s in the definition, (s - r0) mod 32 = (l - r0) mod 32, which receives its rows in increasing order, one per
-// block, and a fixed xor tree combines the lanes: the sums are the definition's, bit for bit.
+// row(s, ref1, alt1, ref2, alt2, het1, het2, t) sets that row's terms t[] and adds the pass's integer statistics to the
+// lane's own registers: integers, so the kernel reduces them over the warp at the end in any order.  The terms move to
+// the lane that owns row s in the definition, (s - r0) mod 32 = (l - r0) mod 32, which receives its rows in increasing
+// order, one per block, and a fixed xor tree combines the lanes: the sums are the definition's, bit for bit.
 //
 // Every lane adds a term in every block, +0.0 for a row outside the segment or one that adds no term.  That leaves a sum
-// bitwise unchanged because no term is negative (each is a non-negative integer over a positive one): every sum starts at
-// +0.0, so none is ever -0.0, and x + (+0.0) is x bit for bit for any x but -0.0.  A term that can be negative breaks this.
+// bitwise unchanged as long as no term is -0.0: every sum starts at +0.0, and under round-to-nearest a sum of operands
+// none of which is -0.0 is never -0.0 (an exact zero sum of operands of opposite signs is +0.0), while x + (+0.0) is x bit
+// for bit for any x but -0.0.  Terms may be negative.  Each pass's terms are an integer numerator over a nonzero integer
+// denominator, converted and divided with round-to-nearest: a zero numerator gives +0.0 and a nonzero one a quotient far
+// above the underflow range, so no term is ever -0.0.
 template <int TW1, int TW2, int NF, typename Row>
 __device__ __forceinline__ void segment_sums(const KeyParams& k, long long r0, long long r1, double (&sum)[NF], Row row) {
   const int lane = threadIdx.x & 31;
@@ -100,9 +108,9 @@ __device__ __forceinline__ void segment_sums(const KeyParams& k, long long r0, l
 #pragma unroll
     for (int i = 0; i < NF; ++i) t[i] = 0.0;
     if (s >= r0 && s < r1) {
-      int ref1, alt1, ref2, alt2;
-      div_counts<TW1, TW2>(k, s, ref1, alt1, ref2, alt2);
-      row(s, ref1, alt1, ref2, alt2, t);
+      int ref1, alt1, ref2, alt2, het1, het2;
+      div_counts<TW1, TW2>(k, s, ref1, alt1, ref2, alt2, het1, het2);
+      row(s, ref1, alt1, ref2, alt2, het1, het2, t);
     }
 #pragma unroll
     for (int i = 0; i < NF; ++i) sum[i] += __shfl_sync(0xffffffffu, t[i], src);
@@ -141,7 +149,7 @@ __global__ void __launch_bounds__(DIV_WARPS * 32) k_diversity(const __grid_const
   if (!segment_rows(p.seg, g, r0, r1)) return;
   double sum[3];  // pi1, pi2, dxy
   int n_sites = 0, snp_count = 0;
-  segment_sums<TW1, TW2>(p.k, r0, r1, sum, [&](long long s, int ref1, int alt1, int ref2, int alt2, double (&t)[3]) {
+  segment_sums<TW1, TW2>(p.k, r0, r1, sum, [&](long long s, int ref1, int alt1, int ref2, int alt2, int, int, double (&t)[3]) {
     snp_count += p.k.flags ? (__ldg(p.k.flags + s) >> 1) & 1 : 1;
     const bool pass = row_filters(p.k, s, ref1, alt1, ref2, alt2);
     const long long n1 = ref1 + alt1, n2 = ref2 + alt2;
@@ -217,7 +225,7 @@ __global__ void __launch_bounds__(DIV_WARPS * 32) k_neutrality(const __grid_cons
   if (!segment_rows(p.seg, g, r0, r1)) return;
   double sum[2];  // theta_pi1, theta_pi2
   int S1 = 0, S2 = 0, nmax1 = 0, nmax2 = 0, snp_count = 0;
-  segment_sums<TW1, TW2>(p.k, r0, r1, sum, [&](long long s, int ref1, int alt1, int ref2, int alt2, double (&t)[2]) {
+  segment_sums<TW1, TW2>(p.k, r0, r1, sum, [&](long long s, int ref1, int alt1, int ref2, int alt2, int, int, double (&t)[2]) {
     snp_count += p.k.flags ? (__ldg(p.k.flags + s) >> 1) & 1 : 1;
     if (row_filters(p.k, s, ref1, alt1, ref2, alt2)) {
       const long long n1 = ref1 + alt1, n2 = ref2 + alt2;
@@ -276,6 +284,89 @@ __global__ void __launch_bounds__(256) k_neut_finish(const __grid_constant__ Neu
   p.theta_pi1[id] = pi1; p.theta_pi2[id] = pi2;
   p.theta_w1[id] = tw1; p.theta_w2[id] = tw2;
   p.tajd1[id] = d1; p.tajd2[id] = d2;
+  p.flags[id] = __ldg(p.seg.whi + id) == __ldg(p.seg.wlo + id) ? TDSFS_F_EMPTY : 0;
+}
+
+// ------------------------------------------------------------------------------------------------ Weir and Cockerham's FST
+// Per row that passes the spectrum filter (snp_flags bit0, read directly: no fix-up is applied, so the calls held as
+// fix-ups count as missing), from the 2-bit codes of population i: n_i called diploids, x_i their alt alleles, h_i their
+// heterozygotes; N = n1 + n2, X = x1 + x2, H = h1 + h2, D = x1 n2 - x2 n1.  The variance components summed over both
+// alleles (scikit-allel's weir_cockerham_fst with r = 2), each an exact int64 numerator over an exact int64 denominator
+// with one rounded division:
+//   a = [D^2 (N-1) - n1 n2 (X(2N-X) - N H)] / [4 n1^2 n2^2 (N-2)]   rows with n1 >= 1, n2 >= 1 and N >= 3 (n_sites)
+//   b = [n1 n2 (X(2N-X) - 2(N-1) H) - D^2] / [2 n1 n2 N (N-2)]      the same rows
+//   c = H / N                                                     rows with N >= 1
+// Every numerator and denominator stays below 2^63 while ns1, ns2 <= WC_MAX_SAMPLES (the largest, 4 n1^2 n2^2 (N-1) and
+// 4 n1^2 n2^2 (N-2), are about 8.19e18 at 4000 + 4000).  The window sums run in the order of the FST pass, and
+// fst = a / ((a + b) + c), NaN when that denominator is 0.
+constexpr int WC_MAX_SAMPLES = 4000;
+
+struct WcPart {  // sums of one segment
+  double a, b, c;
+  int n_sites, snp_count;
+};
+
+struct WcParams {
+  KeyParams k;                 // genotype rows, sample columns, snp_flags
+  SegList seg;
+  WcPart* part;                // [segments]
+  int32_t* snp_count;          // [ncand] outputs
+  int32_t* n_sites;
+  double* a;
+  double* b;
+  double* c;
+  double* fst;
+  uint8_t* flags;
+};
+
+// One warp per segment: its a, b and c sums, rows that entered a and b, and SNPs counted.
+template <int TW1, int TW2>
+__global__ void __launch_bounds__(DIV_WARPS * 32) k_wcfst(const __grid_constant__ WcParams p) {
+  const long long g = (long long)blockIdx.x * DIV_WARPS + (threadIdx.x >> 5);
+  long long r0, r1;
+  if (!segment_rows(p.seg, g, r0, r1)) return;
+  double sum[3];  // a, b, c
+  int n_sites = 0, snp_count = 0;
+  segment_sums<TW1, TW2>(p.k, r0, r1, sum, [&](long long s, int ref1, int alt1, int ref2, int alt2, int het1, int het2,
+                                               double (&t)[3]) {
+    const int f = p.k.flags ? __ldg(p.k.flags + s) : 3;
+    snp_count += (f >> 1) & 1;
+    const int n1 = (ref1 + alt1) >> 1, n2 = (ref2 + alt2) >> 1, N = n1 + n2;  // ref + alt = 2 (ns - missing)
+    if (!(f & 1) || N < 1) return;
+    const int X = alt1 + alt2, H = het1 + het2;
+    t[2] = (double)H / (double)N;
+    if (n1 < 1 || n2 < 1 || N < 3) return;
+    // With ns1, ns2 <= WC_MAX_SAMPLES every factor fits in 32 bits (|D| <= 2 n1 n2, X(2N-X) <= N^2, 2(N-1)H < 2N^2), so
+    // each product is one 32 x 32 -> 64-bit multiply, and at most one more by a 32-bit factor
+    const int D = alt1 * n2 - alt2 * n1, n12 = n1 * n2, Q = X * (2 * N - X);
+    const long long D2 = (long long)D * D;
+    t[0] = (double)(D2 * (N - 1) - (long long)n12 * (Q - N * H)) / (double)((long long)n12 * n12 * (4 * (N - 2)));
+    t[1] = (double)((long long)n12 * (Q - 2 * (N - 1) * H) - D2) / (double)((long long)n12 * N * (2 * (N - 2)));
+    ++n_sites;
+  });
+  n_sites = __reduce_add_sync(0xffffffffu, n_sites);
+  snp_count = __reduce_add_sync(0xffffffffu, snp_count);
+  if ((threadIdx.x & 31) == 0) p.part[g] = WcPart{sum[0], sum[1], sum[2], n_sites, snp_count};
+}
+
+// One thread per window: its segment sums in segment order, then fst = a / ((a + b) + c) (NaN when that is 0).
+__global__ void __launch_bounds__(256) k_wc_finish(const __grid_constant__ WcParams p) {
+  const long long id = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (id >= p.seg.ncand) return;
+  double a = 0.0, b = 0.0, c = 0.0;
+  int n_sites = 0, snp_count = 0;
+  for (long long g = __ldg(p.seg.segoff + id), e = __ldg(p.seg.segoff + id + 1); g < e; ++g) {
+    const WcPart q = p.part[g];
+    a += q.a; b += q.b; c += q.c;
+    n_sites += q.n_sites; snp_count += q.snp_count;
+  }
+  const double den = (a + b) + c;
+  p.snp_count[id] = snp_count;
+  p.n_sites[id] = n_sites;
+  p.a[id] = a;
+  p.b[id] = b;
+  p.c[id] = c;
+  p.fst[id] = den == 0.0 ? __longlong_as_double(0x7FF8000000000000LL) : a / den;
   p.flags[id] = __ldg(p.seg.whi + id) == __ldg(p.seg.wlo + id) ? TDSFS_F_EMPTY : 0;
 }
 

@@ -1229,21 +1229,25 @@ __global__ void __launch_bounds__(LARGE_THREADS) k3_score_large(const __grid_con
   score_large_windows(p, blockIdx.x, gridDim.x);
 }
 
-// (ref1, alt1, ref2, alt2) of SNP s before the fix-ups, from the source rows: the counts entry or the B32 genotype matrix
-// with runtime word counts
-__device__ __forceinline__ void source_counts(const KeyParams& p, long long s, int& ref1, int& alt1, int& ref2, int& alt2) {
+// (ref1, alt1, ref2, alt2) of SNP s before the fix-ups, and the heterozygous calls het1, het2 (0 for the counts entry),
+// from the source rows: the counts entry or the B32 genotype matrix with runtime word counts
+__device__ __forceinline__ void source_counts(const KeyParams& p, long long s, int& ref1, int& alt1, int& ref2, int& alt2,
+                                              int& het1, int& het2) {
   if (p.cnt) {
     const uint2 v = __ldg(reinterpret_cast<const uint2*>(p.cnt) + s);
     ref1 = v.x & 0xFFFF; alt1 = v.x >> 16; ref2 = v.y & 0xFFFF; alt2 = v.y >> 16;
+    het1 = het2 = 0;
     return;
   }
   const int RW = p.W1 + p.W2;
   const uint32_t* row = p.G + ((s >> 5) * RW) * BLK + (s & 31);
   int T[2] = {0, 0}, M[2] = {0, 0};
+  het1 = het2 = 0;  // scalars, not a third indexed array: a caller that ignores them compiles to the same code without them
   for (int w = 0; w < RW; w += 2) {  // (lo plane, hi plane) of 32 samples; W1 and W2 are even
     const uint32_t l = row[(long long)w * BLK], h = row[(long long)(w + 1) * BLK];
     T[w >= p.W1] += __popc(l) + __popc(h);
     M[w >= p.W1] += __popc(h & ~l);
+    (w >= p.W1 ? het2 : het1) += __popc(l & ~h);
   }
   alt1 = T[0] - M[0]; alt2 = T[1] - M[1];
   ref1 = 2 * (p.ns1 - M[0]) - alt1; ref2 = 2 * (p.ns2 - M[1]) - alt2;
@@ -1255,8 +1259,8 @@ __global__ void k_window_hist(const __grid_constant__ KeyParams p, int lo, int h
   for (long long s = lo + blockIdx.x * blockDim.x + threadIdx.x; s < hi; s += gridDim.x * blockDim.x) {
     const uint32_t k = load_rec(p.rec, p.fmt, s, p.n1, p.n2, p.C2).x;
     if (k) atomicAdd(h2 + k, 1u);
-    int ref1, alt1, ref2, alt2;
-    source_counts(p, s, ref1, alt1, ref2, alt2);
+    int ref1, alt1, ref2, alt2, het1, het2;
+    source_counts(p, s, ref1, alt1, ref2, alt2, het1, het2);
     if (row_filters(p, s, ref1, alt1, ref2, alt2)) {
       if (alt1 > 0 && alt1 < p.R1) atomicAdd(h1a + alt1, 1u);
       if (alt2 > 0 && alt2 < p.R2) atomicAdd(h1b + alt2, 1u);

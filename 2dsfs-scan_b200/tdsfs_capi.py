@@ -24,12 +24,13 @@ EXPORTS = [
     "tdsfs_synth_genotypes", "tdsfs_timings", "tdsfs_launch_count", "tdsfs_scan_info", "tdsfs_tail_stamps", "tdsfs_version",
     "tdsfs_diversity_bp", "tdsfs_diversity_snp", "tdsfs_fetch_diversity",
     "tdsfs_neutrality_bp", "tdsfs_neutrality_snp", "tdsfs_fetch_neutrality",
+    "tdsfs_wcfst_bp", "tdsfs_wcfst_snp", "tdsfs_fetch_wcfst",
 ]
 
 
 PEER_BLOB_BYTES = 192  # TDSFS_PEER_BLOB_BYTES
 TIMING_NAMES = ("k1_count", "finalize", "k2_bounds", "k3_small", "k3_large", "background_call", "scan_call", "pass_total",
-                "exchange", "diversity", "neutrality")  # the slots of tdsfs_timings
+                "exchange", "diversity", "neutrality", "wcfst")  # the slots of tdsfs_timings
 
 
 class TdsfsError(RuntimeError):
@@ -45,8 +46,8 @@ class Fixup(C.Structure):
 FIXUP_DTYPE = np.dtype([("snp", "<i8"), ("pop", "<i4"), ("dref", "<i4"), ("dalt", "<i4")], align=True)
 
 
-# Per-window result columns in the member order of tdsfs_result_t, tdsfs_diversity_t and tdsfs_neutrality_t: each of
-# those structs holds one host pointer per column.
+# Per-window result columns in the member order of tdsfs_result_t, tdsfs_diversity_t, tdsfs_neutrality_t and
+# tdsfs_wcfst_t: each of those structs holds one host pointer per column.
 RESULT_DTYPES = dict(chrom=np.int32, start=np.int64, end=np.int64, snp_count=np.int32, n2d=np.int32, n1d_p1=np.int32,
                      n1d_p2=np.int32, T2D=np.float64, T1D_p1=np.float64, T1D_p2=np.float64, flags=np.uint8)
 DIVERSITY_DTYPES = dict(chrom=np.int32, start=np.int64, end=np.int64, snp_count=np.int32, flags=np.uint8, n_sites=np.int32,
@@ -55,6 +56,8 @@ NEUTRALITY_DTYPES = dict(chrom=np.int32, start=np.int64, end=np.int64, snp_count
                          n_seg_p2=np.int32, n_max_p1=np.int32, n_max_p2=np.int32, theta_pi_p1=np.float64,
                          theta_pi_p2=np.float64, theta_w_p1=np.float64, theta_w_p2=np.float64, tajima_d_p1=np.float64,
                          tajima_d_p2=np.float64)
+WCFST_DTYPES = dict(chrom=np.int32, start=np.int64, end=np.int64, snp_count=np.int32, flags=np.uint8, n_sites=np.int32,
+                    a=np.float64, b=np.float64, c=np.float64, fst=np.float64)
 
 
 class Result(C.Structure):
@@ -67,6 +70,10 @@ class Diversity(C.Structure):
 
 class Neutrality(C.Structure):
     _fields_ = [(k, C.c_void_p) for k in NEUTRALITY_DTYPES]
+
+
+class WcFst(C.Structure):
+    _fields_ = [(k, C.c_void_p) for k in WCFST_DTYPES]
 
 
 _lib = None
@@ -260,6 +267,10 @@ class Handle:
     def _alloc_neutrality(n):
         return Handle._alloc(NEUTRALITY_DTYPES, Neutrality, n)
 
+    @staticmethod
+    def _alloc_wcfst(n):
+        return Handle._alloc(WCFST_DTYPES, WcFst, n)
+
     def _into(self, alloc, cap, f, *args):
         """f(handle, *args, out, cap, &n) into the arrays alloc(cap) allocates: dict of their first n entries."""
         arrs, r = alloc(cap)
@@ -301,6 +312,18 @@ class Handle:
 
     def fetch_neutrality(self, cap):
         return self._into(self._alloc_neutrality, cap, self._L.tdsfs_fetch_neutrality)
+
+    def wcfst(self, size, snp_mode=False, fetch=True):
+        """Per-window Weir and Cockerham (1984) FST over the candidate windows of (size, mode), in scan order
+        (tdsfs_wcfst_*), from the genotype calls: a / b / c are the summed variance components (scikit-allel's
+        weir_cockerham_fst summed over both alleles), n_sites the rows that entered a and b, fst = a / (a + b + c), NaN
+        when that is 0.  Calls held as fix-ups count as missing.  Needs load_genotypes with at most 4000 samples per
+        population.  Returns a dict of arrays (chrom / start / end / snp_count / flags as the scan's), or the candidate
+        count when fetch=False (results stay on the device: fetch_wcfst)."""
+        return self._run("wcfst", self._alloc_wcfst, size, snp_mode, fetch)
+
+    def fetch_wcfst(self, cap):
+        return self._into(self._alloc_wcfst, cap, self._L.tdsfs_fetch_wcfst)
 
     def fetch_results(self, cap):
         return self._into(self._alloc_result, cap, self._L.tdsfs_fetch_results)
@@ -358,6 +381,10 @@ class Handle:
     def neutrality_ms(self):
         """CUDA-event time (ms) of the segment + finish kernels of the last neutrality call (tdsfs_timings slot 10)."""
         return self.timings()["neutrality"]
+
+    def wcfst_ms(self):
+        """CUDA-event time (ms) of the segment + finish kernels of the last wcfst call (tdsfs_timings slot 11)."""
+        return self.timings()["wcfst"]
 
     def launch_count(self):
         return int(self._L.tdsfs_launch_count(self._h))

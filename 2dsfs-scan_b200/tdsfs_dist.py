@@ -310,3 +310,11 @@ def sharded_neutrality(handle, pieces, pos, size, device, *, snp_mode=False, gro
     (identical on every rank)."""
     res = handle.neutrality(size, snp_mode=snp_mode)
     return gather_results(localize_results(res, pieces, pos, size, snp_mode), 0, group)
+
+
+def sharded_wcfst(handle, pieces, pos, size, device, *, snp_mode=False, group=None):
+    """Per-window Weir and Cockerham FST of a sharded panel (genotype entry): the counterpart of sharded_diversity, with
+    the same calling convention.  Every result of a window depends on its own rows only, so the gathered arrays equal a
+    single-handle run bit for bit.  Returns the gathered arrays (identical on every rank)."""
+    res = handle.wcfst(size, snp_mode=snp_mode)
+    return gather_results(localize_results(res, pieces, pos, size, snp_mode), 0, group)

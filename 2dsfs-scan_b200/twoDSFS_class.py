@@ -480,22 +480,22 @@ class LikelihoodInference_jointSFS:
         keys, counts, stats, _, _ = self._scan(table, snp_window_size, True, bg_mode=T.BG_PER_CHROM)
         return self._unguarded(keys, counts, stats, with_diff=True, snp_count_fixed=snp_window_size)
 
-    # ------------------------------------------------------------------ diversity and neutrality (not in the reference)
-    def _window_pass(self, data_dict, size, snp_mode, neutrality):
-        """Keys and result columns (lists) of the non-empty windows of (size, mode) from the diversity or the neutrality
-        pass over data_dict."""
+    # ------------------------------------------------------------------ diversity, neutrality, WC FST (not in the reference)
+    def _window_pass(self, data_dict, size, snp_mode, entry):
+        """Keys and result columns (lists) of the non-empty windows of (size, mode) from the per-window pass `entry`
+        (Handle.diversity, .neutrality or .wcfst) over data_dict."""
         table = self._table(data_dict)
         if table.n == 0:
             return [], {}
         self._int_filters()
         eng = self._eng()
         eng.load(table, self.pop1_size, self.pop2_size, self.fold, self._flags(table))
-        res = (eng.h.neutrality if neutrality else eng.h.diversity)(size, snp_mode=snp_mode)
+        res = getattr(eng.h, entry)(size, snp_mode=snp_mode)
         live = (res["flags"] & T.F_EMPTY) == 0
         return window_keys(table, res, live), {k: v[live].tolist() for k, v in res.items()}
 
     def _fst(self, data_dict, size, snp_mode):
-        keys, res = self._window_pass(data_dict, size, snp_mode, False)
+        keys, res = self._window_pass(data_dict, size, snp_mode, "diversity")
         if not keys:
             return {}
         cols = [res[k] for k in ("snp_count", "n_sites", "pi_p1", "pi_p2", "dxy", "fst")]
@@ -529,7 +529,7 @@ class LikelihoodInference_jointSFS:
                         TajimaD_pop2="tajima_d_p2")
 
     def _tajima(self, data_dict, size, snp_mode):
-        keys, res = self._window_pass(data_dict, size, snp_mode, True)
+        keys, res = self._window_pass(data_dict, size, snp_mode, "neutrality")
         if not keys:
             return {}
         cols = [res[c] for c in self._TAJIMA_COLS.values()]
@@ -554,6 +554,34 @@ class LikelihoodInference_jointSFS:
         self.data_dict = data_dict
         self.snp_window_size = snp_window_size
         return self._tajima(data_dict, snp_window_size, True)
+
+    def _wc_fst(self, panel, size, snp_mode):
+        if not isinstance(panel, PackedPanel):
+            raise TypeError("Weir and Cockerham FST needs the genotype calls: pass the PackedPanel of make_packed_panel "
+                            "(a data_dict holds allele counts only, without heterozygotes)")
+        keys, res = self._window_pass(panel, size, snp_mode, "wcfst")
+        if not keys:
+            return {}
+        cols = [res[k] for k in ("snp_count", "n_sites", "a", "b", "c", "fst")]
+        return {k: {"snp_count": c, "n_sites": n, "a": a, "b": b, "c": cc, "FST": None if f != f else f}
+                for k, c, n, a, b, cc, f in zip(keys, *cols)}
+
+    def wc_fst_scan(self, panel, window_size):
+        """Weir and Cockerham's (1984) FST of every non-empty fixed-bp window, computed on the GPU from the genotype calls
+        of a make_packed_panel panel: {"{chrom} {start}-{end}": {"snp_count", "n_sites", "a", "b", "c", "FST"}}, keyed like
+        fst_scan.  a, b and c are the window's sums of scikit-allel's per-SNP variance components (weir_cockerham_fst,
+        summed over both alleles) over the SNPs that pass the constructor's filters, and FST = a / (a + b + c), None when
+        that is 0: scikit-allel's windowed_weir_cockerham_fst, the estimator of pixy's default FST column.  n_sites counts
+        the SNPs with a called diploid in both populations and at least three in all, the ones that enter a and b.  Calls
+        the packer holds as fix-ups (half calls, haploid and multi-allelic calls) count as missing.  At most 4000 samples
+        per population.  Not in the reference; pass the result to save_csv_stats(fst=...)."""
+        self.window_size = window_size
+        return self._wc_fst(panel, window_size, False)
+
+    def wc_fst_scan_bySNPs(self, panel, snp_window_size):
+        """wc_fst_scan over fixed-SNP windows, with the windows and keys of fst_scan_bySNPs."""
+        self.snp_window_size = snp_window_size
+        return self._wc_fst(panel, snp_window_size, True)
 
     # ------------------------------------------------------------------ simulations
     def get_gens(self, main_dir):
@@ -643,9 +671,10 @@ col_names = ['chromosome', 'window_start', 'window_end', 'snp_count', 'T2D', 'T1
 
 def save_csv_stats(stats_dict, output, fst=None, tajima=None):
     """reference :1884-1907: same columns, chromosome mapped through chr_ids, None written as ''.  fst (not in the
-    reference): the dict of fst_scan / fst_scan_bySNPs over the same windows adds a trailing FST column, the layout of the
-    ECB tables the reference's R post-processing writes; '' where FST is None or the window has no entry.  tajima (not in
-    the reference): the dict of tajima_scan / tajima_scan_bySNPs adds TajimaD_p1, TajimaD_p2 after it, '' likewise."""
+    reference): the dict of fst_scan / fst_scan_bySNPs or wc_fst_scan / wc_fst_scan_bySNPs over the same windows adds a
+    trailing FST column, the layout of the ECB tables the reference's R post-processing writes; '' where FST is None or
+    the window has no entry.  tajima (not in the reference): the dict of tajima_scan / tajima_scan_bySNPs adds TajimaD_p1,
+    TajimaD_p2 after it, '' likewise."""
     with open(output, 'w', newline='') as csvfile:
         writer = csv.DictWriter(csvfile, fieldnames=col_names + (['FST'] if fst is not None else [])
                                 + (['TajimaD_p1', 'TajimaD_p2'] if tajima is not None else []))

@@ -280,6 +280,40 @@ int tdsfs_neutrality_bp(tdsfs_t* ctx, int64_t W, tdsfs_neutrality_t* out, int64_
 int tdsfs_neutrality_snp(tdsfs_t* ctx, int64_t N, tdsfs_neutrality_t* out, int64_t cap, int64_t* n_windows);
 int tdsfs_fetch_neutrality(tdsfs_t* ctx, tdsfs_neutrality_t* out, int64_t cap, int64_t* n_windows);
 
+/* ---- per-window Weir and Cockerham (1984) FST from the genotype calls (no reference counterpart; DESIGN.md 7) -------
+ * Same windows, order and spectrum filter as tdsfs_diversity_*, for data loaded with tdsfs_load_genotypes only: the counts
+ * entry has no heterozygote counts (TDSFS_ERR_STATE).  Per row, counts come from the 2-bit codes alone: calls held as
+ * fix-ups (half calls, haploid calls, multi-allelic digits) count as missing.  For population i, n_i = called diploids
+ * (ns_i - #missing), x_i = their alt alleles, h_i = their heterozygotes (code 1); N = n1 + n2, X = x1 + x2, H = h1 + h2,
+ * D = x1 n2 - x2 n1.  The variance components summed over both alleles, each an exact int64 numerator over an exact int64
+ * denominator, converted to fp64 and divided once (round to nearest):
+ *   a = [D^2 (N-1) - n1 n2 (X(2N-X) - N H)] / [4 n1^2 n2^2 (N-2)]
+ *   b = [n1 n2 (X(2N-X) - 2(N-1) H) - D^2] / [2 n1 n2 N (N-2)]
+ *   c = H / N
+ * a and b enter a window's sums for the rows that pass the filter (snp_flags bit0, read directly: no fix-up is applied)
+ * with n1 >= 1, n2 >= 1 and N >= 3 (n_sites counts these rows); c for every row that passes the filter with N >= 1.
+ * This is scikit-allel's weir_cockerham_fst (r = 2) summed over both alleles, with windowed_weir_cockerham_fst's nansum:
+ * it gives NaN for a and b exactly on the rows left out here.  fst = a / ((a + b) + c), NaN when that denominator is 0;
+ * it can be negative.  The sums run in the order of tdsfs_diversity_*, so results are bitwise equal for any sharding that
+ * keeps windows whole.  Panels with more than 4000 samples in a population (the int64 terms would overflow) give
+ * TDSFS_ERR_ARG.  Own window arrays and results, as tdsfs_diversity_*.
+ * out == NULL: enqueue only (honours tdsfs_set_sync(0)); tdsfs_fetch_wcfst copies the results later. */
+typedef struct {            /* caller-owned host SoA, capacity >= tdsfs_candidates_bp / _snp; any member may be NULL */
+  int32_t* chrom;           /* as tdsfs_result_t */
+  int64_t* start;
+  int64_t* end;
+  int32_t* snp_count;       /* count_snps, as tdsfs_result_t */
+  uint8_t* flags;           /* TDSFS_F_EMPTY */
+  int32_t* n_sites;         /* rows that entered the a and b sums */
+  double* a;                /* sum of a: variance between populations */
+  double* b;                /* sum of b: between individuals within populations */
+  double* c;                /* sum of c: between gametes within individuals */
+  double* fst;              /* a / ((a + b) + c), NaN when that is 0 */
+} tdsfs_wcfst_t;
+int tdsfs_wcfst_bp(tdsfs_t* ctx, int64_t W, tdsfs_wcfst_t* out, int64_t cap, int64_t* n_windows);
+int tdsfs_wcfst_snp(tdsfs_t* ctx, int64_t N, tdsfs_wcfst_t* out, int64_t cap, int64_t* n_windows);
+int tdsfs_fetch_wcfst(tdsfs_t* ctx, tdsfs_wcfst_t* out, int64_t cap, int64_t* n_windows);
+
 /* ---- likelihood of explicit spectra ------------------------------------------------------------------------
  * calculate_likelihood_1D / _2D (:478-537, :625-684) on already-interior vectors: x[n] integer counts,
  * b[n] background values, B = sum of b as the caller's language sums it.  *flag = 1 when the reference returns
@@ -299,7 +333,8 @@ int tdsfs_synth_genotypes(tdsfs_t* ctx, void* G_dev, int64_t S, int64_t snp0, in
  * [0]=count kernel (K1), [1]=finalize, [2]=boundaries (K2), [3]=score small windows (K3/K4), [4]=score large windows,
  * [5]=background call, [6]=scan call, [7]=K1 start -> last score kernel end, [8]=peer exchange kernel (n >= 9),
  * [9]=segment + finish kernels of the last tdsfs_diversity_* call (n >= 10),
- * [10]=segment + finish kernels of the last tdsfs_neutrality_* call (n >= 11). */
+ * [10]=segment + finish kernels of the last tdsfs_neutrality_* call (n >= 11),
+ * [11]=segment + finish kernels of the last tdsfs_wcfst_* call (n >= 12). */
 int tdsfs_timings(tdsfs_t* ctx, float* ms, int32_t n);
 int64_t tdsfs_launch_count(tdsfs_t* ctx); /* kernels launched by this handle so far */
 /* Which path scored the last scan: *fused = 1 when the fused pair ran (tdsfs_plan_* before tdsfs_background on the

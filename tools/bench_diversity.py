@@ -1,7 +1,7 @@
 #!/usr/bin/env python
-"""Time the per-window diversity pass (Hudson FST, pi, dxy: tdsfs_diversity_bp) and the neutrality pass (Watterson's theta,
-Tajima's D: tdsfs_neutrality_bp) on bench.py's config 5 and config 4 panels, built in HBM by the same device generator, over
-the same 20 kb windows.
+"""Time the per-window diversity pass (Hudson FST, pi, dxy: tdsfs_diversity_bp), the neutrality pass (Watterson's theta,
+Tajima's D: tdsfs_neutrality_bp) and the Weir and Cockerham FST pass (tdsfs_wcfst_bp) on bench.py's config 5 and config 4
+panels, built in HBM by the same device generator, over the same 20 kb windows.
 
   python tools/bench_diversity.py [--calls 30] [--warmup 5] [--out DIR]
 
@@ -14,7 +14,8 @@ Per workload it reports
   * copy_gbs: a device-to-device copy of the same genotype matrix timed in the same process, read + write bytes over time;
   * the card's name and power limit, read in the same process;
   * the same call / kernel times, GB/s and fractions for the neutrality pass under neutrality_* keys (same panel, same
-    windows, same algorithmic bytes), and neutrality_over_fst_kernel, the ratio of the two kernel medians.
+    windows, same algorithmic bytes), and neutrality_over_fst_kernel, the ratio of the two kernel medians;
+  * the same again for the Weir and Cockerham FST pass under wcfst_* keys, with wcfst_over_fst_kernel.
 One JSON line per workload on stdout; with --out, also DIR/bench_diversity.json.
 """
 import argparse
@@ -47,6 +48,27 @@ def card():
     except Exception:  # noqa: BLE001
         import torch
         return torch.cuda.get_device_name(0), "unknown"
+
+
+def time_pass(entry, W, args, h, torch, stream):
+    """(kernel times of synchronous calls, call time of back-to-back asynchronous calls, fetched results) of the pass
+    Handle.<entry>, timed as the FST pass is."""
+    run, ms = getattr(h, entry), getattr(h, entry + "_ms")
+    for _ in range(args.warmup):
+        run(W, fetch=False)
+    kernel = []
+    for _ in range(args.calls):
+        run(W, fetch=False)
+        kernel.append(ms())
+    h.set_sync(False)
+    ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    ev0.record(stream)
+    for _ in range(args.calls):
+        run(W, fetch=False)
+    ev1.record(stream)
+    torch.cuda.synchronize()
+    h.set_sync(True)
+    return kernel, ev0.elapsed_time(ev1) / args.calls, getattr(h, "fetch_" + entry)(h.candidates(W))
 
 
 def measure(name, cfg, args, h, T, torch, stream):
@@ -82,22 +104,9 @@ def measure(name, cfg, args, h, T, torch, stream):
     h.set_sync(True)
     res = h.fetch_diversity(h.candidates(W))
 
-    # the neutrality pass over the same windows, timed the same way
-    for _ in range(args.warmup):
-        h.neutrality(W, fetch=False)
-    nkernel = []
-    for _ in range(args.calls):
-        h.neutrality(W, fetch=False)
-        nkernel.append(h.neutrality_ms())
-    h.set_sync(False)
-    ev0.record(stream)
-    for _ in range(args.calls):
-        h.neutrality(W, fetch=False)
-    ev1.record(stream)
-    torch.cuda.synchronize()
-    ncall_ms = ev0.elapsed_time(ev1) / args.calls
-    h.set_sync(True)
-    nres = h.fetch_neutrality(h.candidates(W))
+    # the neutrality and the Weir and Cockerham FST passes over the same windows, timed the same way
+    nkernel, ncall_ms, nres = time_pass("neutrality", W, args, h, torch, stream)
+    wkernel, wcall_ms, wres = time_pass("wcfst", W, args, h, torch, stream)
 
     # same-process reference: device-to-device copy of the genotype matrix
     dst = torch.empty_like(G)
@@ -134,7 +143,17 @@ def measure(name, cfg, args, h, T, torch, stream):
                                       "windows_with_tajima_d_p1": int(np.isfinite(nres["tajima_d_p1"][nlive]).sum()),
                                       "mean_tajima_d_p1": float(np.nanmean(nres["tajima_d_p1"][nlive])),
                                       "mean_tajima_d_p2": float(np.nanmean(nres["tajima_d_p2"][nlive]))}})
-    for k in ("kernel", "call", "neutrality_kernel", "neutrality_call"):
+    wk_ms = float(np.median(wkernel))
+    wlive = (wres["flags"] & T.F_EMPTY) == 0
+    out.update({"wcfst_call_ms": wcall_ms, "wcfst_kernel_ms_median": wk_ms,
+                "wcfst_kernel_ms_min": float(np.min(wkernel)), "wcfst_kernel_ms_max": float(np.max(wkernel)),
+                "wcfst_kernel_gbs": algo / (wk_ms * 1e-3) / 1e9, "wcfst_call_gbs": algo / (wcall_ms * 1e-3) / 1e9,
+                "wcfst_over_fst_kernel": wk_ms / k_ms,
+                "wcfst_checks": {"snp_count_sum_equals_S": bool(int(wres["snp_count"].sum()) == S),
+                                 "n_sites": int(wres["n_sites"].sum()),
+                                 "windows_with_fst": int(np.isfinite(wres["fst"][wlive]).sum()),
+                                 "mean_fst": float(np.nanmean(wres["fst"][wlive]))}})
+    for k in ("kernel", "call", "neutrality_kernel", "neutrality_call", "wcfst_kernel", "wcfst_call"):
         out[k + "_frac_of_copy_peak"] = out[k + "_gbs"] / COPY_PEAK_GBS
         out[k + "_frac_of_sheet"] = out[k + "_gbs"] / SHEET_GBS
     del G, pos_dev
