@@ -25,7 +25,7 @@ def _newer(target, sources):
 def build(force=False, verbose=False):
     os.makedirs(os.path.dirname(LIB), exist_ok=True)
     cuda_src = [os.path.join(SRC, "tdsfs.cu"), os.path.join(SRC, "tdsfs_kernels.cuh"), os.path.join(SRC, "tdsfs_fused.cuh"),
-                os.path.join(SRC, "tdsfs_diversity.cuh"),
+                os.path.join(SRC, "tdsfs_diversity.cuh"), os.path.join(SRC, "tdsfs_ld.cuh"),
                 os.path.join(HERE, "..", "include", "tdsfs.h")]
     if force or _newer(LIB, cuda_src):
         nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")

@@ -15,10 +15,11 @@
 #include "tdsfs_kernels.cuh"
 #include "tdsfs_fused.cuh"
 #include "tdsfs_diversity.cuh"
+#include "tdsfs_ld.cuh"
 
 using namespace tdsfs;
 
-#define TDSFS_VERSION 203
+#define TDSFS_VERSION 204
 
 static thread_local std::string g_err;
 
@@ -217,9 +218,18 @@ struct tdsfs_ctx {
   double* d_neut_tab = nullptr;       // a1(n) for n in [0, neut_tab_n], then a2(n) for the same n
   long long neut_tab_n = -1;
   long long n_allele_max = 0;         // the largest n_i = ref_i + alt_i a row of the loaded data can reach
+  // LD pruning (tdsfs_ld_prune): a workspace of its own, so that a pending plan, the scan's results, the step graph and the
+  // window passes' results survive it
+  uint32_t* d_ld_mask = nullptr;      // [S * mask words] pair bits of k_ld_pairs
+  long long ld_mask_cap = 0;
+  uint8_t* d_ld_keep = nullptr;       // [S]
+  long long ld_keep_cap = 0;
+  unsigned long long* d_ld_n = nullptr;  // kept rows
+  cudaEvent_t ev_ld[3] = {};          // before k_ld_pairs, between the kernels, after k_ld_resolve (tdsfs_timings)
+  bool ld_timed = false;
   // instrumentation
   cudaEvent_t ev[NEV] = {};
-  float ms[12] = {};
+  float ms[14] = {};
   long long launches = 0;
 };
 
@@ -292,6 +302,8 @@ extern "C" int tdsfs_create(int device, tdsfs_t** out) {
     CK(cudaEventCreate(&w->ev0));
     CK(cudaEventCreate(&w->ev1));
   }
+  for (cudaEvent_t& e : c->ev_ld) CK(cudaEventCreate(&e));
+  CKR(dev_alloc(&c->d_ld_n, 1));
   CKR(dev_alloc(&c->d_err, 1));
   CKR(dev_alloc(&c->d_nlarge, 1));
   CKR(dev_alloc(&c->d_lnI, LN_TABLE));
@@ -400,6 +412,8 @@ extern "C" void tdsfs_destroy(tdsfs_t* c) {
   free_window_pass(c->neut);
   free_window_pass(c->wc);
   dev_free(c->d_neut_tab);
+  dev_free(c->d_ld_mask); dev_free(c->d_ld_keep); dev_free(c->d_ld_n);
+  for (cudaEvent_t e : c->ev_ld) if (e) cudaEventDestroy(e);
   cudaStreamDestroy(c->own_stream);
   cudaStreamDestroy(c->copy_stream);
   cudaStreamDestroy(c->plan_stream);
@@ -1742,6 +1756,64 @@ extern "C" int tdsfs_wcfst_snp(tdsfs_t* c, int64_t N, tdsfs_wcfst_t* out, int64_
   return wcfst(c, N, true, out, cap, n_windows);
 }
 
+// ------------------------------------------------------------------------------------------------ LD pruning
+// k_ld_pairs (the pair bits of every row) -> k_ld_resolve (the greedy decision per chromosome), then the keep bytes and the
+// kept count to the host.  Synchronous.
+extern "C" int tdsfs_ld_prune(tdsfs_t* c, int32_t size, int32_t step, double threshold, uint8_t* keep, int64_t* n_kept) {
+  if (!c || !keep) return fail(TDSFS_ERR_ARG, "ctx / keep is NULL");
+  if (size < 2 || size > LD_MAX_SIZE || step < 1 || !std::isfinite(threshold) || threshold < 0.0 || threshold > 1.0)
+    return fail(TDSFS_ERR_ARG, "LD pruning takes 2 <= size <= %d, step >= 1 and a threshold in [0, 1] (got %d, %d, %g)",
+                LD_MAX_SIZE, size, step, threshold);
+  if (!c->loaded) return fail(TDSFS_ERR_STATE, "load data first");
+  if (!c->genotypes)
+    return fail(TDSFS_ERR_STATE, "LD pruning needs genotype calls (tdsfs_load_genotypes): the counts entry has no calls");
+  CK(cudaSetDevice(c->device));
+  NvtxRange nvtx("tdsfs:LD pruning");
+  cudaStream_t st = c->stream;
+  for (auto& ch : c->chunks) if (ch.ev) CK(cudaStreamWaitEvent(st, ch.ev, 0));
+  const long long S = c->S;
+  const int mw = (size - 1 + 31) / 32;
+  // the previous call ended with a synchronise: nothing still reads the old buffers
+  if (S * mw > c->ld_mask_cap) {
+    dev_free(c->d_ld_mask);
+    c->ld_mask_cap = 0;
+    CKR(dev_alloc(&c->d_ld_mask, S * mw));
+    c->ld_mask_cap = S * mw;
+  }
+  if (S > c->ld_keep_cap) {
+    dev_free(c->d_ld_keep);
+    c->ld_keep_cap = 0;
+    CKR(dev_alloc(&c->d_ld_keep, S));
+    c->ld_keep_cap = S;
+  }
+  LdParams p;
+  memset(&p, 0, sizeof p);
+  p.G = c->dG; p.S = S; p.W1 = c->W1; p.W2 = c->W2; p.ns1 = c->ns1; p.ns2 = c->ns2;
+  p.chrom_off = c->d_off; p.C = c->C;
+  p.size = size; p.step = step; p.mw = mw; p.thr = threshold;
+  p.mask = c->d_ld_mask; p.keep = c->d_ld_keep; p.n_kept = c->d_ld_n;
+  CK(cudaMemsetAsync(c->d_ld_n, 0, sizeof(unsigned long long), st));
+  CK(cudaEventRecord(c->ev_ld[0], st));
+  if (S > 0) {
+    const auto kern = segment_kernel(c, k_ld_pairs<32, 32>, k_ld_pairs<14, 14>, k_ld_pairs<0, 0>);
+    kern<<<(unsigned)((S + BLK - 1) / BLK), LD_WARPS * 32, 0, st>>>(p);
+    CK(cudaEventRecord(c->ev_ld[1], st));
+    k_ld_resolve<<<c->C, 32, 0, st>>>(p);
+    c->launches += 2;
+    CK(cudaGetLastError());
+  } else {
+    CK(cudaEventRecord(c->ev_ld[1], st));
+  }
+  CK(cudaEventRecord(c->ev_ld[2], st));
+  c->ld_timed = true;
+  unsigned long long nk = 0;
+  if (S > 0) CK(cudaMemcpyAsync(keep, c->d_ld_keep, (size_t)S, cudaMemcpyDeviceToHost, st));
+  CK(cudaMemcpyAsync(&nk, c->d_ld_n, sizeof nk, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  if (n_kept) *n_kept = (int64_t)nk;
+  return 0;
+}
+
 // ------------------------------------------------------------------------------------------------ explicit likelihood
 extern "C" int tdsfs_likelihood(tdsfs_t* c, const int64_t* x, const double* b, int64_t n, double B, double* T, int32_t* flag) {
   if (!c || !T || !flag || n < 0 || (n > 0 && (!x || !b))) return fail(TDSFS_ERR_ARG, "bad argument");
@@ -1812,7 +1884,7 @@ extern "C" int tdsfs_timings(tdsfs_t* c, float* ms, int32_t n) {
   if (!c || !ms) return fail(TDSFS_ERR_ARG, "NULL argument");
   CK(cudaSetDevice(c->device));
   CK(cudaStreamSynchronize(c->stream));
-  for (int i = 0; i < 12; ++i) c->ms[i] = 0.f;
+  for (int i = 0; i < 14; ++i) c->ms[i] = 0.f;
   if (c->keys_ready) cudaEventElapsedTime(&c->ms[0], c->ev[EV_BG0], c->ev[EV_K1]);
   if (c->fin_timed) cudaEventElapsedTime(&c->ms[1], c->ev[EV_FIN0], c->ev[EV_FIN1]);
   if (c->results_ready) {
@@ -1828,8 +1900,12 @@ extern "C" int tdsfs_timings(tdsfs_t* c, float* ms, int32_t n) {
   if (c->div.timed) cudaEventElapsedTime(&c->ms[9], c->div.ev0, c->div.ev1);
   if (c->neut.timed) cudaEventElapsedTime(&c->ms[10], c->neut.ev0, c->neut.ev1);
   if (c->wc.timed) cudaEventElapsedTime(&c->ms[11], c->wc.ev0, c->wc.ev1);
+  if (c->ld_timed) {
+    cudaEventElapsedTime(&c->ms[12], c->ev_ld[0], c->ev_ld[1]);
+    cudaEventElapsedTime(&c->ms[13], c->ev_ld[1], c->ev_ld[2]);
+  }
   cudaGetLastError();
-  for (int i = 0; i < n && i < 12; ++i) ms[i] = c->ms[i];
+  for (int i = 0; i < n && i < 14; ++i) ms[i] = c->ms[i];
   return 0;
 }
 

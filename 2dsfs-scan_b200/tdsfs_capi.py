@@ -25,12 +25,13 @@ EXPORTS = [
     "tdsfs_diversity_bp", "tdsfs_diversity_snp", "tdsfs_fetch_diversity",
     "tdsfs_neutrality_bp", "tdsfs_neutrality_snp", "tdsfs_fetch_neutrality",
     "tdsfs_wcfst_bp", "tdsfs_wcfst_snp", "tdsfs_fetch_wcfst",
+    "tdsfs_ld_prune",
 ]
 
 
 PEER_BLOB_BYTES = 192  # TDSFS_PEER_BLOB_BYTES
 TIMING_NAMES = ("k1_count", "finalize", "k2_bounds", "k3_small", "k3_large", "background_call", "scan_call", "pass_total",
-                "exchange", "diversity", "neutrality", "wcfst")  # the slots of tdsfs_timings
+                "exchange", "diversity", "neutrality", "wcfst", "ld_pairs", "ld_resolve")  # the slots of tdsfs_timings
 
 
 class TdsfsError(RuntimeError):
@@ -119,6 +120,7 @@ class Handle:
         self._check(self._L.tdsfs_create(C.c_int(device), C.byref(self._h)))
         self.n1 = self.n2 = 0
         self.C = 0
+        self.S = 0
 
     def _check(self, rc):
         if rc != 0:
@@ -156,6 +158,7 @@ class Handle:
             flags = np.ascontiguousarray(flags, dtype=np.uint8)
         self._keep = [cnt, pos, off, flags]
         self.C = len(off) - 1
+        self.S = int(S)
         self._check(self._L.tdsfs_load_counts(self._h, _ptr(cnt), C.c_int64(S), _ptr(pos), _ptr(off), C.c_int32(self.C), _ptr(flags)))
 
     def load_genotypes(self, G, S, words1, words2, ns1, ns2, pos, chrom_off, fixups=None, flags=None):
@@ -173,6 +176,7 @@ class Handle:
             fixups = None
         self._keep = [G, pos, off, flags, fixups]
         self.C = len(off) - 1
+        self.S = int(S)
         self._check(self._L.tdsfs_load_genotypes(self._h, _ptr(G), C.c_int64(S), C.c_int32(words1), C.c_int32(words2),
                                                  C.c_int32(ns1), C.c_int32(ns2), _ptr(pos), _ptr(off), C.c_int32(self.C),
                                                  _ptr(fixups), C.c_int64(nfix), _ptr(flags)))
@@ -325,6 +329,18 @@ class Handle:
     def fetch_wcfst(self, cap):
         return self._into(self._alloc_wcfst, cap, self._L.tdsfs_fetch_wcfst)
 
+    def ld_prune(self, size, step, threshold):
+        """LD pruning of the loaded genotype rows (tdsfs_ld_prune): scikit-allel's locate_unlinked(gn, size, step,
+        threshold) per chromosome, r^2 over the samples of both populations called in both rows, exact integer sums with
+        one rounded division.  Returns a bool array over the loaded rows, True = kept."""
+        keep = np.zeros(max(self.S, 1), dtype=np.uint8)
+        n = C.c_int64()
+        self._check(self._L.tdsfs_ld_prune(self._h, C.c_int32(size), C.c_int32(step), C.c_double(threshold), _ptr(keep),
+                                           C.byref(n)))
+        out = keep[:self.S].astype(bool)
+        assert int(out.sum()) == n.value
+        return out
+
     def fetch_results(self, cap):
         return self._into(self._alloc_result, cap, self._L.tdsfs_fetch_results)
 
@@ -385,6 +401,11 @@ class Handle:
     def wcfst_ms(self):
         """CUDA-event time (ms) of the segment + finish kernels of the last wcfst call (tdsfs_timings slot 11)."""
         return self.timings()["wcfst"]
+
+    def ld_prune_ms(self):
+        """CUDA-event time (ms) of the pair and resolve kernels of the last ld_prune call (tdsfs_timings slots 12 + 13)."""
+        t = self.timings()
+        return t["ld_pairs"] + t["ld_resolve"]
 
     def launch_count(self):
         return int(self._L.tdsfs_launch_count(self._h))

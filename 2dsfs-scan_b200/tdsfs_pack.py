@@ -133,6 +133,7 @@ class PackedPanel:
         self.last_key_row = -1
         self.n_records = self.n_skipped = 0
         self.cache_sources = []
+        self.ld_prune = None     # (size, step, threshold) of the LD pruning that produced this panel (subset_panel)
 
     def __len__(self):
         return self.n
@@ -194,6 +195,8 @@ def save_panel(panel, path, sources=()):
               "chroms": list(panel.chroms), "pops": list(panel.pops), "last_key_row": int(panel.last_key_row),
               "n_records": int(panel.n_records), "n_skipped": int(panel.n_skipped), "ann_vocab": [str(v) for v in vocab],
               "sources": _source_stamp(sources), "arrays": {}}
+    if panel.ld_prune is not None:
+        header["ld_prune"] = [int(panel.ld_prune[0]), int(panel.ld_prune[1]), float(panel.ld_prune[2])]
     # two passes: the header's length decides the first offset
     offset = 0
     for _ in range(2):
@@ -249,6 +252,51 @@ def load_panel(path, mmap=True):
     fx = arr("fixups", _FIX_DT)
     P.fixups = np.array(fx) if len(fx) else None
     P.cache_sources = header["sources"]
+    lp = header.get("ld_prune")  # absent: not a pruned panel (every file written before the key existed)
+    P.ld_prune = None if lp is None else (int(lp[0]), int(lp[1]), float(lp[2]))
+    return P
+
+
+def subset_panel(panel, keep, ld_prune=None):
+    """The rows of `panel` where keep[S] is True, as a new PackedPanel that looks like one the packer could have produced
+    from the VCF with only those records: G rebuilt in the B32 layout, positions, annotations and fix-ups (renumbered) of
+    the kept rows, `off` recomputed and chromosomes left without rows dropped.  last_key_row (the row of the VCF's last
+    record) maps to its kept row; when that row is dropped, to the nearest kept row before it on its chromosome (the last
+    record of a position-sorted VCF filtered the same way), else to the panel's last kept row.  n_records / n_skipped stay
+    those of the VCF the panel was packed from.  cache_sources is empty, so that cached_pack_vcf never takes the subset for
+    the VCF's own cache; ld_prune records the (size, step, threshold) that chose the rows, if any.  The matrix goes through
+    row-major form on the host (from_b32 / to_b32): about 3x the panel's genotype bytes of host RAM at the peak."""
+    keep = np.asarray(keep, dtype=bool)
+    if keep.shape != (panel.n,):
+        raise ValueError(f"keep has shape {keep.shape}; the panel has {panel.n} rows")
+    idx = np.flatnonzero(keep)
+    new_row = np.cumsum(keep) - 1  # new index of every kept row
+    off = np.asarray(panel.off, dtype=np.int64)
+    per_chrom = np.array([int(keep[off[c]:off[c + 1]].sum()) for c in range(len(panel.chroms))], dtype=np.int64)
+    P = PackedPanel()
+    P.W1, P.W2, P.ns1, P.ns2, P.pops = panel.W1, panel.W2, panel.ns1, panel.ns2, tuple(panel.pops)
+    P.n = len(idx)
+    P.G = to_b32(from_b32(panel.G, panel.n, panel.W1 + panel.W2)[idx]) if P.n else np.zeros(0, dtype=np.uint32)
+    P.pos = np.asarray(panel.pos, dtype=np.int64)[idx]
+    P.chroms = [c for c, k in zip(panel.chroms, per_chrom) if k > 0]
+    P.off = np.concatenate([[0], np.cumsum(per_chrom[per_chrom > 0])]).astype(np.int64)
+    P.ann = np.asarray(panel.ann, dtype=object)[idx] if P.n else np.array([], dtype=object)
+    P.fixups = None
+    if panel.fixups is not None and len(panel.fixups):
+        fx = np.asarray(panel.fixups)
+        fx = fx[keep[fx["snp"]]].copy()
+        if len(fx):
+            fx["snp"] = new_row[fx["snp"]]
+            P.fixups = fx
+    last = int(panel.last_key_row)
+    P.last_key_row = -1
+    if 0 <= last < panel.n and P.n:
+        c = int(np.searchsorted(off, last, side="right")) - 1
+        before = np.flatnonzero(keep[off[c]:last + 1])
+        P.last_key_row = int(new_row[off[c] + before[-1]]) if len(before) else P.n - 1
+    P.n_records, P.n_skipped = panel.n_records, panel.n_skipped
+    P.cache_sources = []
+    P.ld_prune = None if ld_prune is None else (int(ld_prune[0]), int(ld_prune[1]), float(ld_prune[2]))
     return P
 
 
@@ -260,7 +308,7 @@ def cached_pack_vcf(vcf_filename, popinfo_filename, pop1, pop2, cache_path=None,
     if _os.path.exists(cache_path):
         try:
             P = load_panel(cache_path)
-            if P.cache_sources == _source_stamp(srcs) and tuple(P.pops) == (pop1, pop2):
+            if P.cache_sources == _source_stamp(srcs) and tuple(P.pops) == (pop1, pop2) and P.ld_prune is None:
                 return P
         except (ValueError, KeyError, OSError):
             pass

@@ -583,6 +583,27 @@ class LikelihoodInference_jointSFS:
         self.snp_window_size = snp_window_size
         return self._wc_fst(panel, snp_window_size, True)
 
+    # ------------------------------------------------------------------ LD pruning (not in the reference)
+    def ld_prune(self, panel, size=100, step=20, threshold=0.1):
+        """Drop the SNPs in linkage disequilibrium from a make_packed_panel panel, on the GPU: scikit-allel's
+        locate_unlinked(gn, size, step, threshold) (defaults are its own), the windowed greedy r^2 rule of PLINK's
+        --indep-pairwise.  Per chromosome, windows of `size` SNPs start every `step` SNPs; walking the SNPs in order, a SNP
+        is dropped when its r^2 with an earlier kept SNP of a common window exceeds `threshold`.  r^2 is the squared
+        correlation of the alt-allele dosages (0, 1, 2) over the samples of both populations called at both SNPs; calls the
+        packer holds as fix-ups (half calls, haploid and multi-allelic calls) count as missing.  The constructor's
+        start_position / end_position / variant_type filters are NOT applied: pruning covers every SNP of the panel, and
+        the scans apply their filters to the pruned panel afterwards.  Returns the pruned PackedPanel (tdsfs_pack.subset_panel),
+        which every scan and window pass accepts; its ld_prune attribute holds (size, step, threshold).  2 <= size <= 1024,
+        step >= 1, threshold in [0, 1].  Not in the reference, which reads VCFs pruned beforehand with PLINK."""
+        if not isinstance(panel, PackedPanel):
+            raise TypeError("LD pruning needs the genotype calls: pass the PackedPanel of make_packed_panel "
+                            "(a data_dict holds allele counts only, without genotypes)")
+        import tdsfs_pack
+        eng = self._eng()
+        eng.load(panel, self.pop1_size, self.pop2_size, self.fold)
+        keep = eng.h.ld_prune(int(size), int(step), float(threshold))
+        return tdsfs_pack.subset_panel(panel, keep, (size, step, threshold))
+
     # ------------------------------------------------------------------ simulations
     def get_gens(self, main_dir):
         search_strings = set()

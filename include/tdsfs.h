@@ -314,6 +314,27 @@ int tdsfs_wcfst_bp(tdsfs_t* ctx, int64_t W, tdsfs_wcfst_t* out, int64_t cap, int
 int tdsfs_wcfst_snp(tdsfs_t* ctx, int64_t N, tdsfs_wcfst_t* out, int64_t cap, int64_t* n_windows);
 int tdsfs_fetch_wcfst(tdsfs_t* ctx, tdsfs_wcfst_t* out, int64_t cap, int64_t* n_windows);
 
+/* ---- LD pruning of the genotype rows (no reference counterpart; DESIGN.md 7) -----------------------------------------
+ * scikit-allel's locate_unlinked (the windowed greedy r^2 rule of PLINK's --indep-pairwise) over the rows loaded with
+ * tdsfs_load_genotypes.  Samples: both populations pooled (ns1 + ns2, the padding bits of a population's last pair are not
+ * samples).  Dosage: codes 00, 01, 11 give g = 0, 1, 2; code 10 is missing, and so are the calls held as fix-ups (half
+ * calls, haploid calls, multi-allelic digits are 10 in the matrix).  r^2 of rows i and j over the n samples called in both,
+ * Sx = sum g_i, Sy = sum g_j, Qx = sum g_i^2, Qy = sum g_j^2, P = sum g_i g_j:
+ *   cov = n P - Sx Sy,  vx = n Qx - Sx^2,  vy = n Qy - Sy^2   (exact int64),
+ *   r^2 = double(cov^2) / double(vx vy)                        (each uint64 converted with round to nearest, one division);
+ * undefined, and never pruning, when vx vy = 0 (n = 0 included).  With ns1, ns2 <= 32767 every term is exact.
+ * Per chromosome, over rows in loaded order, c0 the chromosome's first row: window k covers rows [c0 + k step,
+ * c0 + k step + size) clipped to the chromosome; rows i < j are tested iff a window holds both, j - c0 < floor((i - c0) /
+ * step) step + size.  Rows are decided in increasing order: row j is kept iff no kept row i < j tested with j has r^2 >
+ * threshold.  This is the final loc of locate_unlinked(gn, size, step, threshold) run on one chromosome in one block
+ * (gn = g.to_n_alt(fill=-1)), up to its float32 rounding of r^2.  Parity with PLINK is not claimed.
+ * 2 <= size <= 1024, step >= 1 (step > size leaves some neighbouring pairs untested, as in scikit-allel), threshold finite
+ * in [0, 1]; else TDSFS_ERR_ARG, as for a NULL keep.  TDSFS_ERR_STATE when nothing is loaded or the counts entry is (it has
+ * no calls).  Synchronous: keep (caller-owned host buffer of S bytes) receives 1 for a kept row, 0 for a pruned one, and
+ * *n_kept (may be NULL) the kept count.  Own workspace: a pending plan, the scan's unfetched results, the step graph and
+ * the per-window passes' results are left as they were. */
+int tdsfs_ld_prune(tdsfs_t* ctx, int32_t size, int32_t step, double threshold, uint8_t* keep, int64_t* n_kept);
+
 /* ---- likelihood of explicit spectra ------------------------------------------------------------------------
  * calculate_likelihood_1D / _2D (:478-537, :625-684) on already-interior vectors: x[n] integer counts,
  * b[n] background values, B = sum of b as the caller's language sums it.  *flag = 1 when the reference returns
@@ -334,7 +355,8 @@ int tdsfs_synth_genotypes(tdsfs_t* ctx, void* G_dev, int64_t S, int64_t snp0, in
  * [5]=background call, [6]=scan call, [7]=K1 start -> last score kernel end, [8]=peer exchange kernel (n >= 9),
  * [9]=segment + finish kernels of the last tdsfs_diversity_* call (n >= 10),
  * [10]=segment + finish kernels of the last tdsfs_neutrality_* call (n >= 11),
- * [11]=segment + finish kernels of the last tdsfs_wcfst_* call (n >= 12). */
+ * [11]=segment + finish kernels of the last tdsfs_wcfst_* call (n >= 12),
+ * [12]=k_ld_pairs and [13]=k_ld_resolve of the last tdsfs_ld_prune call (n >= 14). */
 int tdsfs_timings(tdsfs_t* ctx, float* ms, int32_t n);
 int64_t tdsfs_launch_count(tdsfs_t* ctx); /* kernels launched by this handle so far */
 /* Which path scored the last scan: *fused = 1 when the fused pair ran (tdsfs_plan_* before tdsfs_background on the
