@@ -117,7 +117,9 @@ __device__ __forceinline__ int next_window_start(const FusedParams& q, int t, in
 // lengths then differ by at most one window instead of two.  nearest = false snaps back instead: the two ends of a launch,
 // because rows past the end may still be uploading.
 // is_start = the returned row starts a window (or lies in none); false when the window holding t began more than WCAP rows
-// earlier (such a window is larger than the warp tables: nobody sums it here, the CTA path scores it).
+// earlier and t itself is returned (such a window is larger than the warp tables: nobody sums it here, the CTA path scores
+// it).  nearest returns t there only when the window also ends more than WCAP rows later; otherwise its end, which keeps
+// the snapped boundaries monotone.
 __device__ __forceinline__ int snap_row(const FusedParams& q, int t, bool& is_start, int lane, bool nearest) {
   const KeyParams& p = q.k;
   is_start = true;
@@ -155,6 +157,12 @@ __device__ __forceinline__ int snap_row(const FusedParams& q, int t, bool& is_st
     back = min(base + __ffs(b2) - 1, t);
   } else if (f == 0) {                   // row lo already belongs to the window
     if (lo != cw.lo) {                   // ... and it began even earlier: larger than WCAP rows
+      // nearest: the window's end when it lies within WCAP rows.  An earlier target of this window may have snapped forward
+      // to that end, and returning t < end would then hand rows [t, end) to two warps (counted twice in the background)
+      if (nearest) {
+        const int fwd = next_window_start(q, t, k, cw, lane);
+        if (fwd >= 0) return fwd;
+      }
       is_start = false;
       return t;
     }
