@@ -19,7 +19,7 @@
 
 using namespace tdsfs;
 
-#define TDSFS_VERSION 204
+#define TDSFS_VERSION 205
 
 static thread_local std::string g_err;
 
@@ -83,14 +83,14 @@ struct CandCache {
 };
 
 // Workspace and results of one per-window pass over the candidate windows of (size, mode) (tdsfs_diversity_*,
-// tdsfs_neutrality_*, tdsfs_wcfst_*): its candidate offsets, window boundaries, segment list, scan scratch, per-segment sums, per-window
-// results and events.
+// tdsfs_neutrality_*, tdsfs_wcfst_*, tdsfs_ld_windows_*): its candidate offsets, window boundaries, segment list, scan
+// scratch, per-segment sums, per-window results and events.
 struct WindowPass {
-  WindowPass(const char* name, size_t part_bytes, int n_i32, int n_f64)
-      : name(name), part_bytes(part_bytes), n_i32(n_i32), n_f64(n_f64) {}
+  WindowPass(const char* name, size_t part_bytes, int n_i32, int n_f64, int n_i64 = 0)
+      : name(name), part_bytes(part_bytes), n_i32(n_i32), n_f64(n_f64), n_i64(n_i64) {}
   const char* name;                   // NVTX range of a call
-  size_t part_bytes;                  // size of the pass's per-segment sums (DivPart, NeutPart, WcPart)
-  int n_i32, n_f64;                   // result columns of the pass in d_i32 / d_f64
+  size_t part_bytes;                  // size of the pass's per-segment sums (DivPart, NeutPart, WcPart; 0: none)
+  int n_i32, n_f64, n_i64;            // result columns of the pass in d_i32 / d_f64 / d_i64
   CandCache cand;
   long long cap = 0, ncand = 0;       // windows the per-window arrays hold / of the last call
   size_t tmp_bytes = 0;
@@ -102,6 +102,7 @@ struct WindowPass {
   void* d_tmp = nullptr;              // CUB scan scratch
   int32_t* d_i32[4] = {};             // [cap] the pass's int32 and fp64 result columns, each in the order of its result
   double* d_f64[6] = {};              // struct in include/tdsfs.h
+  long long* d_i64[4] = {};
   void* d_part = nullptr;             // [part_cap] per-segment sums
   long long part_cap = 0;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;  // around the segment and finish kernels (tdsfs_timings)
@@ -215,6 +216,7 @@ struct tdsfs_ctx {
   WindowPass div{"tdsfs:diversity (FST, pi, dxy)", sizeof(DivPart), 1, 4};                 // tdsfs_diversity_*
   WindowPass neut{"tdsfs:neutrality (theta_W, Tajima's D)", sizeof(NeutPart), 4, 6};      // tdsfs_neutrality_*
   WindowPass wc{"tdsfs:Weir and Cockerham FST", sizeof(WcPart), 1, 4};                    // tdsfs_wcfst_*
+  WindowPass ldw{"tdsfs:LD windows (ZnS, omega)", 0, 2, 4, 4};                             // tdsfs_ld_windows_*
   double* d_neut_tab = nullptr;       // a1(n) for n in [0, neut_tab_n], then a2(n) for the same n
   long long neut_tab_n = -1;
   long long n_allele_max = 0;         // the largest n_i = ref_i + alt_i a row of the loaded data can reach
@@ -227,9 +229,14 @@ struct tdsfs_ctx {
   unsigned long long* d_ld_n = nullptr;  // kept rows
   cudaEvent_t ev_ld[3] = {};          // before k_ld_pairs, between the kernels, after k_ld_resolve (tdsfs_timings)
   bool ld_timed = false;
+  // per-row scratch of tdsfs_ld_windows_* (LdwParams), grown lazily: c and d sums, their pair counts, site bits
+  unsigned long long* d_ldw_sum = nullptr;  // [4 * ldw_cap]
+  uint32_t* d_ldw_cnt = nullptr;            // [4 * ldw_cap]
+  uint8_t* d_ldw_site = nullptr;            // [ldw_cap]
+  long long ldw_cap = 0;
   // instrumentation
   cudaEvent_t ev[NEV] = {};
-  float ms[14] = {};
+  float ms[15] = {};
   long long launches = 0;
 };
 
@@ -298,7 +305,7 @@ extern "C" int tdsfs_create(int device, tdsfs_t** out) {
   CK(cudaEventCreate(&c->ev_plan0));
   c->stream = c->own_stream;
   for (int i = 0; i < NEV; ++i) CK(cudaEventCreate(&c->ev[i]));
-  for (WindowPass* w : {&c->div, &c->neut, &c->wc}) {
+  for (WindowPass* w : {&c->div, &c->neut, &c->wc, &c->ldw}) {
     CK(cudaEventCreate(&w->ev0));
     CK(cudaEventCreate(&w->ev1));
   }
@@ -362,7 +369,7 @@ static void free_data(tdsfs_ctx* c) {
   c->plan_W = -1;
   c->ws_ready = false;
   c->force_wide = false;
-  for (WindowPass* w : {&c->div, &c->neut, &c->wc}) {
+  for (WindowPass* w : {&c->div, &c->neut, &c->wc, &c->ldw}) {
     w->cand.W = -1;
     w->ready = false;
   }
@@ -375,6 +382,7 @@ static void free_pass_windows(WindowPass& w) {
   dev_free(w.d_nseg); dev_free(w.d_segoff); dev_free(w.d_flags); dev_free(w.d_tmp);
   for (int32_t*& a : w.d_i32) dev_free(a);
   for (double*& a : w.d_f64) dev_free(a);
+  for (long long*& a : w.d_i64) dev_free(a);
 }
 
 static void free_window_pass(WindowPass& w) {
@@ -411,8 +419,10 @@ extern "C" void tdsfs_destroy(tdsfs_t* c) {
   free_window_pass(c->div);
   free_window_pass(c->neut);
   free_window_pass(c->wc);
+  free_window_pass(c->ldw);
   dev_free(c->d_neut_tab);
   dev_free(c->d_ld_mask); dev_free(c->d_ld_keep); dev_free(c->d_ld_n);
+  dev_free(c->d_ldw_sum); dev_free(c->d_ldw_cnt); dev_free(c->d_ldw_site);
   for (cudaEvent_t e : c->ev_ld) if (e) cudaEventDestroy(e);
   cudaStreamDestroy(c->own_stream);
   cudaStreamDestroy(c->copy_stream);
@@ -1511,6 +1521,7 @@ extern "C" int tdsfs_window_spectra(tdsfs_t* c, int64_t window, uint64_t* s2, ui
 // Arrays of pass w for ncand windows and `parts` segments, grown after the stream has drained (a previous asynchronous
 // call may still use the old ones).
 static int pass_buffers(tdsfs_ctx* c, WindowPass& w, long long ncand, long long parts) {
+  if (!w.part_bytes) parts = 0;  // a pass without per-segment sums
   if (ncand > w.cap || parts > w.part_cap) CK(cudaStreamSynchronize(c->stream));
   if (ncand > w.cap) {
     free_pass_windows(w);
@@ -1519,6 +1530,7 @@ static int pass_buffers(tdsfs_ctx* c, WindowPass& w, long long ncand, long long 
     CKR(dev_alloc(&w.d_nseg, ncand + 1)); CKR(dev_alloc(&w.d_segoff, ncand + 1)); CKR(dev_alloc(&w.d_flags, ncand));
     for (int i = 0; i < w.n_i32; ++i) CKR(dev_alloc(&w.d_i32[i], ncand));
     for (int i = 0; i < w.n_f64; ++i) CKR(dev_alloc(&w.d_f64[i], ncand));
+    for (int i = 0; i < w.n_i64; ++i) CKR(dev_alloc(&w.d_i64[i], ncand));
     size_t tmp = 0;
     CK(cub::DeviceScan::ExclusiveSum(nullptr, tmp, w.d_nseg, w.d_segoff, (int)(ncand + 1), c->stream));
     CK(cudaMalloc(&w.d_tmp, std::max<size_t>(tmp, 16)));
@@ -1814,6 +1826,73 @@ extern "C" int tdsfs_ld_prune(tdsfs_t* c, int32_t size, int32_t step, double thr
   return 0;
 }
 
+// ------------------------------------------------------------------------------------------------ per-window LD (ZnS, omega)
+extern "C" int tdsfs_fetch_ld_windows(tdsfs_t* c, tdsfs_ld_windows_t* out, int64_t cap, int64_t* n_windows) {
+  if (!c || !out) return fail(TDSFS_ERR_ARG, "NULL argument");
+  const WindowPass& w = c->ldw;
+  if (!w.ready) return fail(TDSFS_ERR_STATE, "no LD window results (tdsfs_ld_windows_bp / _snp first)");
+  if (cap < w.ncand) return fail(TDSFS_ERR_ARG, "result capacity %lld < %lld candidate windows", (long long)cap, w.ncand);
+  CK(cudaSetDevice(c->device));
+  return fetch_columns(c, w.ncand, {{out->chrom, w.d_wchrom}, {out->start, w.d_wstart}, {out->end, w.d_wend},
+                                    {out->snp_count, w.d_count}, {out->flags, w.d_flags}, {out->n_sites_p1, w.d_i32[0]},
+                                    {out->n_sites_p2, w.d_i32[1]}, {out->n_pairs_p1, w.d_i64[0]},
+                                    {out->n_pairs_p2, w.d_i64[1]}, {out->zns_p1, w.d_f64[0]}, {out->zns_p2, w.d_f64[1]},
+                                    {out->omega_p1, w.d_f64[2]}, {out->omega_p2, w.d_f64[3]},
+                                    {out->omega_pos_p1, w.d_i64[2]}, {out->omega_pos_p2, w.d_i64[3]}}, n_windows);
+}
+
+// The pass reads the 2-bit calls, and its per-row scratch (about 49 bytes a row) is grown after the stream has drained (a
+// previous asynchronous call may still use it).
+static int ldw_prepare(tdsfs_ctx* c) {
+  if (!c->genotypes)
+    return fail(TDSFS_ERR_STATE, "LD windows need genotype calls (tdsfs_load_genotypes): the counts entry has no calls");
+  if (c->S > c->ldw_cap) {
+    CK(cudaStreamSynchronize(c->stream));
+    dev_free(c->d_ldw_sum); dev_free(c->d_ldw_cnt); dev_free(c->d_ldw_site);
+    c->ldw_cap = 0;
+    CKR(dev_alloc(&c->d_ldw_sum, 4 * c->S)); CKR(dev_alloc(&c->d_ldw_cnt, 4 * c->S)); CKR(dev_alloc(&c->d_ldw_site, c->S));
+    c->ldw_cap = c->S;
+  }
+  // k_ld_windows adds into d and its counts
+  CK(cudaMemsetAsync(c->d_ldw_sum + 2 * c->S, 0, (size_t)(2 * c->S) * sizeof(unsigned long long), c->stream));
+  CK(cudaMemsetAsync(c->d_ldw_cnt + 2 * c->S, 0, (size_t)(2 * c->S) * sizeof(uint32_t), c->stream));
+  return 0;
+}
+
+// k_ld_windows (one CTA per 32-row block: its own grid, not the segment grid) -> k_ldw_finish.
+static void launch_ld_windows(tdsfs_ctx* c, unsigned) {
+  const WindowPass& w = c->ldw;
+  const long long S = c->S;
+  LdwParams p;
+  memset(&p, 0, sizeof p);
+  p.G = c->dG; p.S = S; p.W1 = c->W1; p.W2 = c->W2; p.ns1 = c->ns1; p.ns2 = c->ns2;
+  p.flags = c->dFlags; p.pos = c->dPos; p.seg = w.segs();
+  p.c = c->d_ldw_sum; p.d = c->d_ldw_sum + 2 * S; p.cn = c->d_ldw_cnt; p.dn = c->d_ldw_cnt + 2 * S; p.site = c->d_ldw_site;
+  p.snp_count = w.d_count; p.out_flags = w.d_flags;
+  for (int i = 0; i < 2; ++i) {
+    p.n_sites[i] = w.d_i32[i]; p.n_pairs[i] = w.d_i64[i]; p.zns[i] = w.d_f64[i]; p.omega[i] = w.d_f64[2 + i];
+    p.omega_pos[i] = w.d_i64[2 + i];
+  }
+  if (S > 0) {
+    const auto kern = segment_kernel(c, k_ld_windows<32, 32>, k_ld_windows<14, 14>, k_ld_windows<0, 0>);
+    kern<<<(unsigned)((S + BLK - 1) / BLK), LD_WARPS * 32, 0, c->stream>>>(p);
+  }
+  k_ldw_finish<<<(unsigned)((w.ncand + LDW_FIN_WARPS - 1) / LDW_FIN_WARPS), LDW_FIN_WARPS * 32, 0, c->stream>>>(p);
+}
+
+// Per-window, per-population Kelly's ZnS and Kim and Nielsen's omega from the genotype calls.
+static int ld_windows(tdsfs_ctx* c, long long W, bool snp_mode, tdsfs_ld_windows_t* out, int64_t cap, int64_t* n_windows) {
+  CKR(window_pass(c, &tdsfs_ctx::ldw, W, snp_mode, out != nullptr, cap, n_windows, ldw_prepare, launch_ld_windows));
+  return out ? tdsfs_fetch_ld_windows(c, out, cap, n_windows) : 0;
+}
+
+extern "C" int tdsfs_ld_windows_bp(tdsfs_t* c, int64_t W, tdsfs_ld_windows_t* out, int64_t cap, int64_t* n_windows) {
+  return ld_windows(c, W, false, out, cap, n_windows);
+}
+extern "C" int tdsfs_ld_windows_snp(tdsfs_t* c, int64_t N, tdsfs_ld_windows_t* out, int64_t cap, int64_t* n_windows) {
+  return ld_windows(c, N, true, out, cap, n_windows);
+}
+
 // ------------------------------------------------------------------------------------------------ explicit likelihood
 extern "C" int tdsfs_likelihood(tdsfs_t* c, const int64_t* x, const double* b, int64_t n, double B, double* T, int32_t* flag) {
   if (!c || !T || !flag || n < 0 || (n > 0 && (!x || !b))) return fail(TDSFS_ERR_ARG, "bad argument");
@@ -1884,7 +1963,7 @@ extern "C" int tdsfs_timings(tdsfs_t* c, float* ms, int32_t n) {
   if (!c || !ms) return fail(TDSFS_ERR_ARG, "NULL argument");
   CK(cudaSetDevice(c->device));
   CK(cudaStreamSynchronize(c->stream));
-  for (int i = 0; i < 14; ++i) c->ms[i] = 0.f;
+  for (int i = 0; i < 15; ++i) c->ms[i] = 0.f;
   if (c->keys_ready) cudaEventElapsedTime(&c->ms[0], c->ev[EV_BG0], c->ev[EV_K1]);
   if (c->fin_timed) cudaEventElapsedTime(&c->ms[1], c->ev[EV_FIN0], c->ev[EV_FIN1]);
   if (c->results_ready) {
@@ -1904,8 +1983,9 @@ extern "C" int tdsfs_timings(tdsfs_t* c, float* ms, int32_t n) {
     cudaEventElapsedTime(&c->ms[12], c->ev_ld[0], c->ev_ld[1]);
     cudaEventElapsedTime(&c->ms[13], c->ev_ld[1], c->ev_ld[2]);
   }
+  if (c->ldw.timed) cudaEventElapsedTime(&c->ms[14], c->ldw.ev0, c->ldw.ev1);
   cudaGetLastError();
-  for (int i = 0; i < n && i < 14; ++i) ms[i] = c->ms[i];
+  for (int i = 0; i < n && i < 15; ++i) ms[i] = c->ms[i];
   return 0;
 }
 

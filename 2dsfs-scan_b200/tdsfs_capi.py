@@ -26,12 +26,14 @@ EXPORTS = [
     "tdsfs_neutrality_bp", "tdsfs_neutrality_snp", "tdsfs_fetch_neutrality",
     "tdsfs_wcfst_bp", "tdsfs_wcfst_snp", "tdsfs_fetch_wcfst",
     "tdsfs_ld_prune",
+    "tdsfs_ld_windows_bp", "tdsfs_ld_windows_snp", "tdsfs_fetch_ld_windows",
 ]
 
 
 PEER_BLOB_BYTES = 192  # TDSFS_PEER_BLOB_BYTES
 TIMING_NAMES = ("k1_count", "finalize", "k2_bounds", "k3_small", "k3_large", "background_call", "scan_call", "pass_total",
-                "exchange", "diversity", "neutrality", "wcfst", "ld_pairs", "ld_resolve")  # the slots of tdsfs_timings
+                "exchange", "diversity", "neutrality", "wcfst", "ld_pairs", "ld_resolve",
+                "ld_windows")  # the slots of tdsfs_timings
 
 
 class TdsfsError(RuntimeError):
@@ -47,8 +49,8 @@ class Fixup(C.Structure):
 FIXUP_DTYPE = np.dtype([("snp", "<i8"), ("pop", "<i4"), ("dref", "<i4"), ("dalt", "<i4")], align=True)
 
 
-# Per-window result columns in the member order of tdsfs_result_t, tdsfs_diversity_t, tdsfs_neutrality_t and
-# tdsfs_wcfst_t: each of those structs holds one host pointer per column.
+# Per-window result columns in the member order of tdsfs_result_t, tdsfs_diversity_t, tdsfs_neutrality_t, tdsfs_wcfst_t
+# and tdsfs_ld_windows_t: each of those structs holds one host pointer per column.
 RESULT_DTYPES = dict(chrom=np.int32, start=np.int64, end=np.int64, snp_count=np.int32, n2d=np.int32, n1d_p1=np.int32,
                      n1d_p2=np.int32, T2D=np.float64, T1D_p1=np.float64, T1D_p2=np.float64, flags=np.uint8)
 DIVERSITY_DTYPES = dict(chrom=np.int32, start=np.int64, end=np.int64, snp_count=np.int32, flags=np.uint8, n_sites=np.int32,
@@ -59,6 +61,10 @@ NEUTRALITY_DTYPES = dict(chrom=np.int32, start=np.int64, end=np.int64, snp_count
                          tajima_d_p2=np.float64)
 WCFST_DTYPES = dict(chrom=np.int32, start=np.int64, end=np.int64, snp_count=np.int32, flags=np.uint8, n_sites=np.int32,
                     a=np.float64, b=np.float64, c=np.float64, fst=np.float64)
+LD_WINDOWS_DTYPES = dict(chrom=np.int32, start=np.int64, end=np.int64, snp_count=np.int32, flags=np.uint8,
+                         n_sites_p1=np.int32, n_sites_p2=np.int32, n_pairs_p1=np.int64, n_pairs_p2=np.int64,
+                         zns_p1=np.float64, zns_p2=np.float64, omega_p1=np.float64, omega_p2=np.float64,
+                         omega_pos_p1=np.int64, omega_pos_p2=np.int64)
 
 
 class Result(C.Structure):
@@ -75,6 +81,10 @@ class Neutrality(C.Structure):
 
 class WcFst(C.Structure):
     _fields_ = [(k, C.c_void_p) for k in WCFST_DTYPES]
+
+
+class LdWindows(C.Structure):
+    _fields_ = [(k, C.c_void_p) for k in LD_WINDOWS_DTYPES]
 
 
 _lib = None
@@ -275,6 +285,10 @@ class Handle:
     def _alloc_wcfst(n):
         return Handle._alloc(WCFST_DTYPES, WcFst, n)
 
+    @staticmethod
+    def _alloc_ld_windows(n):
+        return Handle._alloc(LD_WINDOWS_DTYPES, LdWindows, n)
+
     def _into(self, alloc, cap, f, *args):
         """f(handle, *args, out, cap, &n) into the arrays alloc(cap) allocates: dict of their first n entries."""
         arrs, r = alloc(cap)
@@ -328,6 +342,21 @@ class Handle:
 
     def fetch_wcfst(self, cap):
         return self._into(self._alloc_wcfst, cap, self._L.tdsfs_fetch_wcfst)
+
+    def ld_windows(self, size, snp_mode=False, fetch=True):
+        """Per-window, per-population linkage disequilibrium over the candidate windows of (size, mode), in scan order
+        (tdsfs_ld_windows_*), from the genotype calls: over the rows that pass the spectrum filter and each population's
+        own samples, n_sites_p* the rows whose called dosages are not all equal, n_pairs_p* the row pairs with a defined
+        r^2, zns_p* Kelly's ZnS (their mean r^2, NaN without pairs), omega_p* Kim and Nielsen's omega at its best split
+        (NaN with fewer than 4 sites or no eligible split) and omega_pos_p* the position of the last site left of that
+        split (-1 when omega is NaN).  r^2 enters as rint(r^2 2^32) in exact integer sums: results are bitwise
+        reproducible.  Cost grows with the square of a window's rows.  Calls held as fix-ups count as missing.  Needs
+        load_genotypes.  Returns a dict of arrays (chrom / start / end / snp_count / flags as the scan's), or the
+        candidate count when fetch=False (results stay on the device: fetch_ld_windows)."""
+        return self._run("ld_windows", self._alloc_ld_windows, size, snp_mode, fetch)
+
+    def fetch_ld_windows(self, cap):
+        return self._into(self._alloc_ld_windows, cap, self._L.tdsfs_fetch_ld_windows)
 
     def ld_prune(self, size, step, threshold):
         """LD pruning of the loaded genotype rows (tdsfs_ld_prune): scikit-allel's locate_unlinked(gn, size, step,
@@ -406,6 +435,10 @@ class Handle:
         """CUDA-event time (ms) of the pair and resolve kernels of the last ld_prune call (tdsfs_timings slots 12 + 13)."""
         t = self.timings()
         return t["ld_pairs"] + t["ld_resolve"]
+
+    def ld_windows_ms(self):
+        """CUDA-event time (ms) of the pair + finish kernels of the last ld_windows call (tdsfs_timings slot 14)."""
+        return self.timings()["ld_windows"]
 
     def launch_count(self):
         return int(self._L.tdsfs_launch_count(self._h))

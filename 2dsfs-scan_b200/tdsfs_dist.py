@@ -318,3 +318,12 @@ def sharded_wcfst(handle, pieces, pos, size, device, *, snp_mode=False, group=No
     single-handle run bit for bit.  Returns the gathered arrays (identical on every rank)."""
     res = handle.wcfst(size, snp_mode=snp_mode)
     return gather_results(localize_results(res, pieces, pos, size, snp_mode), 0, group)
+
+
+def sharded_ld_windows(handle, pieces, pos, size, device, *, snp_mode=False, group=None):
+    """Per-window ZnS and omega of a sharded panel (genotype entry): the counterpart of sharded_wcfst, with the same
+    calling convention.  Every result of a window is a function of its own rows (exact integer sums), so the gathered
+    arrays equal a single-handle run bit for bit.  Cost grows with the square of a window's rows.  Returns the gathered
+    arrays (identical on every rank)."""
+    res = handle.ld_windows(size, snp_mode=snp_mode)
+    return gather_results(localize_results(res, pieces, pos, size, snp_mode), 0, group)

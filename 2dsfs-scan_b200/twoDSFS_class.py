@@ -583,6 +583,43 @@ class LikelihoodInference_jointSFS:
         self.snp_window_size = snp_window_size
         return self._wc_fst(panel, snp_window_size, True)
 
+    _LD_COLS = dict(snp_count="snp_count", sites_pop1="n_sites_p1", sites_pop2="n_sites_p2", pairs_pop1="n_pairs_p1",
+                    pairs_pop2="n_pairs_p2", ZnS_pop1="zns_p1", ZnS_pop2="zns_p2", omega_pop1="omega_p1",
+                    omega_pop2="omega_p2", omega_pos_pop1="omega_pos_p1", omega_pos_pop2="omega_pos_p2")
+
+    def _ld(self, panel, size, snp_mode):
+        if not isinstance(panel, PackedPanel):
+            raise TypeError("LD windows need the genotype calls: pass the PackedPanel of make_packed_panel "
+                            "(a data_dict holds allele counts only, without genotypes)")
+        keys, res = self._window_pass(panel, size, snp_mode, "ld_windows")
+        if not keys:
+            return {}
+        cols = [res[c] for c in self._LD_COLS.values()]
+        return {k: {name: None if (v != v or (name.startswith("omega_pos") and v < 0)) else v
+                    for name, v in zip(self._LD_COLS, row)} for k, row in zip(keys, zip(*cols))}
+
+    def ld_scan(self, panel, window_size):
+        """Linkage disequilibrium of each population in every non-empty fixed-bp window, computed on the GPU from the
+        genotype calls of a make_packed_panel panel: {"{chrom} {start}-{end}": {"snp_count", "sites_pop1", "sites_pop2",
+        "pairs_pop1", "pairs_pop2", "ZnS_pop1", "ZnS_pop2", "omega_pop1", "omega_pop2", "omega_pos_pop1",
+        "omega_pos_pop2"}}, keyed like wc_fst_scan.  Per population, over the SNPs that pass the constructor's filters and
+        that population's samples: sites are the SNPs whose called genotypes are not all equal (a SNP where every called
+        sample is heterozygous is not one); pairs the SNP pairs with a defined r^2 (the squared correlation of alt-allele
+        dosages over the samples called at both, as in ld_prune); ZnS (Kelly 1997) their mean r^2; omega (Kim and Nielsen
+        2004) the largest ratio of the mean r^2 within the two sides of a split of the sites to the mean r^2 across it,
+        over the splits with at least two sites on each side, and omega_pos the position of the last site left of the best
+        split.  A sweep leaves high omega near the selected site.  r^2 enters as rint(r^2 2^32) in exact integer sums.
+        None where undefined: ZnS without pairs, omega with fewer than 4 sites or no pair across any split.  Calls the
+        packer holds as fix-ups count as missing.  Cost grows with the square of a window's SNP count (a 500 kb window of
+        2,400 SNPs holds 2.9 million pairs).  Not in the reference; pass the result to save_csv_stats(ld=...)."""
+        self.window_size = window_size
+        return self._ld(panel, window_size, False)
+
+    def ld_scan_bySNPs(self, panel, snp_window_size):
+        """ld_scan over fixed-SNP windows, with the windows and keys of fst_scan_bySNPs."""
+        self.snp_window_size = snp_window_size
+        return self._ld(panel, snp_window_size, True)
+
     # ------------------------------------------------------------------ LD pruning (not in the reference)
     def ld_prune(self, panel, size=100, step=20, threshold=0.1):
         """Drop the SNPs in linkage disequilibrium from a make_packed_panel panel, on the GPU: scikit-allel's
@@ -690,15 +727,17 @@ def load_chr_ids(chromosomes_txt):
 col_names = ['chromosome', 'window_start', 'window_end', 'snp_count', 'T2D', 'T1D_p1', 'T1D_p2', 'new_term_p1', 'new_term_p2', 'T2D_diff']
 
 
-def save_csv_stats(stats_dict, output, fst=None, tajima=None):
+def save_csv_stats(stats_dict, output, fst=None, tajima=None, ld=None):
     """reference :1884-1907: same columns, chromosome mapped through chr_ids, None written as ''.  fst (not in the
     reference): the dict of fst_scan / fst_scan_bySNPs or wc_fst_scan / wc_fst_scan_bySNPs over the same windows adds a
     trailing FST column, the layout of the ECB tables the reference's R post-processing writes; '' where FST is None or
     the window has no entry.  tajima (not in the reference): the dict of tajima_scan / tajima_scan_bySNPs adds TajimaD_p1,
-    TajimaD_p2 after it, '' likewise."""
+    TajimaD_p2 after it, '' likewise.  ld (not in the reference): the dict of ld_scan / ld_scan_bySNPs adds ZnS_p1,
+    ZnS_p2, omega_p1, omega_p2 after those, '' likewise."""
     with open(output, 'w', newline='') as csvfile:
         writer = csv.DictWriter(csvfile, fieldnames=col_names + (['FST'] if fst is not None else [])
-                                + (['TajimaD_p1', 'TajimaD_p2'] if tajima is not None else []))
+                                + (['TajimaD_p1', 'TajimaD_p2'] if tajima is not None else [])
+                                + (['ZnS_p1', 'ZnS_p2', 'omega_p1', 'omega_p2'] if ld is not None else []))
         writer.writeheader()
         for window_coords, result in stats_dict.items():
             chromosome = window_coords.split(' ')[0]
@@ -712,6 +751,10 @@ def save_csv_stats(stats_dict, output, fst=None, tajima=None):
             if tajima is not None:
                 t = tajima.get(window_coords, {})
                 row['TajimaD_p1'], row['TajimaD_p2'] = t.get("TajimaD_pop1"), t.get("TajimaD_pop2")
+            if ld is not None:
+                t = ld.get(window_coords, {})
+                row['ZnS_p1'], row['ZnS_p2'] = t.get("ZnS_pop1"), t.get("ZnS_pop2")
+                row['omega_p1'], row['omega_p2'] = t.get("omega_pop1"), t.get("omega_pop2")
             writer.writerow(row)
 
 

@@ -314,6 +314,52 @@ int tdsfs_wcfst_bp(tdsfs_t* ctx, int64_t W, tdsfs_wcfst_t* out, int64_t cap, int
 int tdsfs_wcfst_snp(tdsfs_t* ctx, int64_t N, tdsfs_wcfst_t* out, int64_t cap, int64_t* n_windows);
 int tdsfs_fetch_wcfst(tdsfs_t* ctx, tdsfs_wcfst_t* out, int64_t cap, int64_t* n_windows);
 
+/* ---- per-window linkage disequilibrium: Kelly's ZnS and Kim and Nielsen's omega per population (no reference
+ * counterpart; DESIGN.md 7) ------------------------------------------------------------------------------------------
+ * Same windows and order as tdsfs_diversity_*, for data loaded with tdsfs_load_genotypes only (the counts entry gives
+ * TDSFS_ERR_STATE).  Rows: the window's rows that pass the spectrum filter (snp_flags bit0, read directly).  Per population
+ * i, samples are its own (not the padding bits of its last pair); dosage and missing calls as in tdsfs_ld_prune (calls held
+ * as fix-ups are missing).
+ *   site       a row whose called dosages are not all equal (vx > 0 over its own calls).  A row where every called sample
+ *              is heterozygous is NOT a site, unlike the segregating sites of tdsfs_neutrality_*;
+ *   pair       rows i < j of the window; over the samples called in both, cov, vx, vy as in tdsfs_ld_prune (exact int64).
+ *              Defined iff vx vy > 0 (never for a non-site row; two sites can still be undefined through missing calls),
+ *              and then r^2 = double(cov^2) / double(vx vy) and q = rint(r^2 2^32) (uint64, round to nearest even);
+ *   n_pairs    the defined pairs; zns = 2^-32 double(sum q) / double(n_pairs), each integer converted with round to
+ *              nearest; NaN when n_pairs = 0: Kelly's (1997) ZnS over the defined pairs;
+ *   omega      with the window's sites s_1 .. s_m in row order, for each split 2 <= k <= m - 2 (L = s_1 .. s_k, R the
+ *              rest): WL, WR, X the sums of q over the defined pairs within L, within R and across, nL, nR, nX their
+ *              counts, omega_k = (double(WL + WR) / double(nL + nR)) / (double(X) / double(nX)), eligible iff nL + nR > 0
+ *              and X > 0.  omega is the largest eligible omega_k (the lowest k on ties), NaN when none is (m < 4
+ *              included).  Without missing calls this is Kim and Nielsen's (2004) omega; parity with OmegaPlus is not
+ *              claimed (no distance cap, no sub-window grid);
+ *   omega_pos  the position of s_k at the best split (the split lies between it and the next site); -1 when omega is NaN.
+ * Every sum is an exact integer (window sums in 128 bits), so results are bitwise the same run to run and for any sharding
+ * that keeps windows whole.  Cost grows with the square of a window's rows.  Own window arrays, results and per-row
+ * scratch (about 49 bytes a loaded row, kept until the handle is destroyed), as tdsfs_diversity_*: a pending plan, the
+ * scan's results, the step graph, the other passes' results and tdsfs_ld_prune's buffers are left as they were.
+ * out == NULL: enqueue only (honours tdsfs_set_sync(0)); tdsfs_fetch_ld_windows copies the results later. */
+typedef struct {            /* caller-owned host SoA, capacity >= tdsfs_candidates_bp / _snp; any member may be NULL */
+  int32_t* chrom;           /* as tdsfs_result_t */
+  int64_t* start;
+  int64_t* end;
+  int32_t* snp_count;       /* count_snps, as tdsfs_result_t */
+  uint8_t* flags;           /* TDSFS_F_EMPTY */
+  int32_t* n_sites_p1;      /* sites m of population 1 */
+  int32_t* n_sites_p2;
+  int64_t* n_pairs_p1;      /* defined pairs */
+  int64_t* n_pairs_p2;
+  double* zns_p1;           /* NaN when n_pairs = 0 */
+  double* zns_p2;
+  double* omega_p1;         /* NaN when no split is eligible */
+  double* omega_p2;
+  int64_t* omega_pos_p1;    /* position of the last site left of the best split; -1 when omega is NaN */
+  int64_t* omega_pos_p2;
+} tdsfs_ld_windows_t;
+int tdsfs_ld_windows_bp(tdsfs_t* ctx, int64_t W, tdsfs_ld_windows_t* out, int64_t cap, int64_t* n_windows);
+int tdsfs_ld_windows_snp(tdsfs_t* ctx, int64_t N, tdsfs_ld_windows_t* out, int64_t cap, int64_t* n_windows);
+int tdsfs_fetch_ld_windows(tdsfs_t* ctx, tdsfs_ld_windows_t* out, int64_t cap, int64_t* n_windows);
+
 /* ---- LD pruning of the genotype rows (no reference counterpart; DESIGN.md 7) -----------------------------------------
  * scikit-allel's locate_unlinked (the windowed greedy r^2 rule of PLINK's --indep-pairwise) over the rows loaded with
  * tdsfs_load_genotypes.  Samples: both populations pooled (ns1 + ns2, the padding bits of a population's last pair are not
@@ -356,7 +402,8 @@ int tdsfs_synth_genotypes(tdsfs_t* ctx, void* G_dev, int64_t S, int64_t snp0, in
  * [9]=segment + finish kernels of the last tdsfs_diversity_* call (n >= 10),
  * [10]=segment + finish kernels of the last tdsfs_neutrality_* call (n >= 11),
  * [11]=segment + finish kernels of the last tdsfs_wcfst_* call (n >= 12),
- * [12]=k_ld_pairs and [13]=k_ld_resolve of the last tdsfs_ld_prune call (n >= 14). */
+ * [12]=k_ld_pairs and [13]=k_ld_resolve of the last tdsfs_ld_prune call (n >= 14),
+ * [14]=pair + finish kernels of the last tdsfs_ld_windows_* call (n >= 15). */
 int tdsfs_timings(tdsfs_t* ctx, float* ms, int32_t n);
 int64_t tdsfs_launch_count(tdsfs_t* ctx); /* kernels launched by this handle so far */
 /* Which path scored the last scan: *fused = 1 when the fused pair ran (tdsfs_plan_* before tdsfs_background on the
