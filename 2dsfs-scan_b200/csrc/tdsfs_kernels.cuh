@@ -874,6 +874,18 @@ __device__ __forceinline__ void write_result(const ScoreParams& p, long long id,
   p.r_flags[id] = f;
 }
 
+// Legacy Poisson score of one window (reference :295-303, :346-371), for both scorers: the sum over the bins with q != 0 of
+// poisson.logpmf(int(x + 1/total), S_w q), S_w = total + bins / total, from the window's sums over its populated bins with
+// q != 0 (xq = sum x, xlnq = sum x ln q, lg0 / lg1 = sum lgamma(x + 1) / lgamma(x + 2)):
+//   (e nQ + xq) ln S_w + e sum ln q + xlnq - S_w sum q - sum lgamma(x + e + 1),   e = 1 only when total == 1
+// (int(x + 1/total) = x + e in every bin).  A window with no counted SNP scores 0: the reference's S_w is 0 then.
+__device__ __forceinline__ double poisson_finish(const ScoreParams& p, int total, double xq, double xlnq, double lg0, double lg1) {
+  if (total == 0) return 0.0;
+  const double Sw = (double)total + (double)p.bins2d / (double)total;
+  const double e = total == 1 ? 1.0 : 0.0;
+  return (e * p.pq_n + xq) * log(Sw) + e * p.pq_lnsum + xlnq - Sw * p.pq_sum - (total == 1 ? lg1 : lg0);
+}
+
 // A group of G warps per candidate window (<= WCAP SNPs), 8 warps per CTA.  Per-group shared memory: an open-addressing
 // table of the window's 2D bins (one word per slot: bin << 10 | multiplicity), the list of occupied slots, packed
 // 16-bit folded 1D histograms and a small reduction scratch.
@@ -1073,6 +1085,9 @@ __global__ void __launch_bounds__(SCORE_WARPS * 32) k3_score_small(const __grid_
     };
     walk1d(h1a, nw1, lb1a, a1a, N1a);
     walk1d(h1b, nw2, lb1b, a1b, N1b);
+    if (EXTRA && p.poisson) {  // no 1D statistics: their slots carry the Poisson sums through the reduction (pz_xq <= N2)
+      a1a = pz_lg0; a1b = pz_lg1; N1a = pz_xq; N1b = 0;
+    }
     // ---- reduce: warp level, then across the group's warps through shared memory
     // N2 | N1a << 10 | N1b << 20 : every total is <= WCAP < 1024
     uint32_t nn = __reduce_add_sync(0xffffffffu, N2 | (N1a << 10) | (N1b << 20));
@@ -1097,23 +1112,14 @@ __global__ void __launch_bounds__(SCORE_WARPS * 32) k3_score_small(const __grid_
       }
     }
     if (EXTRA && p.poisson) {
-      // sum over the bins with q != 0 of poisson.logpmf(int(x + 1/total), S_w q), S_w = total + bins / total (:295-303, :346-371):
-      // (e nQ + X_Q) ln S_w + e sum ln q + sum x ln q - S_w sum q - sum lgamma(x + e + 1), e = 1 only when total == 1
-      pz_lg0 = warp_sum(pz_lg0); pz_lg1 = warp_sum(pz_lg1);
-      pz_xq = __reduce_add_sync(0xffffffffu, pz_xq);
-      // (the host launches the Poisson scan with one warp per window: nothing to combine across warps)
+      // the whole group's sums (the host asks for one warp per window, but panels too wide for eight tables in 200 KB get
+      // G = 2 or 4): lgamma(x + 1) in a1a, lgamma(x + 2) in a1b, the SNPs of the bins with q != 0 in N1a
       if (wg == 0 && lane == 0) {
         if (!has_flags) count = cnt;
         const int total = (int)(nn & 0x3FF);
-        double P = 0.0;
-        if (total > 0) {
-          const double Sw = (double)total + (double)p.bins2d / (double)total;
-          const double e = total == 1 ? 1.0 : 0.0;
-          P = (e * p.pq_n + (double)pz_xq) * log(Sw) + e * p.pq_lnsum + a2 - Sw * p.pq_sum - (total == 1 ? pz_lg1 : pz_lg0);
-        }
         p.r_count[id] = count;
         p.r_flags[id] = 0;
-        p.r_T2[id] = P;
+        p.r_T2[id] = poisson_finish(p, total, (double)((nn >> 10) & 0x3FF), a2, a1a, a1b);
         p.r_n2[id] = total;
         p.r_T1a[id] = 0.0; p.r_T1b[id] = 0.0; p.r_n1a[id] = 0; p.r_n1b[id] = 0;
       }
@@ -1167,7 +1173,9 @@ __device__ __forceinline__ void score_large_windows(const ScoreParams& p, int ct
     const double* lb1b = p.lb1b + (long long)g * (p.n2 + 1);
     int N2 = 0, N1a = 0, N1b = 0, nall = 0, count = 0;
     double a2 = 0.0, a1a = 0.0, a1b = 0.0;
-    double pz_lg = 0.0;  // Poisson score: lgamma term (a window above WCAP SNPs has total > 1)
+    // Poisson score: sums of lgamma(x + 1) and lgamma(x + 2) over the populated bins with q != 0, and their SNPs (rows that
+    // fail the spectrum filter or are monomorphic count in a window's rows but not in its total: total <= 1 happens here too)
+    double pz_lg0 = 0.0, pz_lg1 = 0.0;
     int pz_xq = 0;
     for (int s = lo + tid; s < hi; s += LARGE_THREADS) {
       const uint2 r = load_rec(p.rec, p.fmt, s, p.n1, p.n2, p.C2);
@@ -1187,7 +1195,12 @@ __device__ __forceinline__ void score_large_windows(const ScoreParams& p, int ct
       if (k != 0 && k != last) {
         const uint32_t x = atomicExch(h2 + k, 0u);
         if (x && p.poisson) {
-          if (lb2[k] != -INFINITY) { a2 = fma((double)x, lb2[k], a2); pz_lg += lgamma((double)x + 1.0); pz_xq += (int)x; }
+          if (lb2[k] != -INFINITY) {
+            a2 = fma((double)x, lb2[k], a2);
+            pz_lg0 += lgamma((double)x + 1.0);
+            pz_lg1 += lgamma((double)x + 2.0);
+            pz_xq += (int)x;
+          }
         } else if (x) a2 = fma((double)x, ln_mult(p, x) - lb2[k], a2);
       }
       const int fa = (int)(a & 0xFFFF), fb = (int)(a >> 16);
@@ -1201,7 +1214,7 @@ __device__ __forceinline__ void score_large_windows(const ScoreParams& p, int ct
       }
     }
     // block reduce
-    if (p.poisson) { a1a = pz_lg; N1a = pz_xq; }  // reduced in the slots of the (unused) 1D statistics
+    if (p.poisson) { a1a = pz_lg0; a1b = pz_lg1; N1a = pz_xq; }  // reduced in the slots of the (unused) 1D statistics
     double dv[3] = {a2, a1a, a1b};
     int iv[5] = {N2, N1a, N1b, nall, count};
     for (int q = 0; q < 3; ++q) { dv[q] = warp_sum(dv[q]); if (lane == 0) red_d[q][warp] = dv[q]; }
@@ -1211,12 +1224,10 @@ __device__ __forceinline__ void score_large_windows(const ScoreParams& p, int ct
       for (int q = 0; q < 3; ++q) { double t = 0; for (int x = 0; x < LARGE_THREADS / 32; ++x) t += red_d[q][x]; dv[q] = t; }
       for (int q = 0; q < 5; ++q) { int t = 0; for (int x = 0; x < LARGE_THREADS / 32; ++x) t += red_i[q][x]; iv[q] = t; }
       if (p.poisson) {
-        const int total = iv[0];
-        const double Sw = (double)total + (double)p.bins2d / (double)total;
         p.r_count[id] = iv[4];
         p.r_flags[id] = 0;
-        p.r_T2[id] = (double)iv[1] * log(Sw) + dv[0] - Sw * p.pq_sum - dv[1];
-        p.r_n2[id] = total;
+        p.r_T2[id] = poisson_finish(p, iv[0], (double)iv[1], dv[0], dv[1], dv[2]);
+        p.r_n2[id] = iv[0];
         p.r_T1a[id] = 0.0; p.r_T1b[id] = 0.0; p.r_n1a[id] = 0; p.r_n1b[id] = 0;
       } else {
         write_result(p, id, iv[4], iv[3], iv[0], iv[1], iv[2], dv[0], dv[1], dv[2], p.B + g * 6);
